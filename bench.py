@@ -1,5 +1,6 @@
 #!/usr/bin/env python3
 """Benchmark of the PolyFastA hot path on B200:  python bench.py --gpus N --steps K --warmup W  [--impl reference] [--workload c4|c3|c5]
+[--dump-outputs DIR]
 
 Workloads (BASELINE.json configs; DESIGN.md section 4):
 
@@ -68,7 +69,13 @@ def parse_args():
                          "path); 'nccl' = scan kernel + torch.distributed all_reduce (comparison only)")
     ap.add_argument("--force-validity", action="store_true", help="c4: make the scan read the whole validity plane too (0.375 B/base)")
     ap.add_argument("--gaps-ppm", type=int, default=0, help="c4: gaps per million bases poked into the alignment (sparse validity)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed as DIR/<name>.npy "
+                    "(float64, at most 64 MB in all): c4 site_stats = [S, H, folded SFS]; c3 site_stats and cds_stats [population][71]; "
+                    "c5 locus, S, H, sfs, pi_site, theta_site, tajimas_d (NaN for NA) per locus.  The inputs are seeded, so two builds "
+                    "can be compared output for output")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     dn, ds = {"c4": (N_SEQ, N_SITES), "c3": (C3_N, C3_SITES), "c5": (C5_N, C5_SITES)}[a.workload]
     a.n = a.n or dn
     a.sites = a.sites or ds
@@ -334,6 +341,51 @@ class Env:
         return elapsed_ms, kernel_ms, launches, clocks
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: arrays {name: integer or float array} -> directory/<name>.npy in float64 (integers only where exact)"""
+    import numpy as np
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        f = a.astype(np.float64)
+        if a.dtype.kind in "iu" and not np.array_equal(f.astype(a.dtype), a):
+            raise SystemExit("--dump-outputs: %s holds integers that float64 does not represent exactly" % name)
+        out[name] = f
+    total = sum(f.nbytes for f in out.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(directory, exist_ok=True)
+    for name, f in out.items():
+        np.save(os.path.join(directory, name + ".npy"), f)
+
+
+def c5_outputs(args, env, batches):
+    """the per-locus results of the last batched scan, gathered on rank 0 in locus order: every locus, or a fixed seeded sample
+    of them where all would exceed DUMP_LIMIT"""
+    import numpy as np
+    half = args.n // 2
+    cap = DUMP_LIMIT // (8 * (6 + half))
+    pick = range(args.loci) if args.loci <= cap else np.random.default_rng(0).choice(args.loci, cap, replace=False).tolist()
+    pick = set(pick)
+    rows = []
+    for bt, ids in batches:
+        for j, i in enumerate(ids):
+            if i in pick:
+                r = bt.result(j, 0, want_sfs=True)
+                _, pi, theta, d = r["poly"]
+                rows.append((i, r["S"], r["H"], pi, theta, float("nan") if d == "NA" else d, r["sfs"]))
+    if env.world > 1:
+        got = [None] * env.world if env.rank == 0 else None
+        env.dist.gather_object(rows, got, dst=0)
+        rows = sorted((r for part in got for r in part), key=lambda r: r[0]) if env.rank == 0 else []
+    col = lambda k: np.array([r[k] for r in rows])   # noqa: E731
+    return {"locus": col(0), "S": col(1), "H": col(2), "sfs": np.array([r[6] for r in rows], dtype=np.int64).reshape(len(rows), half),
+            "pi_site": col(3), "theta_site": col(4), "tajimas_d": col(5)}
+
+
 def traffic_for(key):
     """dram__bytes_read.sum + dram__bytes_write.sum per launch from the committed ncu --set full capture of this shape, or None"""
     try:
@@ -391,6 +443,8 @@ def run_c4(args, env):
         result = out.cpu().numpy().copy()
         if fused and xchg.timed_out():
             raise SystemExit("the NVLink exchange timed out on rank %d (a rank did not arrive)" % rank)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"site_stats": result})
         if os.environ.get("PFA_XCHG_STAMPS"):
             per = [a.elapsed_time(b) for a, b in env.kev]
             gaps = [env.kev[i][0].elapsed_time(env.kev[i + 1][0]) for i in range(args.steps - 1)]
@@ -577,6 +631,8 @@ def run_c3(args, env):
         site_vec, cds_vec = d_site.cpu().numpy().copy(), d_cds.cpu().numpy().copy()
         if fused and xchg.timed_out():
             raise SystemExit("the NVLink exchange timed out on rank %d" % rank)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"site_stats": site_vec, "cds_stats": cds_vec.reshape(k, api.PFA_CDS_LEN)})
     value = n * L * args.steps / (elapsed_ms * 1e-3)
     algo_bytes = n * (c1 - c0) * 2 / 8.0   # the codon scan reads the two base planes of the shard once (pure ACGT)
     if fused:
@@ -693,6 +749,10 @@ def run_c5(args, env):
         # the segmented site kernel is timed inside the library (CUDA events around it, pfa_batch_kernel_ms)
         kernel_ms = env.max_over_ranks(sum(ms_acc[-args.steps:]) / args.steps)
         kernel_name = ctx.last_kernel or "pfa_batch_site_kernel"
+        if args.dump_outputs:
+            dumped = c5_outputs(args, env, batches)
+            if rank == 0:
+                dump_outputs(args.dump_outputs, dumped)
     my_bases = n * L * len(mine)
     value = n * L * loci * args.steps / (elapsed_ms * 1e-3)
     algo_bytes = my_bases * 2 / 8.0

@@ -289,6 +289,38 @@ def test_bench_reference_arm_line():
     assert "workload" in d["config"]
 
 
+def test_bench_dump_outputs_helpers(tmp_path, monkeypatch):
+    """--dump-outputs: float64 files, integers only where float64 holds them exactly, and for c5 every locus in locus order
+    or, beyond the size limit, the same seeded sample of loci on every run"""
+    import types
+    import bench
+
+    class FakeBatch:
+        def __init__(self, ids):
+            self.ids = ids
+
+        def result(self, j, pop, want_sfs=False):
+            i = self.ids[j]
+            return {"S": i, "H": 3 * i, "sfs": [i % 7] * 10, "poly": (0, 0, 0, "NA") if i % 5 == 0 else (i, 0.5 * i, 0.25 * i, -1.5)}
+
+    args, env = types.SimpleNamespace(n=20, loci=25), types.SimpleNamespace(world=1, rank=0)
+    batches = [(FakeBatch(list(range(10))), list(range(10))), (FakeBatch(list(range(10, 25))), list(range(10, 25)))]
+    out = bench.c5_outputs(args, env, batches)
+    assert out["locus"].tolist() == list(range(25)) and out["sfs"].shape == (25, 10) and out["H"].tolist() == [3 * i for i in range(25)]
+    assert np.isnan(out["tajimas_d"][[0, 5]]).all() and out["tajimas_d"][1] == -1.5
+    bench.dump_outputs(str(tmp_path / "d"), out)
+    for name, a in out.items():
+        got = np.load(tmp_path / "d" / (name + ".npy"))
+        assert got.dtype == np.float64 and np.array_equal(got, a, equal_nan=True)
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "e"), {"x": np.array([2 ** 53 + 1])})
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 8 * (6 + 10) * 7)   # room for 7 of the 25 loci
+    picks = [bench.c5_outputs(args, env, batches)["locus"].tolist() for _ in range(2)]
+    assert picks[0] == picks[1] and len(picks[0]) == 7 and picks[0] == sorted(picks[0])
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "f"), out)
+
+
 @pytest.mark.parametrize("mapped", ["1", "0"])
 def test_big_file_path_refuses_non_ascii_sequence_bytes(tmp_path, monkeypatch, mapped):
     """bytes >= 0x80 in SEQUENCE lines are refused on every parse path (headers may hold them)"""
