@@ -41,7 +41,8 @@ int pfa_ctx_create(int device, pfa_ctx** out);
 int pfa_ctx_destroy(pfa_ctx* ctx);
 const char* pfa_last_error(const pfa_ctx* ctx);
 int pfa_ctx_sync(pfa_ctx* ctx);
-/* device memory freed by the library stays in the device's stream-ordered pool for reuse; this returns it to the driver */
+/* device memory freed by the library stays in the device's stream-ordered pool for reuse, and the planes of the last freed
+ * alignment stay mapped for the next one; this synchronises the ctx's stream and returns both to the driver */
 int pfa_ctx_trim(pfa_ctx* ctx);
 /* run the library's work for this ctx on a caller-owned stream (cudaStream_t as void*; e.g. torch's
  * current stream) so that a collective enqueued by the caller is ordered after the kernels. NULL restores
@@ -114,6 +115,10 @@ int64_t pfa_aln_nsites(const pfa_aln* a);        /* sites in this shard */
 int64_t pfa_aln_num_escapes(const pfa_aln* a);   /* entries in the exception list */
 int64_t pfa_aln_packed_bytes(const pfa_aln* a);  /* bytes of the three planes */
 int pfa_aln_has_invalid(const pfa_aln* a);       /* any non-ACGT symbol in the shard */
+/* where the planes live: 0 = the device's stream-ordered pool, 1 = a virtual-memory range (cuMemCreate), 2 = the same, in
+ * compressible memory.  PFA_PLANE_ALLOC = pool | vmm | compressible (default) chooses for planes of at least
+ * PFA_PLANE_ALLOC_MIN_BYTES (default 64 MB); a device that does not grant compression gets 1 or 0 */
+int pfa_aln_plane_alloc(const pfa_aln* a);
 /* benchmarking: force the scans to read the validity plane even though the shard is pure ACGT (flag != 0) */
 int pfa_aln_force_validity(pfa_aln* a, int flag);
 /* measurement aid (bench.py): time `reps` passes of a kernel that only READS the first `planes` planes of this shard with the

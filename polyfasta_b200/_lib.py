@@ -20,7 +20,7 @@ EXPORTS = [
     "pfa_fasta_parse_file", "pfa_fasta_parse_buffer", "pfa_fasta_free", "pfa_fasta_nseq", "pfa_fasta_seqlen",
     "pfa_fasta_row_len", "pfa_fasta_header", "pfa_fasta_copy_row",
     "pfa_aln_from_fasta", "pfa_aln_from_rows", "pfa_aln_from_device_rows", "pfa_aln_synthetic", "pfa_synth_text_device", "pfa_aln_poke_gaps", "pfa_aln_force_validity", "pfa_aln_free",
-    "pfa_aln_nseq", "pfa_aln_nsites", "pfa_aln_num_escapes", "pfa_aln_packed_bytes", "pfa_aln_has_invalid",
+    "pfa_aln_nseq", "pfa_aln_nsites", "pfa_aln_num_escapes", "pfa_aln_packed_bytes", "pfa_aln_has_invalid", "pfa_aln_plane_alloc",
     "pfa_aln_copy_plane", "pfa_aln_read_probe", "pfa_aln_mask_words", "pfa_aln_set_pops", "pfa_aln_num_pops", "pfa_aln_pop_size",
     "pfa_site_len", "pfa_site_offset", "pfa_site_stats_device", "pfa_site_stats",
     "pfa_cds_stats_device", "pfa_cds_stats", "pfa_codon_pair_labels", "pfa_codon_set_labels", "pfa_codon_syn3",
@@ -98,6 +98,7 @@ def lib():
         "pfa_aln_num_escapes": (i64, [p]),
         "pfa_aln_packed_bytes": (i64, [p]),
         "pfa_aln_has_invalid": (c.c_int, [p]),
+        "pfa_aln_plane_alloc": (c.c_int, [p]),
         "pfa_aln_poke_gaps": (c.c_int, [p, c.c_uint64, c.c_uint32]),
         "pfa_aln_copy_plane": (c.c_int, [p, c.c_int, p, sz]),
         "pfa_aln_read_probe": (c.c_int, [p, c.c_int, c.c_int, c.POINTER(c.c_double)]),

@@ -325,6 +325,11 @@ class Alignment:
         check(lib().pfa_aln_force_validity(self.handle, int(bool(flag))), self.ctx.handle)
 
     @property
+    def plane_alloc(self):
+        """where the planes live: "pool", "vmm" or "compressible" (PFA_PLANE_ALLOC at the time of the upload)"""
+        return ("pool", "vmm", "compressible")[lib().pfa_aln_plane_alloc(self.handle)]
+
+    @property
     def packed_bytes(self):
         return int(lib().pfa_aln_packed_bytes(self.handle))
 

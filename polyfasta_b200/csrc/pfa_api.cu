@@ -6,11 +6,176 @@
 #include <cstring>
 #include <new>
 
+#include <cuda.h>
+#include <cudaTypedefs.h>
+
 #include "pfa_common.cuh"
 #include "pfa_host.h"
 #include "pfa_sites.cuh"
 
 static thread_local std::string g_error;
+
+// ---- plane memory ----------------------------------------------------------------------------------------
+// Most 128-byte lines of the planes are uniform (a monomorphic site's record is all zeros or all ones in each plane), and
+// Blackwell compresses such lines between L2 and HBM in memory allocated as compressible.  Stream-ordered pools cannot ask for
+// that, so large planes get their own virtual-memory range over one cuMemCreate allocation.  The driver entry points come
+// through the runtime: the library links only libcudart.
+
+struct VmmApi {
+    PFN_cuDeviceGet_v2000 device_get = nullptr;
+    PFN_cuDeviceGetAttribute_v2000 attribute = nullptr;
+    PFN_cuMemGetAllocationGranularity_v10020 granularity = nullptr;
+    PFN_cuMemCreate_v10020 create = nullptr;
+    PFN_cuMemRelease_v10020 release = nullptr;
+    PFN_cuMemAddressReserve_v10020 reserve = nullptr;
+    PFN_cuMemAddressFree_v10020 address_free = nullptr;
+    PFN_cuMemMap_v10020 map = nullptr;
+    PFN_cuMemUnmap_v10020 unmap = nullptr;
+    PFN_cuMemSetAccess_v10020 set_access = nullptr;
+    PFN_cuMemGetAllocationPropertiesFromHandle_v10020 properties = nullptr;
+    bool ok = false;
+};
+
+template <typename F>
+static bool driver_entry(const char* name, F* fn) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+    if (cudaGetDriverEntryPointByVersion(name, &p, 12000, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    *fn = reinterpret_cast<F>(p);
+    return p != nullptr;
+}
+
+static const VmmApi& vmm_api() {
+    static const VmmApi api = [] {
+        VmmApi v;
+        v.ok = driver_entry("cuDeviceGet", &v.device_get) && driver_entry("cuDeviceGetAttribute", &v.attribute) &&
+               driver_entry("cuMemGetAllocationGranularity", &v.granularity) && driver_entry("cuMemCreate", &v.create) &&
+               driver_entry("cuMemRelease", &v.release) && driver_entry("cuMemAddressReserve", &v.reserve) &&
+               driver_entry("cuMemAddressFree", &v.address_free) && driver_entry("cuMemMap", &v.map) &&
+               driver_entry("cuMemUnmap", &v.unmap) && driver_entry("cuMemSetAccess", &v.set_access) &&
+               driver_entry("cuMemGetAllocationPropertiesFromHandle", &v.properties);
+        return v;
+    }();
+    return api;
+}
+
+static void vmm_release(pfa_vmm_range* r) {
+    if (!r->ptr) return;
+    const VmmApi& api = vmm_api();
+    const CUdeviceptr p = reinterpret_cast<CUdeviceptr>(r->ptr);
+    api.unmap(p, r->size);
+    api.address_free(p, r->size);
+    api.release(static_cast<CUmemGenericAllocationHandle>(r->handle));
+    *r = pfa_vmm_range();
+}
+
+// a new range of at least `bytes` on the ctx's device; false (nothing held) on any failure
+static bool vmm_create(pfa_ctx* ctx, size_t bytes, int want, pfa_vmm_range* out) {
+    const VmmApi& api = vmm_api();
+    if (!api.ok) return false;
+    CUdevice dev;
+    if (api.device_get(&dev, ctx->device) != CUDA_SUCCESS) return false;
+    CUmemAllocationProp prop = {};
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = dev;
+    if (want == PFA_PLANES_COMPRESSIBLE) {
+        int supported = 0;
+        if (api.attribute(&supported, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, dev) != CUDA_SUCCESS || !supported) return false;
+        prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    }
+    size_t gran = 0;
+    if (api.granularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED) != CUDA_SUCCESS || gran == 0) return false;
+    const size_t size = (size_t)pfa_round_up((int64_t)bytes, (int64_t)gran);
+    CUmemGenericAllocationHandle h;
+    if (api.create(&h, size, &prop, 0) != CUDA_SUCCESS) return false;
+    CUdeviceptr p = 0;
+    if (api.reserve(&p, size, gran, 0, 0) != CUDA_SUCCESS) {
+        api.release(h);
+        return false;
+    }
+    CUmemAccessDesc access = {};
+    access.location = prop.location;
+    access.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+    bool mapped = false;
+    if (api.map(p, size, 0, h, 0) == CUDA_SUCCESS) {
+        mapped = true;
+        if (api.set_access(p, size, &access, 1) == CUDA_SUCCESS) {
+            // what the driver granted: compression can be refused (no compression resources left, a virtualised device)
+            CUmemAllocationProp got = {};
+            const bool compressed = want == PFA_PLANES_COMPRESSIBLE && api.properties(&got, h) == CUDA_SUCCESS &&
+                                    got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC;
+            out->ptr = reinterpret_cast<void*>(p);
+            out->size = size;
+            out->handle = static_cast<unsigned long long>(h);
+            out->want = want;
+            out->kind = compressed ? PFA_PLANES_COMPRESSIBLE : PFA_PLANES_VMM;
+            return true;
+        }
+    }
+    if (mapped) api.unmap(p, size);
+    api.address_free(p, size);
+    api.release(h);
+    return false;
+}
+
+// PFA_PLANE_ALLOC = pool | vmm | compressible (default) for planes of at least PFA_PLANE_ALLOC_MIN_BYTES (default 64 MB); both
+// are read at every allocation so that one process can compare the kinds
+static int plane_alloc_wanted(size_t bytes) {
+    int want = PFA_PLANES_COMPRESSIBLE;
+    if (const char* e = getenv("PFA_PLANE_ALLOC")) {
+        if (!strcmp(e, "pool")) want = PFA_PLANES_POOL;
+        else if (!strcmp(e, "vmm")) want = PFA_PLANES_VMM;
+    }
+    size_t min_bytes = (size_t)64 << 20;
+    if (const char* e = getenv("PFA_PLANE_ALLOC_MIN_BYTES")) min_bytes = (size_t)strtoull(e, nullptr, 10);
+    return bytes >= min_bytes ? want : PFA_PLANES_POOL;
+}
+
+// the planes of `a`: the ctx's cached range when it fits, a new range, or (no VMM wanted, or any failure) the pool
+static cudaError_t plane_alloc(pfa_ctx* ctx, pfa_aln* a, size_t bytes) {
+    const int want = plane_alloc_wanted(bytes);
+    if (want != PFA_PLANES_POOL) {
+        pfa_vmm_range& c = ctx->plane_cache;
+        if (c.ptr && (c.want != want || c.size < bytes)) {
+            // kernels of earlier alignments may still read the cached range
+            const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+            if (e != cudaSuccess) return e;
+            vmm_release(&c);
+        }
+        if (c.ptr || vmm_create(ctx, bytes, want, &c)) {
+            a->plane_vmm = c;
+            c = pfa_vmm_range();
+            a->planes = static_cast<uint4*>(a->plane_vmm.ptr);
+            a->plane_alloc = a->plane_vmm.kind;
+            return cudaSuccess;
+        }
+    }
+    a->plane_alloc = PFA_PLANES_POOL;
+    return pfa_dmalloc(ctx, &a->planes, bytes);
+}
+
+// the planes of a freed alignment go back to the ctx's cache; of two ranges the larger one stays
+static void plane_free(pfa_ctx* ctx, pfa_aln* a) {
+    if (a->plane_alloc == PFA_PLANES_POOL) {
+        pfa_dfree(ctx, a->planes);
+        return;
+    }
+    pfa_vmm_range& c = ctx->plane_cache;
+    if (c.ptr) {
+        cudaStreamSynchronize(ctx->stream);
+        if (c.size >= a->plane_vmm.size) {
+            vmm_release(&a->plane_vmm);
+            return;
+        }
+        vmm_release(&c);
+    }
+    c = a->plane_vmm;
+    a->plane_vmm = pfa_vmm_range();
+}
 
 void pfa_set_global_error(const char* fmt, ...) {
     char buf[1024];
@@ -144,6 +309,7 @@ int pfa_ctx_destroy(pfa_ctx* ctx) {
     if (!ctx) return PFA_OK;
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
+    vmm_release(&ctx->plane_cache);
     if (ctx->h_scratch) cudaFreeHost(ctx->h_scratch);
     if (ctx->d_scratch) cudaFree(ctx->d_scratch);
     if (ctx->d_work) cudaFree(ctx->d_work);
@@ -169,6 +335,7 @@ int pfa_ctx_trim(pfa_ctx* ctx) {
     if (!ctx) return PFA_ERR_ARG;
     PFA_CUDA(ctx, cudaSetDevice(ctx->device));
     PFA_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    vmm_release(&ctx->plane_cache);
     cudaMemPool_t pool;
     PFA_CUDA(ctx, cudaDeviceGetDefaultMemPool(&pool, ctx->device));
     PFA_CUDA(ctx, cudaMemPoolTrimTo(pool, 0));
@@ -199,7 +366,7 @@ int pfa_aln_free(pfa_aln* a) {
     if (!a) return PFA_OK;
     pfa_ctx* ctx = a->ctx;
     cudaSetDevice(ctx->device);
-    pfa_dfree(ctx, a->planes);
+    plane_free(ctx, a);
     pfa_dfree(ctx, a->vflag);
     pfa_dfree(ctx, a->exc_keys);
     pfa_dfree(ctx, a->exc_heads);
@@ -254,6 +421,7 @@ int64_t pfa_aln_nsites(const pfa_aln* a) { return a ? a->ns : 0; }
 int64_t pfa_aln_num_escapes(const pfa_aln* a) { return a ? a->n_exc : 0; }
 int64_t pfa_aln_packed_bytes(const pfa_aln* a) { return a ? 3 * a->ns * (int64_t)a->Wq * 16 : 0; }
 int pfa_aln_has_invalid(const pfa_aln* a) { return a ? a->has_invalid : 0; }
+int pfa_aln_plane_alloc(const pfa_aln* a) { return a ? a->plane_alloc : -1; }
 int pfa_aln_force_validity(pfa_aln* a, int flag) {
     if (!a) return PFA_ERR_ARG;
     if (flag) a->has_invalid |= 2;
@@ -417,7 +585,7 @@ int pfa_aln_alloc(pfa_ctx* ctx, int64_t n, int64_t L, int64_t col_begin, int64_t
     // ceil(n/128), long site records padded to whole 32-byte sectors so that no sector is shared by two sites
     a->Wq = (int)(pfa_mask_words_for(n) / 4);
     a->plane_bytes = (size_t)pfa_round_up(std::max<int64_t>(a->ns * (int64_t)a->Wq * 16, 16), 256);
-    cudaError_t e = pfa_dmalloc(ctx, &a->planes, 3 * a->plane_bytes);
+    cudaError_t e = plane_alloc(ctx, a, 3 * a->plane_bytes);
     if (e != cudaSuccess) {
         const size_t want = 3 * a->plane_bytes;
         delete a;

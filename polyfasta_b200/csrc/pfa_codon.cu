@@ -1348,7 +1348,7 @@ int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg*
         {                                                                                                                 \
             cudaFuncSetAttribute(pfa_cds_scan_tma_kernel<L_, I_, V_, M_, N_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn); \
             pfa_cds_scan_tma_kernel<L_, I_, V_, M_, N_><<<tgrid, N_, dyn, st>>>(args, tma_stages, m);                      \
-            pfa_note_kernel(ctx, "pfa_cds_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d,NT=%d> grid=%u slots=%d passes_per_slot=%d v_records_per_slot=%d", L_, I_, (int)V_, (int)M_, N_, tgrid, tma_stages, m, args.s.vs); \
+            pfa_note_kernel(ctx, "pfa_cds_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d,NT=%d> grid=%u slots=%d passes_per_slot=%d v_records_per_slot=%d planes=%s", L_, I_, (int)V_, (int)M_, N_, tgrid, tma_stages, m, args.s.vs, pfa_plane_alloc_name(a->plane_alloc)); \
         }
 #define PFA_CDS_TMA_CASE(L_, I_, N_)                                                                                    \
         if (!launched && lps == L_ && iter == I_ && dyn <= PFA_TMA_SMEM_MAX) {                                                  \
@@ -1392,8 +1392,8 @@ int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg*
         return pfa_fail(ctx, PFA_ERR_ARG, "cds scan: no kernel for lps=%d iter=%d", lps, iter);
     }
 #undef PFA_CDS_CASE
-    pfa_note_kernel(ctx, "%s<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d", generic ? "pfa_cds_scan_kernel" : "pfa_cds_scan_reg_kernel", lps, iter,
-                    (int)hv, (int)multi, grid.x, PFA_SITE_THREADS);
+    pfa_note_kernel(ctx, "%s<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d planes=%s", generic ? "pfa_cds_scan_kernel" : "pfa_cds_scan_reg_kernel", lps, iter,
+                    (int)hv, (int)multi, grid.x, PFA_SITE_THREADS, pfa_plane_alloc_name(a->plane_alloc));
     PFA_LAUNCH_CHECK(ctx);
     if (x) pfa_xchg_commit(x);
     if (!x && a->n_exc_sites > 0) return launch_cds_escape(a, args);

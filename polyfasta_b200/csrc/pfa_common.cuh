@@ -11,6 +11,18 @@
 
 #define PFA_SM_COUNT_FALLBACK 148
 
+// where an alignment's planes live (pfa_aln_plane_alloc)
+enum { PFA_PLANES_POOL = 0, PFA_PLANES_VMM = 1, PFA_PLANES_COMPRESSIBLE = 2 };
+
+// a virtual-memory range mapped onto one physical allocation (cuMemCreate): `want` is the kind asked for, `kind` the kind
+// granted (a device without compressible memory grants PFA_PLANES_VMM)
+struct pfa_vmm_range {
+    void* ptr = nullptr;
+    size_t size = 0;
+    unsigned long long handle = 0;  // CUmemGenericAllocationHandle
+    int want = 0, kind = 0;
+};
+
 // ---- handles ----------------------------------------------------------------------------------------
 struct pfa_ctx {
     int device = 0;
@@ -39,6 +51,9 @@ struct pfa_ctx {
     bool codon_tables_ready = false;  // constant-memory tables of K4 uploaded (first codon scan)
     int host_threads = 0;  // host threads the ingest may use; 0 = PFA_HOST_THREADS or all hardware threads
     int64_t ingest_stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // last upload: chunks sent as text, chunks packed on the host, dirty chunks, threads, H2D bytes as text, H2D bytes packed, packed chunks that carried a validity bitmap
+    // the VMM range of the planes of the last freed alignment: the next alignment that fits takes it over (mapping tens of GB
+    // costs milliseconds).  Unmapped only after a synchronise of the stream (pfa_ctx_trim, pfa_ctx_destroy, a larger request).
+    pfa_vmm_range plane_cache;
 };
 
 struct pfa_aln {
@@ -49,6 +64,8 @@ struct pfa_aln {
     int64_t ns = 0;         // sites in this shard
     int Wq = 0;             // uint4 per site per plane = ceil(n/128)
     uint4* planes = nullptr;  // one allocation: b0 | b1 | v
+    int plane_alloc = PFA_PLANES_POOL;  // where `planes` came from
+    pfa_vmm_range plane_vmm;  // the range behind `planes` unless they came from the pool
     uint4 *b0 = nullptr, *b1 = nullptr, *v = nullptr;
     size_t plane_bytes = 0;  // bytes of ONE plane (ns*Wq*16, padded to 256)
     int has_invalid = 0;  // bit 0: a row shows a symbol outside ACGT somewhere; bit 1: forced (benchmarks: read the v plane everywhere)
@@ -80,6 +97,9 @@ struct pfa_aln {
 int pfa_fail(pfa_ctx* ctx, int code, const char* fmt, ...);
 void pfa_set_global_error(const char* fmt, ...);
 void pfa_note_kernel(pfa_ctx* ctx, const char* fmt, ...);
+static inline const char* pfa_plane_alloc_name(int kind) {
+    return kind == PFA_PLANES_COMPRESSIBLE ? "compressible" : kind == PFA_PLANES_VMM ? "vmm" : "pool";
+}
 
 #define PFA_CUDA(ctx, call)                                                                       \
     do {                                                                                          \

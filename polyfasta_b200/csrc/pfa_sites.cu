@@ -746,9 +746,9 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
     // over n = 100 ... 20,000 (scripts/probe_k2_shapes.py): 1-2 % faster at n = 10,000, 6-20 % at n = 2,000 ... 6,000 and
     // 16,000, ~10 % for n <= 384; slower only for records of 4 ... 10 chunks handled by 1-2 lanes (n = 385 ... 1,280), which
     // stay on the register kernel.  ONE slot per warp: a second one puts more bytes in flight than the memory system likes
-    // (7.0 -> 6.5 TB/s).  PFA_SITE_TMA=<slots> (0 = off), PFA_SITE_TMA_M (passes per slot).
+    // (7.0 -> 6.5 TB/s).  PFA_SITE_TMA=<slots> (0 = off, at most 2 for measurements), PFA_SITE_TMA_M (passes per slot).
     int tma_stages = 1;
-    if (const char* e = getenv("PFA_SITE_TMA")) tma_stages = std::max(0, std::min(1, atoi(e)));  // 0: off; one slot per warp
+    if (const char* e = getenv("PFA_SITE_TMA")) tma_stages = std::max(0, std::min(2, atoi(e)));
     bool use_tma = lps >= 4 || a->Wq <= 3;
     if (const char* e = getenv("PFA_SITE_TMA_MIN_LPS")) use_tma = lps >= std::max(1, atoi(e));
     if (tma_stages > 0 && !generic && use_tma) {
@@ -797,7 +797,7 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
         {                                                                                                                 \
             cudaFuncSetAttribute(pfa_site_scan_tma_kernel<L_, I_, V_, M_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn); \
             pfa_site_scan_tma_kernel<L_, I_, V_, M_><<<tgrid, nt, dyn, st>>>(args, tma_stages, m);                         \
-            pfa_note_kernel(ctx, "pfa_site_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d slots=%d passes_per_slot=%d v_records_per_slot=%d", L_, I_, (int)V_, (int)M_, tgrid, nt, tma_stages, m, args.vs); \
+            pfa_note_kernel(ctx, "pfa_site_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d slots=%d passes_per_slot=%d v_records_per_slot=%d planes=%s", L_, I_, (int)V_, (int)M_, tgrid, nt, tma_stages, m, args.vs, pfa_plane_alloc_name(a->plane_alloc)); \
         }
 #define PFA_TMA_CASE(L_, I_)                                                                                            \
         if (!launched && lps == L_ && iter == I_ && dyn <= PFA_TMA_SMEM_MAX) {                                                  \
@@ -847,8 +847,8 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
         return pfa_fail(ctx, PFA_ERR_ARG, "site scan: no kernel for lps=%d iter=%d", lps, iter);
     }
 #undef PFA_REG_CASE
-    pfa_note_kernel(ctx, "%s<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d", generic ? "pfa_site_scan_kernel" : "pfa_site_scan_reg_kernel", lps, iter,
-                    (int)hv, (int)multi, grid.x, PFA_SITE_THREADS);
+    pfa_note_kernel(ctx, "%s<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d planes=%s", generic ? "pfa_site_scan_kernel" : "pfa_site_scan_reg_kernel", lps, iter,
+                    (int)hv, (int)multi, grid.x, PFA_SITE_THREADS, pfa_plane_alloc_name(a->plane_alloc));
     PFA_LAUNCH_CHECK(ctx);
     if (x && !defer) pfa_xchg_commit(x);
     if (!x && a->n_exc_sites > 0) return launch_escape_sites(a, args);
