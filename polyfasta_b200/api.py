@@ -60,7 +60,8 @@ class Context:
 
     @property
     def last_kernel(self):
-        """the scan kernel of the last K2 / K4 launch as instantiated, e.g. 'pfa_site_scan_tma_kernel<LPS=16,ITER=5,...> grid=148 ...'"""
+        """the scan kernel of the last K2 / K4 launch as instantiated, with its grid and, for the TMA kernels, passes and
+        validity records per slot, e.g. 'pfa_site_scan_tma_kernel<LPS=16,ITER=5,...> grid=148 block=512 passes_per_slot=1 ...'"""
         return lib().pfa_ctx_last_kernel(self.handle).decode()
 
     @property

@@ -339,7 +339,7 @@ __device__ __forceinline__ unsigned pfa_cds_pass1(const uint4 (&x0)[3][ITER], co
 }
 
 // everything after pass 1 of one codon column whose three site records are in registers (f: the 18 flag bits of pass 1);
-// shared by the register-resident kernel, the TMA kernel's per-group path and the batched kernel
+// shared by the TMA kernel's per-group path and the batched kernel
 template <int LPS, int ITER, bool HAS_V, bool MULTI>
 __device__ __forceinline__ void pfa_cds_finish_regs(const PfaCdsView& a, int64_t site0, unsigned f, const uint4 (&x0)[3][ITER],
                                                     const uint4 (&x1)[3][ITER], const uint4 (&xv)[3][ITER], const uint4 (&um)[ITER], int sub,
@@ -536,73 +536,6 @@ __device__ __forceinline__ void pfa_cds_process(const PfaCdsView& a, int64_t sit
                                                 unsigned long long* sm_acc, unsigned& u_nstops, unsigned& u_missing, unsigned& u_sum3) {
     const unsigned f = pfa_cds_pass1<LPS, ITER, HAS_V>(x0, x1, xv, um, gmask);
     pfa_cds_finish_regs<LPS, ITER, HAS_V, MULTI>(a, site0, f, x0, x1, xv, um, sub, gmask, Wq, sm_acc, u_nstops, u_missing, u_sum3);
-}
-
-// Register-resident variant (Wq <= 3*32 chunks): the three site records of a codon column are loaded once -- all
-// loads back to back -- and pass 1, the class counts and the codon peeling of pass 2 all work on registers.
-
-template <int LPS, int ITER, bool HAS_V, bool MULTI>
-__global__ void __launch_bounds__(PFA_SITE_THREADS, (ITER >= 3) ? 1 : 2) pfa_cds_scan_reg_kernel(const PfaCdsArgs a) {
-    extern __shared__ unsigned long long smem[];
-    const int nacc = 3 + (a.acc_in_smem ? a.s.k * PFA_CDS_LEN : 0);
-    for (int i = threadIdx.x; i < nacc; i += blockDim.x) smem[i] = 0ull;
-    __syncthreads();
-    unsigned long long* sm_acc = smem + 3;
-
-    const int lane = threadIdx.x & 31;
-    const int sub = lane & (LPS - 1);
-    const unsigned gmask = LPS == 32 ? 0xffffffffu : (((1u << LPS) - 1u) << (lane - sub));
-    const int64_t gid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / LPS;
-    const int64_t ngroups = (int64_t)gridDim.x * blockDim.x / LPS;
-    const int Wq = a.s.Wq;
-    unsigned u_nstops = 0, u_missing = 0, u_sum3 = 0;
-
-    uint4 um[ITER];
-#pragma unroll
-    for (int i = 0; i < ITER; ++i) {
-        const int j = sub + LPS * i;
-        um[i] = j < Wq ? __ldg(a.s.umask + j) : make_uint4(0, 0, 0, 0);
-    }
-
-    for (int64_t cc = gid; cc < a.ncf; cc += ngroups) {
-        const int64_t site0 = cc * 3;
-        uint4 x0[3][ITER], x1[3][ITER], xv[3][ITER];
-#pragma unroll
-        for (int t = 0; t < 3; ++t)
-#pragma unroll
-            for (int i = 0; i < ITER; ++i) {
-                const int j = sub + LPS * i;
-                x0[t][i] = x1[t][i] = make_uint4(0, 0, 0, 0);
-                xv[t][i] = um[i];
-                if (j < Wq) {
-                    x0[t][i] = pfa_ld_stream(a.s.b0 + (site0 + t) * Wq + j);
-                    x1[t][i] = pfa_ld_stream(a.s.b1 + (site0 + t) * Wq + j);
-                    if (HAS_V) xv[t][i] = pfa_ld_stream(a.s.v + (site0 + t) * Wq + j);
-                }
-            }
-        pfa_cds_process<LPS, ITER, HAS_V, MULTI>(pfa_cds_view(a), site0, x0, x1, xv, um, sub, gmask, Wq, sm_acc, u_nstops, u_missing, u_sum3);
-    }
-    if (a.has_partial && blockIdx.x == 0 && threadIdx.x == 0) u_missing += 3;
-    for (int off = 16; off; off >>= 1) {
-        u_nstops += __shfl_xor_sync(0xffffffffu, u_nstops, off);
-        u_missing += __shfl_xor_sync(0xffffffffu, u_missing, off);
-        u_sum3 += __shfl_xor_sync(0xffffffffu, u_sum3, off);
-    }
-    if (lane == 0) {
-        if (u_nstops) atomicAdd(&smem[0], (unsigned long long)u_nstops);
-        if (u_missing) atomicAdd(&smem[1], (unsigned long long)u_missing);
-        if (u_sum3) atomicAdd(&smem[2], (unsigned long long)u_sum3);
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < a.s.k * PFA_CDS_LEN; i += blockDim.x) {
-        const int e = i % PFA_CDS_LEN;
-        unsigned long long x = a.acc_in_smem ? sm_acc[i] : 0ull;
-        if (e == PFA_CDS_NSTOPS) x += smem[0];
-        if (e == PFA_CDS_MISSING) x += smem[1];
-        if (e == PFA_CDS_SUM3 + 1) x += smem[2];
-        if (x) atomicAdd(reinterpret_cast<unsigned long long*>(a.out) + i, x);
-    }
-    if (a.s.x.world) pfa_xchg_epilogue(a.s.x);
 }
 
 // ---- deferred bookkeeping of the variable codon columns ---------------------------------------------------------------------
@@ -1018,11 +951,11 @@ __device__ __forceinline__ void pfa_cds_tma_pass(const PfaCdsArgs& a, const unsi
     }
 }
 
-// TMA variant (see pfa_site_scan_tma_kernel): every warp owns shared-memory slots holding the site records of the codon
+// TMA variant (see pfa_site_scan_tma_kernel): every warp owns a shared-memory slot holding the site records of the codon
 // columns of m of its passes (3 * 32/LPS consecutive sites per pass), fed by one cp.async.bulk per plane.  Pass 1 runs per
 // group on registers; variable columns (LPS >= 4) are finished by the whole warp one at a time from the slot (pfa_cds_coop).
 template <int LPS, int ITER, bool HAS_V, bool MULTI, int NT>
-__global__ void __launch_bounds__(NT, 1) pfa_cds_scan_tma_kernel(const PfaCdsArgs a, int stages, int m) {
+__global__ void __launch_bounds__(NT, 1) pfa_cds_scan_tma_kernel(const PfaCdsArgs a, int m) {
     extern __shared__ __align__(128) unsigned char dyn[];
     constexpr bool COOP = LPS >= 4;  // three site records per column: holding them through pass 2 spills (ptxas), the slot does not
     constexpr int GW = 32 / LPS;        // codon columns per warp pass
@@ -1036,12 +969,12 @@ __global__ void __launch_bounds__(NT, 1) pfa_cds_scan_tma_kernel(const PfaCdsArg
     const unsigned slot_bytes = (unsigned)pfa_slot_bytes(HAS_V, (unsigned)SPS, VS, rec);
     const bool sparse = HAS_V && a.s.vflag != nullptr;  // fetch only the flagged cells of the v plane
     const int gc = a.s.gc, gcw = a.s.gc * 4;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(dyn + (size_t)NWARP * stages * slot_bytes);
-    unsigned long long* smem = reinterpret_cast<unsigned long long*>(bars + NWARP * stages);  // [3] uniform + accumulators
+    uint64_t* bars = reinterpret_cast<uint64_t*>(dyn + (size_t)NWARP * slot_bytes);
+    unsigned long long* smem = reinterpret_cast<unsigned long long*>(bars + NWARP);  // [3] uniform + accumulators
     const int nacc = 3 + (a.acc_in_smem ? a.s.k * PFA_CDS_LEN : 0);
     for (int i = threadIdx.x; i < nacc; i += blockDim.x) smem[i] = 0ull;
     if (threadIdx.x == 0) {
-        for (int i = 0; i < NWARP * stages; ++i) pfa_mbar_init(&bars[i], 1);
+        for (int i = 0; i < NWARP; ++i) pfa_mbar_init(&bars[i], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
@@ -1053,8 +986,8 @@ __global__ void __launch_bounds__(NT, 1) pfa_cds_scan_tma_kernel(const PfaCdsArg
     unsigned u_nstops = 0, u_missing = 0, u_sum3 = 0;
     uint32_t* qbuf = reinterpret_cast<uint32_t*>(smem + nacc) + wib * (PFA_CDS_QFIELDS * 32);  // this warp's queue (COOP)
     int qcount = 0;
-    unsigned char* ring = dyn + (size_t)wib * stages * slot_bytes;
-    uint64_t* bar = bars + wib * stages;
+    unsigned char* ring = dyn + (size_t)wib * slot_bytes;
+    uint64_t* bar = bars + wib;
     const int64_t nw = (int64_t)gridDim.x * NWARP;
     const int64_t nblk = (a.ncf + CPS - 1) / CPS;                    // blocks of CPS consecutive codon columns
     const unsigned char* planes[3] = {reinterpret_cast<const unsigned char*>(a.s.b0), reinterpret_cast<const unsigned char*>(a.s.b1),
@@ -1245,15 +1178,6 @@ static void launch_cds(const PfaCdsArgs& args, bool has_v, dim3 grid, size_t sme
     else pfa_cds_scan_kernel<LPS, false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
 }
 
-static int launch_cds_escape(pfa_aln* a, const PfaCdsArgs& args) {
-    pfa_ctx* ctx = a->ctx;
-    int64_t eb = (a->n_exc_sites + 7) / 8;
-    if (eb > (int64_t)ctx->sm_count * 8) eb = (int64_t)ctx->sm_count * 8;
-    pfa_cds_escape_kernel<<<(unsigned)eb, 256, 0, ctx->stream>>>(args, a->exc_keys, a->n_exc, a->exc_heads, a->n_exc_sites);
-    PFA_LAUNCH_CHECK(ctx);
-    return PFA_OK;
-}
-
 int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg* x) {
     pfa_ctx* ctx = a->ctx;
     if (!ctx->codon_tables_ready) {
@@ -1286,124 +1210,66 @@ int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg*
     const size_t smem = 8 * (3 + (args.acc_in_smem ? (size_t)a->k * PFA_CDS_LEN : 0));
     int lps = 1;
     while (lps < 32 && (a->Wq + lps - 1) / lps > 2) lps *= 2;
-    int iter = (a->Wq + lps - 1) / lps;
-    const bool probe_sparse = getenv("PFA_PROBE_SPARSE_V") != nullptr;  // measurement aid: the validity-aware kernel on a clean shard
-    const bool hv = a->has_invalid != 0 || probe_sparse, multi = a->k > 1;
+    const int iter = (a->Wq + lps - 1) / lps;
+    const bool hv = pfa_scan_has_v(a), multi = a->k > 1;
     const bool generic = iter > 3 || getenv("PFA_GENERIC_SCAN") != nullptr;
     if (generic) {
         lps = 1;
         while (lps < 32 && (a->Wq + lps - 1) / lps > 4) lps *= 2;
     }
+    const char* planes = pfa_plane_alloc_name(a->plane_alloc);
+    cudaStream_t st = ctx->stream;
     if (x) {  // escape columns first: the scan kernel's last block runs the exchange over the complete shard vector
         if (a->n_exc_sites > 0) {
-            int rc = launch_cds_escape(a, args);
+            int rc = pfa_launch_escape(a, pfa_cds_escape_kernel, args);
             if (rc) return rc;
         }
         int rc = pfa_xchg_fill(x, carry + out_len, d_out, &args.s.x, true);  // the TMA kernels run one CTA per SM
         if (rc) return rc;
     }
-    const int64_t groups_per_block = PFA_SITE_THREADS / lps;
-    int64_t blocks = (std::max<int64_t>(args.ncf, 1) + groups_per_block - 1) / groups_per_block;
-    const int64_t max_blocks = (int64_t)ctx->sm_count * (generic ? 4 : (iter >= 3 ? 1 : 2));
-    if (blocks > max_blocks) blocks = max_blocks;
-    dim3 grid((unsigned)blocks);
-    cudaStream_t st = ctx->stream;
-    // TMA variant: per-warp shared-memory slots of ~5 KB per plane fed by cp.async.bulk (PFA_CDS_TMA=0 turns it off)
-    int tma_stages = 1;
-    if (const char* e = getenv("PFA_CDS_TMA")) tma_stages = std::max(0, std::min(1, atoi(e)));  // 0: off; one slot per warp
-    if (tma_stages > 0 && !generic && a->ns >= 3) {
+    if (!generic) {
+        // TMA variant: per-warp shared-memory slots of ~10 KB per plane (three site records per codon column) fed by cp.async.bulk
         const int nt = iter >= 3 ? 256 : 512;
         const int gw = 32 / lps, nwarp = nt / 32;
-        int m = (int)std::max<int64_t>(1, 10000 / ((int64_t)gw * 3 * a->Wq * 16));
-        if (const char* e = getenv("PFA_CDS_TMA_M")) m = std::max(1, atoi(e));
-        // validity flags: fetch only the flagged pieces of the v plane (see pfa_launch_site_scan)
-        const bool sparse_v = (a->has_invalid == 1 || (probe_sparse && a->has_invalid == 0)) && lps >= 4 && a->Wq >= 4 && !(getenv("PFA_VFLAG") && atoi(getenv("PFA_VFLAG")) == 0);
-        if (sparse_v) {
-            args.s.vflag = a->vflag;
-            m = std::max(1, std::min(m, 32 * PFA_VF_REGS / (3 * gw)));
-        }
-        // sparse validity: the fewer sites are flagged, the smaller the slots' v area and the more passes per slot (see
-        // pfa_launch_site_scan); 2,000 rows: two passes per slot as in the pure-ACGT kernel instead of one
-        int64_t flagged_sites = 0;
-        if (sparse_v)
-            if (int rc = pfa_aln_flagged_sites(a, &flagged_sites)) return rc;
-        int v_div = 1;  // v area = sites per slot / v_div records (at least one codon column)
-        if (sparse_v && !(getenv("PFA_VCOMPACT") && atoi(getenv("PFA_VCOMPACT")) == 0))
-            v_div = flagged_sites * 64 <= a->ns ? 8 : flagged_sites * 16 <= a->ns ? 4 : flagged_sites * 4 <= a->ns ? 2 : 1;
-        if (sparse_v && getenv("PFA_VDIV")) v_div = std::max(1, std::min(8, atoi(getenv("PFA_VDIV"))));  // tests: force a small v area
-        if (v_div > 1 && !getenv("PFA_CDS_TMA_M")) m = std::max(1, std::min(m + (m + 1) / 2, 32 * PFA_VF_REGS / (3 * gw)));
-        auto vs_for = [&](int mm) { return hv ? std::max(3, 3 * gw * mm / v_div) : 0; };
-        auto dyn_for = [&](int mm) {
-            return (size_t)nwarp * tma_stages * pfa_slot_bytes(hv, (unsigned)(3 * gw * mm), (unsigned)vs_for(mm), (unsigned)a->Wq * 16u) +
-                   sizeof(uint64_t) * nwarp * tma_stages + smem + 1024 /* unconditional chunk loads may run past the last record */ +
-                   (lps >= 4 ? (size_t)nwarp * PFA_CDS_QFIELDS * 32 * sizeof(uint32_t) : 0);
-        };
-        while (m > 1 && dyn_for(m) > PFA_TMA_SMEM_MAX) --m;
-        const size_t dyn = dyn_for(m);
-        args.s.vs = vs_for(m);
-        const int64_t per_cta = (int64_t)gw * m * nwarp;
-        const unsigned tgrid = (unsigned)std::min<int64_t>(ctx->sm_count, (std::max<int64_t>(args.ncf, 1) + per_cta - 1) / per_cta);
-        bool launched = false;
-#define PFA_CDS_TMA_LAUNCH(L_, I_, V_, M_, N_)                                                                          \
-        {                                                                                                                 \
-            cudaFuncSetAttribute(pfa_cds_scan_tma_kernel<L_, I_, V_, M_, N_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn); \
-            pfa_cds_scan_tma_kernel<L_, I_, V_, M_, N_><<<tgrid, N_, dyn, st>>>(args, tma_stages, m);                      \
-            pfa_note_kernel(ctx, "pfa_cds_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d,NT=%d> grid=%u slots=%d passes_per_slot=%d v_records_per_slot=%d planes=%s", L_, I_, (int)V_, (int)M_, N_, tgrid, tma_stages, m, args.s.vs, pfa_plane_alloc_name(a->plane_alloc)); \
-        }
-#define PFA_CDS_TMA_CASE(L_, I_, N_)                                                                                    \
-        if (!launched && lps == L_ && iter == I_ && dyn <= PFA_TMA_SMEM_MAX) {                                                  \
-            if (hv && multi) PFA_CDS_TMA_LAUNCH(L_, I_, true, true, N_)                                                   \
-            else if (hv) PFA_CDS_TMA_LAUNCH(L_, I_, true, false, N_)                                                      \
-            else if (multi) PFA_CDS_TMA_LAUNCH(L_, I_, false, true, N_)                                                   \
-            else PFA_CDS_TMA_LAUNCH(L_, I_, false, false, N_)                                                             \
-            launched = true;                                                                                              \
-        }
-        PFA_CDS_TMA_CASE(1, 1, 512) PFA_CDS_TMA_CASE(1, 2, 512) PFA_CDS_TMA_CASE(2, 2, 512) PFA_CDS_TMA_CASE(4, 2, 512)
-        PFA_CDS_TMA_CASE(8, 2, 512) PFA_CDS_TMA_CASE(16, 2, 512) PFA_CDS_TMA_CASE(32, 2, 512) PFA_CDS_TMA_CASE(32, 3, 256)
-#undef PFA_CDS_TMA_CASE
-#undef PFA_CDS_TMA_LAUNCH
-        if (launched) {
-            PFA_LAUNCH_CHECK(ctx);
-            if (x) pfa_xchg_commit(x);
-            if (!x && a->n_exc_sites > 0) return launch_cds_escape(a, args);
-            return PFA_OK;
-        }
+        const size_t queues = lps >= 4 ? (size_t)nwarp * PFA_CDS_QFIELDS * 32 * sizeof(uint32_t) : 0;  // pfa_cds_flush
+        const int m = (int)std::max<int64_t>(1, 10000 / ((int64_t)gw * 3 * a->Wq * 16));
+        const PfaTmaShape shape = {3, args.ncf, lps, nt, m, "PFA_CDS_TMA_M", 8, 1, smem + queues, hv};
+        PfaTmaPlan p;
+        if (int rc = pfa_tma_plan(a, shape, &p)) return rc;
+        if (p.sparse_v) args.s.vflag = a->vflag;
+        args.s.vs = p.vs;
+        const bool found = pfa_for_shape<1, 1, 1, 2, 2, 2, 4, 2, 8, 2, 16, 2, 32, 2, 32, 3>(lps, iter, [&](auto L, auto I) {
+            pfa_for_v_multi(hv, multi, [&](auto V, auto M) {
+                constexpr int NT = decltype(I)::value >= 3 ? 256 : 512;
+                auto kernel = pfa_cds_scan_tma_kernel<decltype(L)::value, decltype(I)::value, decltype(V)::value, decltype(M)::value, NT>;
+                cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.dyn);
+                kernel<<<p.grid, NT, p.dyn, st>>>(args, p.m);
+            });
+        });
+        if (!found) return pfa_fail(ctx, PFA_ERR_ARG, "cds scan: no TMA kernel for lps=%d iter=%d", lps, iter);
+        pfa_note_kernel(ctx, "pfa_cds_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d,NT=%d> grid=%u passes_per_slot=%d v_records_per_slot=%d planes=%s",
+                        lps, iter, (int)hv, (int)multi, nt, p.grid, p.m, args.s.vs, planes);
+        return pfa_scan_done(a, x, true, pfa_cds_escape_kernel, args);
     }
     args.s.x.wide = 0;  // see pfa_launch_site_scan
-#define PFA_CDS_CASE(L_, I_)                                                                                          \
-    if (lps == L_ && iter == I_) {                                                                                    \
-        if (hv && multi) pfa_cds_scan_reg_kernel<L_, I_, true, true><<<grid, PFA_SITE_THREADS, smem, st>>>(args);       \
-        else if (hv) pfa_cds_scan_reg_kernel<L_, I_, true, false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);          \
-        else if (multi) pfa_cds_scan_reg_kernel<L_, I_, false, true><<<grid, PFA_SITE_THREADS, smem, st>>>(args);       \
-        else pfa_cds_scan_reg_kernel<L_, I_, false, false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);                 \
-    } else
-    if (generic) {
-        switch (lps) {
-            case 1: launch_cds<1>(args, hv, grid, smem, st); break;
-            case 2: launch_cds<2>(args, hv, grid, smem, st); break;
-            case 4: launch_cds<4>(args, hv, grid, smem, st); break;
-            case 8: launch_cds<8>(args, hv, grid, smem, st); break;
-            case 16: launch_cds<16>(args, hv, grid, smem, st); break;
-            default: launch_cds<32>(args, hv, grid, smem, st); break;
-        }
-    } else {
-        PFA_CDS_CASE(1, 1) PFA_CDS_CASE(1, 2) PFA_CDS_CASE(2, 2) PFA_CDS_CASE(4, 2) PFA_CDS_CASE(8, 2) PFA_CDS_CASE(16, 2)
-        PFA_CDS_CASE(32, 2) PFA_CDS_CASE(32, 3)
-        return pfa_fail(ctx, PFA_ERR_ARG, "cds scan: no kernel for lps=%d iter=%d", lps, iter);
+    const int64_t groups_per_block = PFA_SITE_THREADS / lps;
+    const dim3 grid((unsigned)std::min<int64_t>((std::max<int64_t>(args.ncf, 1) + groups_per_block - 1) / groups_per_block, (int64_t)ctx->sm_count * 4));
+    switch (lps) {
+        case 1: launch_cds<1>(args, hv, grid, smem, st); break;
+        case 2: launch_cds<2>(args, hv, grid, smem, st); break;
+        case 4: launch_cds<4>(args, hv, grid, smem, st); break;
+        case 8: launch_cds<8>(args, hv, grid, smem, st); break;
+        case 16: launch_cds<16>(args, hv, grid, smem, st); break;
+        default: launch_cds<32>(args, hv, grid, smem, st); break;
     }
-#undef PFA_CDS_CASE
-    pfa_note_kernel(ctx, "%s<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d planes=%s", generic ? "pfa_cds_scan_kernel" : "pfa_cds_scan_reg_kernel", lps, iter,
-                    (int)hv, (int)multi, grid.x, PFA_SITE_THREADS, pfa_plane_alloc_name(a->plane_alloc));
-    PFA_LAUNCH_CHECK(ctx);
-    if (x) pfa_xchg_commit(x);
-    if (!x && a->n_exc_sites > 0) return launch_cds_escape(a, args);
-    return PFA_OK;
+    pfa_note_kernel(ctx, "pfa_cds_scan_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d planes=%s", lps, iter, (int)hv, (int)multi, grid.x,
+                    PFA_SITE_THREADS, planes);
+    return pfa_scan_done(a, x, true, pfa_cds_escape_kernel, args);
 }
-
 
 // ---- K4b: the codon scan over a batch of small loci (--dir --cds; PolyFastA.py:104 calling :165, :284-315) ----------------
 // One warp per tile of PFA_BATCH_CTILE consecutive codon columns of ONE locus (the tile finds its locus by binary search);
-// a group of LPS lanes owns a codon column, as in pfa_cds_scan_reg_kernel, and runs the same per-column code
+// a group of LPS lanes owns a codon column, as in pfa_cds_scan_tma_kernel, and runs the same per-column code
 // (pfa_cds_process) on a view of the locus.  Contributions that are the same for every population of the locus -- the
 // monomorphic columns -- stay in registers until the end of the tile.
 template <int LPS, int ITER>

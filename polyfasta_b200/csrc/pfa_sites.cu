@@ -453,8 +453,8 @@ __device__ __forceinline__ void pfa_site_gap_apply(const PfaSiteArgs& a, int64_t
 }
 
 // TMA variant of the register-resident kernel: the bytes in flight are bounded by shared memory instead of registers.
-// Every WARP owns a private ring of STAGES shared-memory slots; a slot holds the records of the consecutive sites of m of the
-// warp's passes (contiguous in each plane), fetched with one cp.async.bulk per plane that completes on the slot's mbarrier.
+// Every WARP owns one private shared-memory slot; it holds the records of the consecutive sites of m of the warp's passes
+// (contiguous in each plane), fetched with one cp.async.bulk per plane that completes on the slot's mbarrier.
 // No block-wide synchronisation: a warp waits for its own slot and runs pass 1 of every site on registers (a group of LPS
 // lanes per site).  Variable sites (LPS >= 4): the whole warp takes them one at a time, reading the record back from the slot
 // (pfa_site_coop); narrow records handled by 1-2 lanes keep the per-group second pass (every lane has its own site there).
@@ -462,7 +462,7 @@ __device__ __forceinline__ void pfa_site_gap_apply(const PfaSiteArgs& a, int64_t
 // else after their second pass -- every shared-memory read of the slot has then been consumed (its value was used), and a
 // proxy fence orders those generic-proxy reads before the bulk copy's async-proxy writes.
 template <int LPS, int ITER, bool HAS_V, bool MULTI>
-__global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSiteArgs a, int stages, int m) {
+__global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSiteArgs a, int m) {
     constexpr int NT = 512;
     // whole-warp second pass for groups of 4-8 lanes; (half-)warp groups keep it on their registers -- unless the validity plane
     // is read too: three planes held through pass 2 do not fit 128 registers (ptxas: 150-360 bytes of spills), the slot does
@@ -480,15 +480,15 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
     const int gc = a.gc;
     const unsigned gcr = pfa_cell_rcp(a.gc * 4);
     unsigned char* ring_base = dyn;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(dyn + (size_t)NWARP * stages * slot_bytes);  // [warp][stage]
-    unsigned long long* sm_SH = reinterpret_cast<unsigned long long*>(bars + NWARP * stages);
+    uint64_t* bars = reinterpret_cast<uint64_t*>(dyn + (size_t)NWARP * slot_bytes);  // [warp]
+    unsigned long long* sm_SH = reinterpret_cast<unsigned long long*>(bars + NWARP);
     unsigned int* sm_sfs = reinterpret_cast<unsigned int*>(sm_SH + 2 * a.k);
     if (a.x.world && blockIdx.x == 0 && threadIdx.x == 0) a.x.stamps[5] = pfa_globaltimer();
     for (int i = threadIdx.x; i < 2 * a.k; i += blockDim.x) sm_SH[i] = 0ull;
     if (a.sfs_in_smem)
         for (int i = threadIdx.x; i < a.sfs_bins; i += blockDim.x) sm_sfs[i] = 0u;
     if (threadIdx.x == 0) {
-        for (int i = 0; i < NWARP * stages; ++i) pfa_mbar_init(&bars[i], 1);
+        for (int i = 0; i < NWARP; ++i) pfa_mbar_init(&bars[i], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
@@ -496,8 +496,8 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int sub = lane & (LPS - 1), grp = lane / LPS;
     const unsigned gmask = LPS == 32 ? 0xffffffffu : (((1u << LPS) - 1u) << (lane - sub));
-    unsigned char* ring = ring_base + (size_t)wib * stages * slot_bytes;
-    uint64_t* bar = bars + wib * stages;
+    unsigned char* ring = ring_base + (size_t)wib * slot_bytes;
+    uint64_t* bar = bars + wib;
     const int64_t nw = (int64_t)gridDim.x * NWARP;
     const int64_t nblk = (a.ns + SPS - 1) / SPS;                     // blocks of SPS consecutive sites
     const unsigned char* planes[3] = {reinterpret_cast<const unsigned char*>(a.b0), reinterpret_cast<const unsigned char*>(a.b1),
@@ -689,12 +689,49 @@ static void launch_scan(const PfaSiteArgs& args, bool has_v, dim3 grid, size_t s
     else pfa_site_scan_kernel<LPS, false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
 }
 
-static int launch_escape_sites(pfa_aln* a, const PfaSiteArgs& args) {
+bool pfa_scan_has_v(const pfa_aln* a) { return a->has_invalid != 0 || getenv("PFA_PROBE_SPARSE_V") != nullptr; }
+
+int pfa_tma_plan(pfa_aln* a, const PfaTmaShape& s, PfaTmaPlan* p) {
     pfa_ctx* ctx = a->ctx;
-    int64_t eb = (a->n_exc_sites + 7) / 8;
-    if (eb > (int64_t)ctx->sm_count * 8) eb = (int64_t)ctx->sm_count * 8;
-    pfa_escape_sites_kernel<<<(unsigned)eb, 256, 0, ctx->stream>>>(args, a->exc_keys, a->n_exc, a->exc_heads, a->n_exc_sites);
-    PFA_LAUNCH_CHECK(ctx);
+    const char* m_env = getenv(s.m_env);
+    const char* vflag = getenv("PFA_VFLAG");
+    const char* vcompact = getenv("PFA_VCOMPACT");
+    const char* vdiv = getenv("PFA_VDIV");
+    const int gw = 32 / s.lps, nwarp = s.nt / 32;
+    const int m_sparse = std::max(1, 32 * PFA_VF_REGS / (s.recs * gw));  // sparse validity: a slot's flag words fit PFA_VF_REGS per lane
+    int m = m_env ? std::max(1, atoi(m_env)) : s.m;
+    // validity flags: a shard with a few non-ACGT symbols fetches only the flagged pieces of its v plane (pfa_slot_issue); not
+    // when the validity plane is forced (benchmarks of the 3-plane worst case) or PFA_VFLAG=0
+    p->sparse_v = s.has_v && !(a->has_invalid & 2) && s.lps >= 4 && a->Wq >= 4 && !(vflag && atoi(vflag) == 0);
+    if (p->sparse_v) m = std::min(m, m_sparse);
+    // sparse validity: the fewer sites are flagged, the smaller the slots' v area and the more shared memory goes into passes per
+    // slot -- with two passes per slot the validity-aware K2 runs a clean or nearly clean 10,000-row shard as fast as the
+    // pure-ACGT kernel (0.73 against 0.77 ms with one; scripts/probe_gaps5.py), K4 at 2,000 rows two passes instead of one
+    p->flagged_sites = 0;
+    if (p->sparse_v)
+        if (int rc = pfa_aln_flagged_sites(a, &p->flagged_sites)) return rc;
+    p->v_div = 1;
+    if (p->sparse_v && !(vcompact && atoi(vcompact) == 0))
+        for (int d = s.v_div_max; d > 1 && p->v_div == 1; d /= 2)
+            if (p->flagged_sites * d * d <= a->ns) p->v_div = d;
+    if (p->sparse_v && vdiv) p->v_div = std::max(1, std::min(8, atoi(vdiv)));  // tests: force a small v area
+    if (p->v_div > 1 && !m_env) m = std::min(m + (m * s.m_raise + 1) / 2, m_sparse);
+    auto vs_for = [&](int mm) { return s.has_v ? std::max(s.recs, s.recs * gw * mm / p->v_div) : 0; };
+    auto dyn_for = [&](int mm) {
+        return (size_t)nwarp * pfa_slot_bytes(s.has_v, (unsigned)(s.recs * gw * mm), (unsigned)vs_for(mm), (unsigned)a->Wq * 16u) +
+               sizeof(uint64_t) * nwarp + s.smem + 1024;  // + slack: unconditional chunk loads may run past the last record
+    };
+    while (m > 1 && dyn_for(m) > PFA_TMA_SMEM_MAX) --m;
+    // At the widest record of either scan (160 chunks) one pass per slot fits for any k below ~6,600 populations.  Above
+    // k = 3,072 the register kernels' 16 k bytes of dynamic shared memory passed 48 KB: they could not take this case either.
+    if (dyn_for(m) > PFA_TMA_SMEM_MAX)
+        return pfa_fail(ctx, PFA_ERR_ARG, "TMA scan: one pass per slot needs %zu bytes of shared memory (k = %d populations, %d chunks per record)",
+                        dyn_for(m), a->k, a->Wq);
+    p->m = m;
+    p->vs = vs_for(m);
+    p->dyn = dyn_for(m);
+    const int64_t per_cta = (int64_t)gw * m * nwarp;
+    p->grid = (unsigned)std::min<int64_t>(ctx->sm_count, (std::max<int64_t>(s.units, 1) + per_cta - 1) / per_cta);
     return PFA_OK;
 }
 
@@ -717,7 +754,7 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
         // the scan kernel's last block sees the complete shard vector when it runs the exchange
         args.out = reinterpret_cast<int64_t*>(pfa_xchg_partial(x));
         if (a->n_exc_sites > 0) {
-            int rc = launch_escape_sites(a, args);
+            int rc = pfa_launch_escape(a, pfa_escape_sites_kernel, args);
             if (rc) return rc;
         }
         if (!defer) {
@@ -726,108 +763,53 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
         }
     }
     // lanes per site: the smallest power of two that leaves every lane at most 5 chunks
-    // (measured over n = 100 ... 10,000, scripts/probe_k2_shapes.py: fewer chunks per lane with more lanes per site, at
-    // higher occupancy, is never faster -- bytes in flight per lane win)
+    // (measured over n = 100 ... 10,000, DESIGN.md section 3: fewer chunks per lane with more lanes per site, at higher
+    // occupancy, is never faster -- bytes in flight per lane win)
     int lps = 1;
     while (lps < 32 && (a->Wq + lps - 1) / lps > 5) lps *= 2;
     const int iter = (a->Wq + lps - 1) / lps;
     const size_t smem = sizeof(unsigned long long) * 2 * (size_t)a->k + (args.sfs_in_smem ? sizeof(unsigned int) * (size_t)args.sfs_bins : 0);
-    const int64_t groups_per_block = PFA_SITE_THREADS / lps;
-    int64_t blocks = (a->ns + groups_per_block - 1) / groups_per_block;
-    const bool probe_sparse = getenv("PFA_PROBE_SPARSE_V") != nullptr;  // measurement aid: the validity-aware kernel on a clean shard
-    const bool hv = a->has_invalid != 0 || probe_sparse, multi = a->k > 1;
+    const bool hv = pfa_scan_has_v(a), multi = a->k > 1;
     const bool generic = iter > 5 || getenv("PFA_GENERIC_SCAN") != nullptr;
-    const int64_t max_blocks = (int64_t)ctx->sm_count * (generic ? 4 : 2);
-    if (blocks > max_blocks) blocks = max_blocks;
-    dim3 grid((unsigned)blocks);
+    const char* planes = pfa_plane_alloc_name(a->plane_alloc);
     cudaStream_t st = ctx->stream;
     // The TMA variant: one CTA of 512 threads per SM, every warp fed by cp.async.bulk through its own shared-memory slot of
     // about 5 KB per plane (several passes of the warp for narrow records).  Measured against the register-resident kernel
-    // over n = 100 ... 20,000 (scripts/probe_k2_shapes.py): 1-2 % faster at n = 10,000, 6-20 % at n = 2,000 ... 6,000 and
-    // 16,000, ~10 % for n <= 384; slower only for records of 4 ... 10 chunks handled by 1-2 lanes (n = 385 ... 1,280), which
-    // stay on the register kernel.  ONE slot per warp: a second one puts more bytes in flight than the memory system likes
-    // (7.0 -> 6.5 TB/s).  PFA_SITE_TMA=<slots> (0 = off, at most 2 for measurements), PFA_SITE_TMA_M (passes per slot).
-    int tma_stages = 1;
-    if (const char* e = getenv("PFA_SITE_TMA")) tma_stages = std::max(0, std::min(2, atoi(e)));
-    bool use_tma = lps >= 4 || a->Wq <= 3;
-    if (const char* e = getenv("PFA_SITE_TMA_MIN_LPS")) use_tma = lps >= std::max(1, atoi(e));
-    if (tma_stages > 0 && !generic && use_tma) {
-        const int nt = 512;
+    // over n = 100 ... 20,000 (DESIGN.md section 3): 1-2 % faster at n = 10,000, 6-20 % at n = 2,000 ... 6,000 and 16,000,
+    // ~10 % for n <= 384; slower only for records of 4 ... 10 chunks handled by 1-2 lanes (n = 385 ... 1,280), which stay on
+    // the register kernel.
+    if (!generic && (lps >= 4 || a->Wq <= 3)) {
+        constexpr int nt = 512;
         const int gw = 32 / lps, nwarp = nt / 32;
         const int64_t pass_bytes = (int64_t)gw * a->Wq * 16;  // one pass of a warp, per plane
         // passes per slot: ~5 KB per plane.  Rounded to the nearest when every warp still gets >= 512 blocks (C4 on one GPU, two
         // passes of 2.5 KB: 3.46 ms against 3.55 with one), else rounded down: on a 1.25 Mb shard of C4 (one of 8 GPUs) the larger
         // blocks cost 4 % (0.476 against 0.458 ms), at 5 Mb they break even
         int m = (int)std::max<int64_t>(1, 5000 / pass_bytes);
-        {
-            const int64_t m_near = std::max<int64_t>(1, (5000 + pass_bytes / 2) / pass_bytes);
-            if (m_near > m && a->ns / ((int64_t)gw * m_near * nwarp * ctx->sm_count) >= 512) m = (int)m_near;
-        }
-        if (const char* e = getenv("PFA_SITE_TMA_M")) m = std::max(1, atoi(e));
-        // validity flags: a shard with a few non-ACGT symbols fetches only the flagged pieces of its v plane (pfa_slot_issue);
-        // not when the validity plane is forced (benchmarks of the 3-plane worst case) or PFA_VFLAG=0
-        const bool sparse_v = (a->has_invalid == 1 || (probe_sparse && a->has_invalid == 0)) && lps >= 4 && a->Wq >= 4 && !(getenv("PFA_VFLAG") && atoi(getenv("PFA_VFLAG")) == 0);
-        if (sparse_v) {
-            args.vflag = a->vflag;
-            m = std::min(m, 32 * PFA_VF_REGS / gw);
-        }
-        // sparse validity: the fewer sites are flagged, the smaller the slots' v area (a half, a quarter of a plane) and the more
-        // shared memory goes into passes per slot -- with two passes per slot the validity-aware kernel runs a clean or nearly
-        // clean 10,000-row shard as fast as the pure-ACGT kernel (0.73 against 0.77 ms with one; scripts/probe_gaps5.py)
-        int64_t flagged_sites = 0;
-        if (sparse_v)
-            if (int rc = pfa_aln_flagged_sites(a, &flagged_sites)) return rc;
-        int v_div = 1;  // v area = sites per slot / v_div records
-        if (sparse_v && !(getenv("PFA_VCOMPACT") && atoi(getenv("PFA_VCOMPACT")) == 0))
-            v_div = flagged_sites * 16 <= a->ns ? 4 : flagged_sites * 4 <= a->ns ? 2 : 1;
-        if (sparse_v && getenv("PFA_VDIV")) v_div = std::max(1, std::min(8, atoi(getenv("PFA_VDIV"))));  // tests: force a small v area
-        if (v_div > 1 && !getenv("PFA_SITE_TMA_M")) m = std::min(2 * m, 32 * PFA_VF_REGS / gw);
-        auto vs_for = [&](int mm) { return hv ? std::max(1, gw * mm / v_div) : 0; };
-        auto dyn_for = [&](int mm) {
-            return (size_t)nwarp * tma_stages * pfa_slot_bytes(hv, (unsigned)(gw * mm), (unsigned)vs_for(mm), (unsigned)a->Wq * 16u) +
-                   sizeof(uint64_t) * nwarp * tma_stages + smem + 1024;  // + slack: unconditional chunk loads may run past the last record
-        };
-        while (m > 1 && dyn_for(m) > PFA_TMA_SMEM_MAX) --m;
-        const size_t dyn = dyn_for(m);
-        args.vs = vs_for(m);
-        const int64_t per_cta = (int64_t)gw * m * nwarp;
-        const unsigned tgrid = (unsigned)std::min<int64_t>(ctx->sm_count, (a->ns + per_cta - 1) / per_cta);
-        bool launched = false;
-#define PFA_TMA_LAUNCH(L_, I_, V_, M_)                                                                                  \
-        {                                                                                                                 \
-            cudaFuncSetAttribute(pfa_site_scan_tma_kernel<L_, I_, V_, M_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn); \
-            pfa_site_scan_tma_kernel<L_, I_, V_, M_><<<tgrid, nt, dyn, st>>>(args, tma_stages, m);                         \
-            pfa_note_kernel(ctx, "pfa_site_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d slots=%d passes_per_slot=%d v_records_per_slot=%d planes=%s", L_, I_, (int)V_, (int)M_, tgrid, nt, tma_stages, m, args.vs, pfa_plane_alloc_name(a->plane_alloc)); \
-        }
-#define PFA_TMA_CASE(L_, I_)                                                                                            \
-        if (!launched && lps == L_ && iter == I_ && dyn <= PFA_TMA_SMEM_MAX) {                                                  \
-            if (hv && multi) PFA_TMA_LAUNCH(L_, I_, true, true)                                                           \
-            else if (hv) PFA_TMA_LAUNCH(L_, I_, true, false)                                                              \
-            else if (multi) PFA_TMA_LAUNCH(L_, I_, false, true)                                                           \
-            else PFA_TMA_LAUNCH(L_, I_, false, false)                                                                     \
-            launched = true;                                                                                              \
-        }
-        PFA_TMA_CASE(16, 3) PFA_TMA_CASE(16, 4) PFA_TMA_CASE(16, 5) PFA_TMA_CASE(32, 3) PFA_TMA_CASE(32, 4) PFA_TMA_CASE(32, 5)
-        PFA_TMA_CASE(1, 1) PFA_TMA_CASE(1, 2) PFA_TMA_CASE(1, 3) PFA_TMA_CASE(1, 4) PFA_TMA_CASE(1, 5)
-        PFA_TMA_CASE(2, 3) PFA_TMA_CASE(2, 4) PFA_TMA_CASE(2, 5) PFA_TMA_CASE(4, 3) PFA_TMA_CASE(4, 4) PFA_TMA_CASE(4, 5)
-        PFA_TMA_CASE(8, 3) PFA_TMA_CASE(8, 4) PFA_TMA_CASE(8, 5)
-#undef PFA_TMA_CASE
-#undef PFA_TMA_LAUNCH
-        if (launched) {
-            PFA_LAUNCH_CHECK(ctx);
-            if (x && !defer) pfa_xchg_commit(x);
-            if (!x && a->n_exc_sites > 0) return launch_escape_sites(a, args);
-            return PFA_OK;
-        }
+        const int64_t m_near = std::max<int64_t>(1, (5000 + pass_bytes / 2) / pass_bytes);
+        if (m_near > m && a->ns / ((int64_t)gw * m_near * nwarp * ctx->sm_count) >= 512) m = (int)m_near;
+        const PfaTmaShape shape = {1, a->ns, lps, nt, m, "PFA_SITE_TMA_M", 4, 2, smem, hv};
+        PfaTmaPlan p;
+        if (int rc = pfa_tma_plan(a, shape, &p)) return rc;
+        if (p.sparse_v) args.vflag = a->vflag;
+        args.vs = p.vs;
+        const bool found = pfa_for_shape<1, 1, 1, 2, 1, 3, 4, 3, 4, 4, 4, 5, 8, 3, 8, 4, 8, 5, 16, 3, 16, 4, 16, 5, 32, 3, 32, 4, 32, 5>(
+            lps, iter, [&](auto L, auto I) {
+                pfa_for_v_multi(hv, multi, [&](auto V, auto M) {
+                    auto kernel = pfa_site_scan_tma_kernel<decltype(L)::value, decltype(I)::value, decltype(V)::value, decltype(M)::value>;
+                    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.dyn);
+                    kernel<<<p.grid, nt, p.dyn, st>>>(args, p.m);
+                });
+            });
+        if (!found) return pfa_fail(ctx, PFA_ERR_ARG, "site scan: no TMA kernel for lps=%d iter=%d", lps, iter);
+        pfa_note_kernel(ctx, "pfa_site_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d passes_per_slot=%d v_records_per_slot=%d planes=%s",
+                        lps, iter, (int)hv, (int)multi, p.grid, nt, p.m, args.vs, planes);
+        return pfa_scan_done(a, x, !defer, pfa_escape_sites_kernel, args);
     }
     args.x.wide = 0;  // several CTAs per SM, grids beyond the resident set: the last block alone runs the exchange
-#define PFA_REG_CASE(L_, I_)                                                                                          \
-    if (lps == L_ && iter == I_) {                                                                                    \
-        if (hv && multi) pfa_site_scan_reg_kernel<L_, I_, true, true><<<grid, PFA_SITE_THREADS, smem, st>>>(args);      \
-        else if (hv) pfa_site_scan_reg_kernel<L_, I_, true, false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);         \
-        else if (multi) pfa_site_scan_reg_kernel<L_, I_, false, true><<<grid, PFA_SITE_THREADS, smem, st>>>(args);      \
-        else pfa_site_scan_reg_kernel<L_, I_, false, false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);                \
-    } else
+    const int64_t groups_per_block = PFA_SITE_THREADS / lps;
+    const int64_t blocks = std::min<int64_t>((a->ns + groups_per_block - 1) / groups_per_block, (int64_t)ctx->sm_count * (generic ? 4 : 2));
+    const dim3 grid((unsigned)blocks);
     if (generic) {
         switch (lps) {
             case 1: launch_scan<1>(args, hv, grid, smem, st); break;
@@ -838,21 +820,17 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
             default: launch_scan<32>(args, hv, grid, smem, st); break;
         }
     } else {
-        PFA_REG_CASE(1, 1) PFA_REG_CASE(1, 2) PFA_REG_CASE(1, 3) PFA_REG_CASE(1, 4) PFA_REG_CASE(1, 5)
-        PFA_REG_CASE(2, 3) PFA_REG_CASE(2, 4) PFA_REG_CASE(2, 5)
-        PFA_REG_CASE(4, 3) PFA_REG_CASE(4, 4) PFA_REG_CASE(4, 5)
-        PFA_REG_CASE(8, 3) PFA_REG_CASE(8, 4) PFA_REG_CASE(8, 5)
-        PFA_REG_CASE(16, 3) PFA_REG_CASE(16, 4) PFA_REG_CASE(16, 5)
-        PFA_REG_CASE(32, 3) PFA_REG_CASE(32, 4) PFA_REG_CASE(32, 5)
-        return pfa_fail(ctx, PFA_ERR_ARG, "site scan: no kernel for lps=%d iter=%d", lps, iter);
+        const bool found = pfa_for_shape<1, 4, 1, 5, 2, 3, 2, 4, 2, 5>(lps, iter, [&](auto L, auto I) {
+            pfa_for_v_multi(hv, multi, [&](auto V, auto M) {
+                pfa_site_scan_reg_kernel<decltype(L)::value, decltype(I)::value, decltype(V)::value, decltype(M)::value>
+                    <<<grid, PFA_SITE_THREADS, smem, st>>>(args);
+            });
+        });
+        if (!found) return pfa_fail(ctx, PFA_ERR_ARG, "site scan: no kernel for lps=%d iter=%d", lps, iter);
     }
-#undef PFA_REG_CASE
     pfa_note_kernel(ctx, "%s<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d planes=%s", generic ? "pfa_site_scan_kernel" : "pfa_site_scan_reg_kernel", lps, iter,
-                    (int)hv, (int)multi, grid.x, PFA_SITE_THREADS, pfa_plane_alloc_name(a->plane_alloc));
-    PFA_LAUNCH_CHECK(ctx);
-    if (x && !defer) pfa_xchg_commit(x);
-    if (!x && a->n_exc_sites > 0) return launch_escape_sites(a, args);
-    return PFA_OK;
+                    (int)hv, (int)multi, grid.x, PFA_SITE_THREADS, planes);
+    return pfa_scan_done(a, x, !defer, pfa_escape_sites_kernel, args);
 }
 
 // ---- measurement aid: how fast can this GPU READ the planes at all? -------------------------------------------------------

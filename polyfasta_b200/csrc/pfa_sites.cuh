@@ -1,5 +1,8 @@
 // Device helpers shared by the site scan (K2), the escape-site kernel and the codon scan (K4).
 #pragma once
+#include <algorithm>
+#include <type_traits>
+
 #include "pfa_common.cuh"
 #include "pfa_xchg.cuh"
 
@@ -380,3 +383,78 @@ __device__ __forceinline__ bool pfa_slot_issue(unsigned char* slot, uint64_t* ba
 
 void pfa_fill_site_args(const pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, PfaSiteArgs* args);
 int pfa_aln_flagged_sites(pfa_aln* a, int64_t* out);
+
+// ---- launch plan of the TMA scans (K2, K4) -----------------------------------------------------------------------------------
+// does a scan of this shard read the validity plane?  (PFA_PROBE_SPARSE_V: the validity-aware kernels on a clean shard)
+bool pfa_scan_has_v(const pfa_aln* a);
+
+// what the site scan (a unit = one site record) and the codon scan (a unit = a codon column, three site records) tell the planner
+struct PfaTmaShape {
+    int recs;           // site records per unit; a slot's validity area holds at least one unit
+    int64_t units;      // units in the shard
+    int lps;            // lanes per unit
+    int nt;             // threads per CTA
+    int m;              // passes per slot, unless m_env is set
+    const char* m_env;  // the variable that overrides m
+    int v_div_max;      // sparse validity: the v area is 1/d of the slot's records, d = the largest power of two <= v_div_max
+                        // with at most 1/d^2 of the sites flagged
+    int m_raise;        // a v area below a whole slot raises m to m + ceil(m * m_raise / 2) (no m_env)
+    size_t smem;        // shared memory beyond the slots and their mbarriers: accumulators, queues
+    bool has_v;         // pfa_scan_has_v
+};
+struct PfaTmaPlan {
+    bool sparse_v;          // fetch only the flagged cells of the v plane (PfaSiteArgs::vflag)
+    int64_t flagged_sites;  // sites with a flagged cell (sparse_v)
+    int v_div;              // v area = records per slot / v_div
+    int m;                  // passes per slot
+    int vs;                 // validity records per slot (PfaSiteArgs::vs)
+    size_t dyn;             // dynamic shared memory of a CTA
+    unsigned grid;          // CTAs: at most one per SM
+};
+int pfa_tma_plan(pfa_aln* a, const PfaTmaShape& s, PfaTmaPlan* p);
+
+// f(integral_constant<int, L>, integral_constant<int, I>) for the pair (L, I) of the list that equals (lps, iter); false: none
+template <class F>
+bool pfa_for_shape(int, int, F&&) {
+    return false;
+}
+template <int L, int I, int... Rest, class F>
+bool pfa_for_shape(int lps, int iter, F&& f) {
+    if (lps == L && iter == I) {
+        f(std::integral_constant<int, L>{}, std::integral_constant<int, I>{});
+        return true;
+    }
+    return pfa_for_shape<Rest...>(lps, iter, f);
+}
+
+// f(integral_constant<bool, HAS_V>, integral_constant<bool, MULTI>) for the runtime pair
+template <class F>
+void pfa_for_v_multi(bool has_v, bool multi, F&& f) {
+    using T = std::true_type;
+    using N = std::false_type;
+    if (has_v && multi) f(T{}, T{});
+    else if (has_v) f(T{}, N{});
+    else if (multi) f(N{}, T{});
+    else f(N{}, N{});
+}
+
+// one warp per site (K2) or codon column (K4) that holds an escape symbol
+template <class Args>
+int pfa_launch_escape(pfa_aln* a, void (*kernel)(Args, const unsigned long long*, int64_t, const int64_t*, int64_t), const Args& args) {
+    pfa_ctx* ctx = a->ctx;
+    const int64_t eb = std::min<int64_t>((a->n_exc_sites + 7) / 8, (int64_t)ctx->sm_count * 8);
+    kernel<<<(unsigned)eb, 256, 0, ctx->stream>>>(args, a->exc_keys, a->n_exc, a->exc_heads, a->n_exc_sites);
+    PFA_LAUNCH_CHECK(ctx);
+    return PFA_OK;
+}
+
+// after the scan kernel: check its launch, then commit the exchange it feeds (x, commit) -- whose escape kernel went first, so
+// that the scan's last block sees the complete shard vector -- or, without an exchange, run the escape kernel now
+template <class Args>
+int pfa_scan_done(pfa_aln* a, pfa_xchg* x, bool commit, void (*escape)(Args, const unsigned long long*, int64_t, const int64_t*, int64_t),
+                  const Args& args) {
+    PFA_LAUNCH_CHECK(a->ctx);
+    if (x && commit) pfa_xchg_commit(x);
+    if (!x && a->n_exc_sites > 0) return pfa_launch_escape(a, escape, args);
+    return PFA_OK;
+}

@@ -7,8 +7,8 @@ itself on the first:
   random  random ACGT text made on the device and encoded through from_device_ptr (incompressible: must not gain)
   allA    an all-A alignment (every line uniform)
 The vmm arm is the same mapping without compression: it separates page-size or mapping effects from compression.
---sweep adds passes per slot (PFA_SITE_TMA_M 1..4) x slots per warp (PFA_SITE_TMA 1, 2) for K2 on C4, and PFA_CDS_TMA_M 1..4
-for the codon scan (K4) on C3, pool against compressible planes.
+--sweep adds passes per slot (PFA_SITE_TMA_M 1..4) for K2 on C4, and PFA_CDS_TMA_M 1..4 for the codon scan (K4) on C3, pool
+against compressible planes.
 
   python scripts/probe_plane_compression.py [--reps 3] [--launches 10] [--sweep] [--small]
 """
@@ -128,17 +128,15 @@ def sweep(torch, stream, pf, ctx, args, n, L):
         alns[kind] = pf.Alignment.synthetic(ctx, n, L, 4)
     out = torch.zeros(alns["pool"].site_len(), dtype=torch.int64, device="cuda")
     for rep in range(2):
-        for slots in ("1", "2"):
-            for m in ("1", "2", "3", "4"):
-                os.environ["PFA_SITE_TMA"], os.environ["PFA_SITE_TMA_M"] = slots, m
-                line = []
-                for kind in ("pool", "compressible") if rep == 0 else ("compressible", "pool"):
-                    ms = time_launches(torch, stream, lambda: alns[kind].site_stats_device(out.data_ptr()), args.launches)
-                    line.append("%s %.3f" % (kind, ms))
-                print("  rep %d K2 slots=%s passes_per_slot=%s: %s  (%s)" % (rep, slots, m, "  ".join(line), ctx.last_kernel.split(" grid=")[1]))
-                sys.stdout.flush()
-    for k in ("PFA_SITE_TMA", "PFA_SITE_TMA_M"):
-        os.environ.pop(k)
+        for m in ("1", "2", "3", "4"):
+            os.environ["PFA_SITE_TMA_M"] = m
+            line = []
+            for kind in ("pool", "compressible") if rep == 0 else ("compressible", "pool"):
+                ms = time_launches(torch, stream, lambda: alns[kind].site_stats_device(out.data_ptr()), args.launches)
+                line.append("%s %.3f" % (kind, ms))
+            print("  rep %d K2 passes_per_slot=%s: %s  (%s)" % (rep, m, "  ".join(line), ctx.last_kernel.split(" grid=")[1]))
+            sys.stdout.flush()
+    os.environ.pop("PFA_SITE_TMA_M")
     for a in alns.values():
         a.free()
     ctx.trim()

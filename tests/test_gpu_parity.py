@@ -176,11 +176,13 @@ def _upper(mat):
 
 @pytest.mark.parametrize("p_junk", [0.0, 0.01])
 @pytest.mark.parametrize("n,L", [(1, 50), (2, 333), (31, 1000), (32, 999), (33, 1001), (127, 700), (128, 701), (129, 650),
-                                 (300, 5000), (1000, 6001), (2049, 3000), (5000, 1500), (10001, 600)])
+                                 (300, 5000), (1000, 6001), (2049, 3000), (5000, 1500), (10001, 600),
+                                 (300, 1), (300, 2), (300, 4), (2000, 1), (2000, 2), (2000, 4)])
 def test_against_c_oracle(ctx, n, L, p_junk):
     """seeded alignments of many shapes (word / chunk boundary cases for n), three overlapping populations.
     p_junk = 0: pure ACGT, i.e. the two-plane (HAS_V = false) instantiations every throughput figure is quoted on;
-    p_junk = 0.01: gaps / N / ? / IUPAC codes, the three-plane instantiations plus the escape kernels"""
+    p_junk = 0.01: gaps / N / ? / IUPAC codes, the three-plane instantiations plus the escape kernels.
+    L = 1, 2: codon shards without a whole codon column (only the trailing partial one) through the TMA codon scan"""
     rng = np.random.default_rng(n * 1000003 + L)
     text = _random_text(rng, n, L, p_junk=p_junk)
     up = _upper(text)
