@@ -598,8 +598,7 @@ __global__ void __launch_bounds__(256) pfa_batch_escape_kernel(const PfaBatchArg
         for (int q = 0; q < d.k; ++q) {
             const uint4* mq = a.masks + d.mask_off + (long long)q * Wq;
             uint32_t c[PFA_NCLASS];
-            pfa_class_counts<32, true>(a.b0 + d.plane_off + s * Wq, a.b1 + d.plane_off + s * Wq, a.v + d.plane_off + s * Wq, mq, Wq, lane,
-                                       0xffffffffu, c);
+            pfa_class_counts<true>(a.b0 + d.plane_off + s * Wq, a.b1 + d.plane_off + s * Wq, a.v + d.plane_off + s * Wq, mq, Wq, lane, c);
             if (c[PFA_C_ESC] == 0) continue;
             for (int b = lane; b < 256; b += 32) hist[wib][b] = 0u;
             __syncwarp();

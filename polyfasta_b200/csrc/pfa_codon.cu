@@ -9,12 +9,11 @@
 //   sum3_by_len[popc(mask)] += sum_{c in mask} 3*syncodfreq(c)       (:307, kept as exact integers)
 //   labels of the three positions from the sense codons of the mask  (:311, tables in constant memory)
 //   S_s/H_s and S_n/H_n: for each labelled position the FULL column's n^2 - sum_a c_a^2 (:169-170)
-// A group of LPS lanes owns one codon column (three consecutive site records).  Pass 1 proves, with logic ops
+// A warp owns one codon column (three consecutive site records).  Pass 1 proves, with logic ops
 // only, that all three sites are monomorphic over the union of the populations -- then every population sees
 // the same single codon and the contribution is uniform.  Otherwise pass 2 builds the presence mask per
 // population by peeling distinct codons off each 32-row word, and counts the three columns with popcounts.
 #include <algorithm>
-#include <cstdlib>
 
 #include "pfa_batch.cuh"
 #include "pfa_codon_rules.h"
@@ -103,18 +102,18 @@ __device__ __forceinline__ int pfa_labels_from_set(unsigned long long g) {
     return lab[0] | (lab[1] << 2) | (lab[2] << 4);
 }
 
-// presence mask of clean codons among the rows of one population, OR-reduced over the group
-template <int LPS, bool HAS_V>
+// presence mask of clean codons among the rows of one population, OR-reduced over the warp
+template <bool HAS_V>
 __device__ __forceinline__ unsigned long long pfa_codon_presence(const uint4* __restrict__ b0, const uint4* __restrict__ b1,
                                                                   const uint4* __restrict__ v, int64_t site, int Wq,
-                                                                  const uint4* __restrict__ mq, int sub, unsigned gmask) {
+                                                                  const uint4* __restrict__ mq, int lane) {
     unsigned long long P = 0;
     const uint32_t* q0 = reinterpret_cast<const uint32_t*>(b0 + site * Wq);
     const uint32_t* q1 = reinterpret_cast<const uint32_t*>(b1 + site * Wq);
     const uint32_t* qv = reinterpret_cast<const uint32_t*>(v + site * Wq);
     const uint32_t* qm = reinterpret_cast<const uint32_t*>(mq);
     const int Wn = Wq * 4;
-    for (int j = sub; j < Wq; j += LPS) {
+    for (int j = lane; j < Wq; j += 32) {
 #pragma unroll
         for (int w = 0; w < 4; ++w) {
             const int o = j * 4 + w;
@@ -142,13 +141,8 @@ __device__ __forceinline__ unsigned long long pfa_codon_presence(const uint4* __
             }
         }
     }
-    if (LPS > 1) {
-        uint32_t lo = (uint32_t)P, hi = (uint32_t)(P >> 32);
-        lo = pfa_group_or<LPS>(lo, gmask);
-        hi = pfa_group_or<LPS>(hi, gmask);
-        P = ((unsigned long long)hi << 32) | lo;
-    }
-    return P;
+    const uint32_t lo = __reduce_or_sync(0xffffffffu, (uint32_t)P), hi = __reduce_or_sync(0xffffffffu, (uint32_t)(P >> 32));
+    return ((unsigned long long)hi << 32) | lo;
 }
 
 // everything one (codon column, population) contributes, given its presence mask and the class counts of its sites
@@ -198,7 +192,7 @@ __device__ __forceinline__ void pfa_cds_contribute_one(unsigned long long P, con
     if (labels) labels[site0 + tv] = (uint8_t)li;
 }
 
-template <int LPS, bool HAS_V>
+template <bool HAS_V>
 __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_cds_scan_kernel(const PfaCdsArgs a) {
     extern __shared__ unsigned long long smem[];  // [3] uniform + [k][PFA_CDS_LEN] when acc_in_smem
     const int nacc = 3 + (a.acc_in_smem ? a.s.k * PFA_CDS_LEN : 0);
@@ -207,14 +201,12 @@ __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_cds_scan_kernel(const Pf
     unsigned long long* sm_acc = smem + 3;
 
     const int lane = threadIdx.x & 31;
-    const int sub = lane & (LPS - 1);
-    const unsigned gmask = LPS == 32 ? 0xffffffffu : (((1u << LPS) - 1u) << (lane - sub));
-    const int64_t gid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / LPS;
-    const int64_t ngroups = (int64_t)gridDim.x * blockDim.x / LPS;
+    const int64_t wid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / 32;
+    const int64_t nwarps = (int64_t)gridDim.x * blockDim.x / 32;
     const int Wq = a.s.Wq;
     unsigned u_nstops = 0, u_missing = 0, u_sum3 = 0;  // contributions identical for every population
 
-    for (int64_t cc = gid; cc < a.ncf; cc += ngroups) {
+    for (int64_t cc = wid; cc < a.ncf; cc += nwarps) {
         const int64_t site0 = cc * 3;
         // ---- pass 1: are the three sites monomorphic over the union of the populations? ----
         uint32_t acc[3][6];
@@ -222,7 +214,7 @@ __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_cds_scan_kernel(const Pf
         for (int t = 0; t < 3; ++t)
 #pragma unroll
             for (int i = 0; i < 6; ++i) acc[t][i] = 0;
-        for (int j = sub; j < Wq; j += LPS) {
+        for (int j = lane; j < Wq; j += 32) {
             const uint4 m = __ldg(a.s.umask + j);
 #pragma unroll
             for (int t = 0; t < 3; ++t) {
@@ -246,7 +238,7 @@ __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_cds_scan_kernel(const Pf
         for (int t = 0; t < 3; ++t)
 #pragma unroll
             for (int i = 0; i < 6; ++i) f |= (acc[t][i] ? 1u : 0u) << (6 * t + i);
-        f = pfa_group_or<LPS>(f, gmask);
+        f = __reduce_or_sync(0xffffffffu, f);
         bool uniform = true, clean = true;
         int codon = 0;
 #pragma unroll
@@ -259,7 +251,7 @@ __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_cds_scan_kernel(const Pf
             codon = (codon << 2) | ((ft & 4u) ? 2 : 0) | ((ft & 1u) ? 1 : 0);
         }
         if (uniform) {
-            if (sub == 0) {
+            if (lane == 0) {
                 if (clean) {
                     u_nstops += (unsigned)((c_stop_mask >> codon) & 1ull);
                     u_sum3 += c_syn3[codon];
@@ -275,11 +267,11 @@ __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_cds_scan_kernel(const Pf
             uint32_t cnt[3][PFA_NCLASS];
 #pragma unroll
             for (int t = 0; t < 3; ++t)
-                pfa_class_counts<LPS, HAS_V>(a.s.b0 + (site0 + t) * Wq, a.s.b1 + (site0 + t) * Wq, a.s.v + (site0 + t) * Wq, mq, Wq,
-                                             sub, gmask, cnt[t]);
+                pfa_class_counts<HAS_V>(a.s.b0 + (site0 + t) * Wq, a.s.b1 + (site0 + t) * Wq, a.s.v + (site0 + t) * Wq, mq, Wq, lane,
+                                        cnt[t]);
             if (cnt[0][PFA_C_ESC] | cnt[1][PFA_C_ESC] | cnt[2][PFA_C_ESC]) continue;  // finished by pfa_cds_escape_kernel
-            const unsigned long long P = pfa_codon_presence<LPS, HAS_V>(a.s.b0, a.s.b1, a.s.v, site0, Wq, mq, sub, gmask);
-            if (sub != 0) continue;
+            const unsigned long long P = pfa_codon_presence<HAS_V>(a.s.b0, a.s.b1, a.s.v, site0, Wq, mq, lane);
+            if (lane != 0) continue;
             const uint32_t escd[3] = {0, 0, 0};
             const unsigned long long escsq[3] = {0, 0, 0};
             unsigned long long* dst = a.acc_in_smem ? sm_acc + q * PFA_CDS_LEN
@@ -1156,26 +1148,19 @@ __global__ void __launch_bounds__(256) pfa_cds_escape_kernel(const PfaCdsArgs a,
             uint32_t cnt[3][PFA_NCLASS];
 #pragma unroll
             for (int t = 0; t < 3; ++t)
-                pfa_class_counts<32, true>(a.s.b0 + (site0 + t) * Wq, a.s.b1 + (site0 + t) * Wq, a.s.v + (site0 + t) * Wq, mq, Wq, lane,
-                                           0xffffffffu, cnt[t]);
+                pfa_class_counts<true>(a.s.b0 + (site0 + t) * Wq, a.s.b1 + (site0 + t) * Wq, a.s.v + (site0 + t) * Wq, mq, Wq, lane, cnt[t]);
             if (!(cnt[0][PFA_C_ESC] | cnt[1][PFA_C_ESC] | cnt[2][PFA_C_ESC])) continue;  // the main kernel counted it
             uint32_t escd[3] = {0, 0, 0};
             unsigned long long escsq[3] = {0, 0, 0};
             for (int t = 0; t < 3; ++t)
                 if (cnt[t][PFA_C_ESC])
                     pfa_escape_stats(keys, seg0[t], seg1[t], reinterpret_cast<const uint32_t*>(mq), hist[wib], lane, &escd[t], &escsq[t]);
-            const unsigned long long P = pfa_codon_presence<32, true>(a.s.b0, a.s.b1, a.s.v, site0, Wq, mq, lane, 0xffffffffu);
+            const unsigned long long P = pfa_codon_presence<true>(a.s.b0, a.s.b1, a.s.v, site0, Wq, mq, lane);
             if (lane != 0) continue;
             pfa_cds_contribute(P, cnt, a.s.pop_n[q], escd, escsq, reinterpret_cast<unsigned long long*>(a.out + (int64_t)q * PFA_CDS_LEN),
                                a.labels ? a.labels + (int64_t)q * a.s.ns : nullptr, site0);
         }
     }
-}
-
-template <int LPS>
-static void launch_cds(const PfaCdsArgs& args, bool has_v, dim3 grid, size_t smem, cudaStream_t st) {
-    if (has_v) pfa_cds_scan_kernel<LPS, true><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
-    else pfa_cds_scan_kernel<LPS, false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
 }
 
 int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg* x) {
@@ -1211,12 +1196,8 @@ int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg*
     int lps = 1;
     while (lps < 32 && (a->Wq + lps - 1) / lps > 2) lps *= 2;
     const int iter = (a->Wq + lps - 1) / lps;
-    const bool hv = pfa_scan_has_v(a), multi = a->k > 1;
-    const bool generic = iter > 3 || getenv("PFA_GENERIC_SCAN") != nullptr;
-    if (generic) {
-        lps = 1;
-        while (lps < 32 && (a->Wq + lps - 1) / lps > 4) lps *= 2;
-    }
+    const bool hv = a->has_invalid != 0, multi = a->k > 1;
+    const bool generic = iter > 3;  // lps = 32: records of more than 96 chunks (n > 12,288) stream through one warp per column
     const char* planes = pfa_plane_alloc_name(a->plane_alloc);
     cudaStream_t st = ctx->stream;
     if (x) {  // escape columns first: the scan kernel's last block runs the exchange over the complete shard vector
@@ -1252,16 +1233,10 @@ int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg*
         return pfa_scan_done(a, x, true, pfa_cds_escape_kernel, args);
     }
     args.s.x.wide = 0;  // see pfa_launch_site_scan
-    const int64_t groups_per_block = PFA_SITE_THREADS / lps;
-    const dim3 grid((unsigned)std::min<int64_t>((std::max<int64_t>(args.ncf, 1) + groups_per_block - 1) / groups_per_block, (int64_t)ctx->sm_count * 4));
-    switch (lps) {
-        case 1: launch_cds<1>(args, hv, grid, smem, st); break;
-        case 2: launch_cds<2>(args, hv, grid, smem, st); break;
-        case 4: launch_cds<4>(args, hv, grid, smem, st); break;
-        case 8: launch_cds<8>(args, hv, grid, smem, st); break;
-        case 16: launch_cds<16>(args, hv, grid, smem, st); break;
-        default: launch_cds<32>(args, hv, grid, smem, st); break;
-    }
+    const int64_t warps_per_block = PFA_SITE_THREADS / 32;
+    const dim3 grid((unsigned)std::min<int64_t>((std::max<int64_t>(args.ncf, 1) + warps_per_block - 1) / warps_per_block, (int64_t)ctx->sm_count * 4));
+    if (hv) pfa_cds_scan_kernel<true><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
+    else pfa_cds_scan_kernel<false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
     pfa_note_kernel(ctx, "pfa_cds_scan_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d planes=%s", lps, iter, (int)hv, (int)multi, grid.x,
                     PFA_SITE_THREADS, planes);
     return pfa_scan_done(a, x, true, pfa_cds_escape_kernel, args);
@@ -1369,14 +1344,14 @@ __global__ void __launch_bounds__(256) pfa_batch_cds_escape_kernel(const PfaBatc
             uint32_t cnt[3][PFA_NCLASS];
 #pragma unroll
             for (int t = 0; t < 3; ++t)
-                pfa_class_counts<32, true>(p0 + (site0 + t) * Wq, p1 + (site0 + t) * Wq, pv + (site0 + t) * Wq, mq, Wq, lane, 0xffffffffu, cnt[t]);
+                pfa_class_counts<true>(p0 + (site0 + t) * Wq, p1 + (site0 + t) * Wq, pv + (site0 + t) * Wq, mq, Wq, lane, cnt[t]);
             if (!(cnt[0][PFA_C_ESC] | cnt[1][PFA_C_ESC] | cnt[2][PFA_C_ESC])) continue;  // the main kernel counted it
             uint32_t escd[3] = {0, 0, 0};
             unsigned long long escsq[3] = {0, 0, 0};
             for (int t = 0; t < 3; ++t)
                 if (cnt[t][PFA_C_ESC])
                     pfa_escape_stats(keys, seg0[t], seg1[t], reinterpret_cast<const uint32_t*>(mq), hist[wib], lane, &escd[t], &escsq[t]);
-            const unsigned long long P = pfa_codon_presence<32, true>(p0, p1, pv, site0, Wq, mq, lane, 0xffffffffu);
+            const unsigned long long P = pfa_codon_presence<true>(p0, p1, pv, site0, Wq, mq, lane);
             if (lane != 0) continue;
             pfa_cds_contribute(P, cnt, a.popn[d.pop_base + q], escd, escsq, reinterpret_cast<unsigned long long*>(a.cds_out + (d.pop_base + q) * PFA_CDS_LEN),
                                nullptr, site0);

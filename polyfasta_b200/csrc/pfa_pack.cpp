@@ -8,7 +8,6 @@
 // travels as text instead (gaps, N, IUPAC codes need the validity plane and the exception list of K1).
 #include <immintrin.h>
 #include <stdint.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
@@ -32,8 +31,6 @@ struct Lut {
     }
 };
 const Lut g_lut;
-const int64_t kPrefetchAhead = getenv("PFA_PACK_PREFETCH") ? atoi(getenv("PFA_PACK_PREFETCH")) : 0;  // bytes ahead of the loads
-const bool g_stream_stores = getenv("PFA_PACK_NT") ? atoi(getenv("PFA_PACK_NT")) != 0 : false;
 
 int pack_scalar(const uint8_t* src, int64_t cols, uint8_t* dst) {
     unsigned bad = 0;
@@ -87,27 +84,7 @@ __attribute__((target("avx512f,avx512bw,avx512vl"))) int pack_avx512(const uint8
     const __m512i w14 = _mm512_set1_epi16(0x0401), w116 = _mm512_set1_epi32(0x00100001);
     __mmask64 ok = ~0ull;
     int64_t i = 0;
-    if (g_stream_stores && (reinterpret_cast<uintptr_t>(dst) & 63) == 0) {
-        // 256 bases -> one 64-byte line, written with a non-temporal store (no read-for-ownership of the staging buffer)
-        for (; i + 256 <= cols; i += 256) {
-            __m512i line = _mm512_undefined_epi32();
-#pragma GCC unroll 4
-            for (int u = 0; u < 4; ++u) {
-                const __m512i x = _mm512_loadu_si512(src + i + 64 * u);
-                const __m512i c = _mm512_and_si512(_mm512_srli_epi16(x, 1), three);
-                ok &= _mm512_cmpeq_epi8_mask(_mm512_shuffle_epi8(letters, c), _mm512_and_si512(x, fold));
-                const __m128i p = _mm512_cvtepi32_epi8(_mm512_madd_epi16(_mm512_maddubs_epi16(c, w14), w116));
-                line = u == 0 ? _mm512_castsi128_si512(p) : _mm512_inserti32x4(line, p, u);
-            }
-            _mm512_stream_si512(reinterpret_cast<__m512i*>(dst + (i >> 2)), line);
-        }
-        _mm_sfence();
-    }
     for (; i + 128 <= cols; i += 128) {  // two vectors per iteration: independent chains
-        if (kPrefetchAhead) {  // helps a lone packer (+10 %), hurts next to the copy engine's reads: off by default
-            _mm_prefetch(reinterpret_cast<const char*>(src + i + kPrefetchAhead), _MM_HINT_T0);
-            _mm_prefetch(reinterpret_cast<const char*>(src + i + kPrefetchAhead + 64), _MM_HINT_T0);
-        }
         const __m512i x0 = _mm512_loadu_si512(src + i), x1 = _mm512_loadu_si512(src + i + 64);
         const __m512i c0 = _mm512_and_si512(_mm512_srli_epi16(x0, 1), three), c1 = _mm512_and_si512(_mm512_srli_epi16(x1, 1), three);
         ok &= _mm512_cmpeq_epi8_mask(_mm512_shuffle_epi8(letters, c0), _mm512_and_si512(x0, fold));

@@ -4,11 +4,11 @@
 // wattersons_theta (:494-497) and getsfs (:274-282): one pass over the planes yields, for every population at
 // once, S = #columns with > 1 distinct character, H = sum_cols (n^2 - sum_a c_a^2) and the folded SFS.
 //
-// A group of LPS lanes owns one site; its lanes stride over the Wq 128-bit chunks of the site record.
+// A warp owns one site; its lanes stride over the Wq 128-bit chunks of the site record.
 // Pass 1 (every site, 2 or 3 coalesced 128-bit loads per chunk, logic ops only) decides whether all rows
 // of the union of the populations carry the same symbol.  Monomorphic sites -- the overwhelming majority of
 // a real alignment -- end there.  Pass 2 (variable sites only; re-reads the record from L1/L2) counts the
-// symbol classes per population with popcounts and group shuffles.  Sites holding "escape" symbols (IUPAC
+// symbol classes per population with popcounts and warp reductions.  Sites holding "escape" symbols (IUPAC
 // codes etc., which are distinct alleles in the reference) are finished by pfa_escape_sites_kernel from the
 // sorted exception list.
 #include <cstdio>
@@ -16,7 +16,7 @@
 
 #include "pfa_sites.cuh"
 
-template <int LPS, bool HAS_V>
+template <bool HAS_V>
 __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_site_scan_kernel(const PfaSiteArgs a) {
     extern __shared__ unsigned long long smem[];
     if (a.x.world && blockIdx.x == 0 && threadIdx.x == 0) a.x.stamps[5] = pfa_globaltimer();
@@ -29,20 +29,18 @@ __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_site_scan_kernel(const P
     __syncthreads();
 
     const int lane = threadIdx.x & 31;
-    const int sub = lane & (LPS - 1);
-    const unsigned gmask = LPS == 32 ? 0xffffffffu : (((1u << LPS) - 1u) << (lane - sub));
-    const int64_t gid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / LPS;
-    const int64_t ngroups = (int64_t)gridDim.x * blockDim.x / LPS;
+    const int64_t wid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / 32;
+    const int64_t nwarps = (int64_t)gridDim.x * blockDim.x / 32;
     const int Wq = a.Wq;
 
-    for (int64_t s = gid; s < a.ns; s += ngroups) {
+    for (int64_t s = wid; s < a.ns; s += nwarps) {
         const uint4* p0 = a.b0 + s * Wq;
         const uint4* p1 = a.b1 + s * Wq;
         const uint4* pv = a.v + s * Wq;
         // ---- pass 1: is the column monomorphic over the union of the populations? ----
         uint32_t o0 = 0, z0 = 0, o1 = 0, z1 = 0, ov = 0, zv = 0;
 #pragma unroll 2
-        for (int j = sub; j < Wq; j += LPS) {
+        for (int j = lane; j < Wq; j += 32) {
             const uint4 m = __ldg(a.umask + j);
             const uint4 x0 = pfa_ld_stream(p0 + j);
             const uint4 x1 = pfa_ld_stream(p1 + j);
@@ -59,19 +57,19 @@ __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_site_scan_kernel(const P
             }
         }
         unsigned f = (o0 ? 1u : 0u) | (z0 ? 2u : 0u) | (o1 ? 4u : 0u) | (z1 ? 8u : 0u) | (ov ? 16u : 0u) | (zv ? 32u : 0u);
-        f = pfa_group_or<LPS>(f, gmask);
+        f = __reduce_or_sync(0xffffffffu, f);
         const bool mono = ((f & 3u) != 3u) && ((f & 12u) != 12u) && ((f & 48u) != 48u);
         const bool all_escape = (f & 1u) && (f & 4u) && !(f & 16u);  // every row shows the escape class
         if (mono && !all_escape) {
-            if (a.isvar && sub == 0)
+            if (a.isvar && lane == 0)
                 for (int q = 0; q < a.k; ++q) a.isvar[(int64_t)q * a.ns + s] = 0;
             continue;
         }
         // ---- pass 2: class counts per population ----
         for (int q = 0; q < a.k; ++q) {
             uint32_t c[PFA_NCLASS];
-            pfa_class_counts<LPS, HAS_V>(p0, p1, pv, a.masks + (int64_t)q * Wq, Wq, sub, gmask, c);
-            if (sub != 0) continue;
+            pfa_class_counts<HAS_V>(p0, p1, pv, a.masks + (int64_t)q * Wq, Wq, lane, c);
+            if (lane != 0) continue;
             const int64_t nq = a.pop_n[q];
             PfaSiteResult r = pfa_site_result(c, nq, 0u, 0ull);
             if (r.has_escape) continue;  // finished by pfa_escape_sites_kernel
@@ -325,7 +323,7 @@ __global__ void __launch_bounds__(256) pfa_escape_sites_kernel(const PfaSiteArgs
         const uint4* pv = a.v + s * a.Wq;
         for (int q = 0; q < a.k; ++q) {
             uint32_t c[PFA_NCLASS];
-            pfa_class_counts<32, true>(p0, p1, pv, a.masks + (int64_t)q * a.Wq, a.Wq, lane, 0xffffffffu, c);
+            pfa_class_counts<true>(p0, p1, pv, a.masks + (int64_t)q * a.Wq, a.Wq, lane, c);
             if (c[PFA_C_ESC] == 0) continue;  // warp-uniform: the main kernel already counted this (site, pop)
             for (int b = lane; b < 256; b += 32) hist[wib][b] = 0u;
             __syncwarp();
@@ -683,14 +681,6 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
     if (a.x.world) pfa_xchg_epilogue(a.x);
 }
 
-template <int LPS>
-static void launch_scan(const PfaSiteArgs& args, bool has_v, dim3 grid, size_t smem, cudaStream_t st) {
-    if (has_v) pfa_site_scan_kernel<LPS, true><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
-    else pfa_site_scan_kernel<LPS, false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
-}
-
-bool pfa_scan_has_v(const pfa_aln* a) { return a->has_invalid != 0 || getenv("PFA_PROBE_SPARSE_V") != nullptr; }
-
 int pfa_tma_plan(pfa_aln* a, const PfaTmaShape& s, PfaTmaPlan* p) {
     pfa_ctx* ctx = a->ctx;
     const char* m_env = getenv(s.m_env);
@@ -769,8 +759,8 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
     while (lps < 32 && (a->Wq + lps - 1) / lps > 5) lps *= 2;
     const int iter = (a->Wq + lps - 1) / lps;
     const size_t smem = sizeof(unsigned long long) * 2 * (size_t)a->k + (args.sfs_in_smem ? sizeof(unsigned int) * (size_t)args.sfs_bins : 0);
-    const bool hv = pfa_scan_has_v(a), multi = a->k > 1;
-    const bool generic = iter > 5 || getenv("PFA_GENERIC_SCAN") != nullptr;
+    const bool hv = a->has_invalid != 0, multi = a->k > 1;
+    const bool generic = iter > 5;  // lps = 32: records of more than 160 chunks (n > 20,480) stream through one warp per site
     const char* planes = pfa_plane_alloc_name(a->plane_alloc);
     cudaStream_t st = ctx->stream;
     // The TMA variant: one CTA of 512 threads per SM, every warp fed by cp.async.bulk through its own shared-memory slot of
@@ -811,14 +801,8 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
     const int64_t blocks = std::min<int64_t>((a->ns + groups_per_block - 1) / groups_per_block, (int64_t)ctx->sm_count * (generic ? 4 : 2));
     const dim3 grid((unsigned)blocks);
     if (generic) {
-        switch (lps) {
-            case 1: launch_scan<1>(args, hv, grid, smem, st); break;
-            case 2: launch_scan<2>(args, hv, grid, smem, st); break;
-            case 4: launch_scan<4>(args, hv, grid, smem, st); break;
-            case 8: launch_scan<8>(args, hv, grid, smem, st); break;
-            case 16: launch_scan<16>(args, hv, grid, smem, st); break;
-            default: launch_scan<32>(args, hv, grid, smem, st); break;
-        }
+        if (hv) pfa_site_scan_kernel<true><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
+        else pfa_site_scan_kernel<false><<<grid, PFA_SITE_THREADS, smem, st>>>(args);
     } else {
         const bool found = pfa_for_shape<1, 4, 1, 5, 2, 3, 2, 4, 2, 5>(lps, iter, [&](auto L, auto I) {
             pfa_for_v_multi(hv, multi, [&](auto V, auto M) {
@@ -835,9 +819,10 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
 
 // ---- measurement aid: how fast can this GPU READ the planes at all? -------------------------------------------------------
 // The same streaming 128-bit loads as K2 over the same bytes, nothing else (XOR into a register, one store per thread that
-// never happens in practice).  bench.py reports K2 against this read-only ceiling next to the read+write copy peak.
-template <int UNROLL>
+// never happens in practice), 8 loads in flight per thread.  bench.py reports K2 against this read-only ceiling next to the
+// read+write copy peak.
 __global__ void __launch_bounds__(256) pfa_read_probe_kernel(const uint4* __restrict__ p, int64_t n16, unsigned int* __restrict__ sink) {
+    constexpr int UNROLL = 8;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     uint4 acc = make_uint4(0, 0, 0, 0);
@@ -857,45 +842,6 @@ __global__ void __launch_bounds__(256) pfa_read_probe_kernel(const uint4* __rest
     if ((acc.x ^ acc.y ^ acc.z ^ acc.w) == 0x9e3779b9u && acc.x == 0x7f4a7c15u) *sink = acc.x;
 }
 
-// the same bytes through the bulk-copy engine (TMA, cp.async.bulk) into a ring of shared-memory stages, one CTA per SM:
-// bytes in flight are bounded by shared memory (stages x stage size), not by registers
-__global__ void __launch_bounds__(256, 1) pfa_read_probe_tma_kernel(const unsigned char* __restrict__ p, int64_t bytes, int stages,
-                                                                    int stage_bytes, unsigned int* __restrict__ sink) {
-    extern __shared__ __align__(128) unsigned char ring[];
-    __shared__ uint64_t full[16];
-    const int64_t nblk = (bytes + stage_bytes - 1) / stage_bytes;
-    const int64_t mine = blockIdx.x < nblk ? (nblk - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < stages; ++s) pfa_mbar_init(&full[s], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    auto issue = [&](int64_t k) {
-        const int64_t off = ((int64_t)blockIdx.x + k * gridDim.x) * stage_bytes;
-        const unsigned len = (unsigned)min((int64_t)stage_bytes, bytes - off);
-        const int s = (int)(k % stages);
-        pfa_mbar_expect_tx(&full[s], len);
-        pfa_bulk_load(ring + (size_t)s * stage_bytes, p + off, len, &full[s]);
-    };
-    if (threadIdx.x == 0)
-        for (int64_t k = 0; k < mine && k < stages; ++k) issue(k);
-    uint4 acc = make_uint4(0, 0, 0, 0);
-    for (int64_t k = 0; k < mine; ++k) {
-        const int s = (int)(k % stages);
-        pfa_mbar_wait(&full[s], (unsigned)((k / stages) & 1));
-        const int64_t off = ((int64_t)blockIdx.x + k * gridDim.x) * stage_bytes;
-        const int n16 = (int)(min((int64_t)stage_bytes, bytes - off) / 16);
-        const uint4* q = reinterpret_cast<const uint4*>(ring + (size_t)s * stage_bytes);
-        for (int i = threadIdx.x; i < n16; i += blockDim.x) {
-            const uint4 x = q[i];
-            acc.x ^= x.x; acc.y ^= x.y; acc.z ^= x.z; acc.w ^= x.w;
-        }
-        __syncthreads();
-        if (threadIdx.x == 0 && k + stages < mine) issue(k + stages);
-    }
-    if ((acc.x ^ acc.y ^ acc.z ^ acc.w) == 0x9e3779b9u && acc.x == 0x7f4a7c15u) *sink = acc.x;
-}
-
 extern "C" int pfa_aln_read_probe(pfa_aln* a, int planes, int reps, double* ms_per_pass) {
     if (!a || !ms_per_pass || planes < 1 || planes > 3 || reps < 1) return PFA_ERR_ARG;
     pfa_ctx* ctx = a->ctx;
@@ -906,26 +852,8 @@ extern "C" int pfa_aln_read_probe(pfa_aln* a, int planes, int reps, double* ms_p
     PFA_CUDA(ctx, cudaEventCreate(&e0));
     PFA_CUDA(ctx, cudaEventCreate(&e1));
     const int64_t n16 = (int64_t)(a->plane_bytes / 16) * planes;  // b0 | b1 | v are one allocation
-    // PFA_PROBE="<blocks per SM>,<loads in flight per thread>" (experiments); default 8 CTAs x 8 loads of 16 bytes
-    int bps = 8, unroll = 8;
-    if (const char* e = getenv("PFA_PROBE")) sscanf(e, "%d,%d", &bps, &unroll);
-    const unsigned grid = (unsigned)ctx->sm_count * (unsigned)std::max(1, bps);
-    int tma_stages = 0, tma_kb = 0;
-    if (const char* e = getenv("PFA_PROBE_TMA")) sscanf(e, "%d,%d", &tma_stages, &tma_kb);  // "<stages>,<KB per stage>"
-    if (tma_stages > 0) {
-        tma_stages = std::min(tma_stages, 16);
-        const size_t smem = (size_t)tma_stages * tma_kb * 1024;
-        cudaError_t ea = cudaFuncSetAttribute(pfa_read_probe_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (ea != cudaSuccess) return pfa_fail(ctx, PFA_ERR_CUDA, "read probe: %s", cudaGetErrorString(ea));
-    }
-    auto launch = [&]() {
-        if (tma_stages > 0)
-            pfa_read_probe_tma_kernel<<<(unsigned)ctx->sm_count, 256, (size_t)tma_stages * tma_kb * 1024, ctx->stream>>>(
-                reinterpret_cast<const unsigned char*>(a->planes), n16 * 16, tma_stages, tma_kb * 1024, sink);
-        else if (unroll >= 16) pfa_read_probe_kernel<16><<<grid, 256, 0, ctx->stream>>>(a->planes, n16, sink);
-        else if (unroll <= 4) pfa_read_probe_kernel<4><<<grid, 256, 0, ctx->stream>>>(a->planes, n16, sink);
-        else pfa_read_probe_kernel<8><<<grid, 256, 0, ctx->stream>>>(a->planes, n16, sink);
-    };
+    const unsigned grid = (unsigned)ctx->sm_count * 8u;           // 8 CTAs per SM
+    auto launch = [&]() { pfa_read_probe_kernel<<<grid, 256, 0, ctx->stream>>>(a->planes, n16, sink); };
     launch();  // warm-up
     cudaEventRecord(e0, ctx->stream);
     for (int r = 0; r < reps; ++r) launch();

@@ -65,14 +65,14 @@ __device__ __forceinline__ uint32_t pfa_group_add(uint32_t x, unsigned gmask) {
     return x;
 }
 
-// counts of the seven packed classes among the rows of one population at one site, summed over the group
-template <int LPS, bool HAS_V>
+// counts of the seven packed classes among the rows of one population at one site, summed over the warp
+template <bool HAS_V>
 __device__ __forceinline__ void pfa_class_counts(const uint4* __restrict__ p0, const uint4* __restrict__ p1,
                                                  const uint4* __restrict__ pv, const uint4* __restrict__ mq, int Wq,
-                                                 int sub, unsigned gmask, uint32_t c[PFA_NCLASS]) {
+                                                 int lane, uint32_t c[PFA_NCLASS]) {
 #pragma unroll
     for (int i = 0; i < PFA_NCLASS; ++i) c[i] = 0;
-    for (int j = sub; j < Wq; j += LPS) {
+    for (int j = lane; j < Wq; j += 32) {
         const uint4 m4 = __ldg(mq + j), a4 = __ldg(p0 + j), b4 = __ldg(p1 + j);
         uint4 v4 = m4;
         if (HAS_V) v4 = __ldg(pv + j);
@@ -95,11 +95,9 @@ __device__ __forceinline__ void pfa_class_counts(const uint4* __restrict__ p0, c
             }
         }
     }
-    if (LPS > 1) {
 #pragma unroll
-        for (int i = 0; i < PFA_NCLASS; ++i)
-            if (HAS_V || i < 4) c[i] = pfa_group_add<LPS>(c[i], gmask);
-    }
+    for (int i = 0; i < PFA_NCLASS; ++i)
+        if (HAS_V || i < 4) c[i] = __reduce_add_sync(0xffffffffu, c[i]);
 }
 
 struct PfaSiteResult {
@@ -385,9 +383,6 @@ void pfa_fill_site_args(const pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, PfaS
 int pfa_aln_flagged_sites(pfa_aln* a, int64_t* out);
 
 // ---- launch plan of the TMA scans (K2, K4) -----------------------------------------------------------------------------------
-// does a scan of this shard read the validity plane?  (PFA_PROBE_SPARSE_V: the validity-aware kernels on a clean shard)
-bool pfa_scan_has_v(const pfa_aln* a);
-
 // what the site scan (a unit = one site record) and the codon scan (a unit = a codon column, three site records) tell the planner
 struct PfaTmaShape {
     int recs;           // site records per unit; a slot's validity area holds at least one unit
@@ -400,7 +395,7 @@ struct PfaTmaShape {
                         // with at most 1/d^2 of the sites flagged
     int m_raise;        // a v area below a whole slot raises m to m + ceil(m * m_raise / 2) (no m_env)
     size_t smem;        // shared memory beyond the slots and their mbarriers: accumulators, queues
-    bool has_v;         // pfa_scan_has_v
+    bool has_v;         // the scan reads the validity plane (pfa_aln::has_invalid)
 };
 struct PfaTmaPlan {
     bool sparse_v;          // fetch only the flagged cells of the v plane (PfaSiteArgs::vflag)

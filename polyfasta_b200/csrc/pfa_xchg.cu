@@ -46,8 +46,7 @@ int pfa_xchg_fill(pfa_xchg* x, int64_t len, int64_t* d_out, PfaXchgDev* dev, boo
     dev->epoch = x->epoch;
     dev->len = (int)len;
     dev->zero_len = x->high_water;
-    static const bool wide_off = getenv("PFA_XCHG_WIDE") && atoi(getenv("PFA_XCHG_WIDE")) == 0;
-    dev->wide = coresident && x->distinct_devices && x->world > 1 && !wide_off;
+    dev->wide = coresident && x->distinct_devices && x->world > 1;
     dev->cap = x->cap;
     dev->timeout_ns = x->timeout_ns;
     dev->partial = x->partial;

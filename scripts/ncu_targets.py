@@ -18,17 +18,6 @@ if which == "k4":
         aln.cds_stats_device(out.data_ptr())
     ctx.sync()
     print("k4", out[:6].tolist())
-elif which == "k2v":
-    # the site scan on a clean 2000 x 3 Mb shard: the pure kernel twice, then the validity-aware kernel (no flag set) twice
-    aln = pf.Alignment.synthetic(ctx, 2000, 3_000_000, 3)
-    out = torch.zeros(aln.site_len(), dtype=torch.int64, device="cuda")
-    for probe in (False, False, True, True):
-        os.environ.pop("PFA_PROBE_SPARSE_V", None)
-        if probe:
-            os.environ["PFA_PROBE_SPARSE_V"] = "1"
-        aln.site_stats_device(out.data_ptr())
-        ctx.sync()
-    print("k2v", out[:2].tolist())
 elif which == "k2g":
     # the site scan with sparse gaps: 2000 x 3 Mb at 10 gaps per 10^6 bases, then 10000 x 2 Mb at 100
     for n, L, ppm in ((2000, 3_000_000, 10), (10000, 2_000_000, 100)):

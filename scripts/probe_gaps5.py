@@ -25,8 +25,6 @@ with torch.cuda.stream(stream):
             aln = pf.Alignment.synthetic(ctx, n, L, 4)
             if ppm:
                 aln.poke_gaps(4, ppm)
-            else:
-                os.environ["PFA_PROBE_SPARSE_V"] = "1"
             out = torch.zeros(aln.site_len(), dtype=torch.int64, device="cuda")
             cds = torch.zeros(71, dtype=torch.int64, device="cuda")
             row = []
@@ -41,6 +39,5 @@ with torch.cuda.stream(stream):
                 k4 = timed(lambda: aln.cds_stats_device(cds.data_ptr()))
                 kn4 = ctx.last_kernel.split("passes_per_slot=")[1]
                 row.append("compact=%s K2 %.3f [m=%s] K4 %.3f [m=%s]" % (compact, k2, kn2.replace(" v_records_per_slot=", " vs="), k4, kn4.replace(" v_records_per_slot=", " vs=")))
-            os.environ.pop("PFA_PROBE_SPARSE_V", None)
             print("%d x %d %3d ppm: %s" % (n, L, ppm, " | ".join(row)), flush=True)
             aln.free()

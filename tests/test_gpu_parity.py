@@ -518,13 +518,11 @@ def test_large_file_rows_in_place(ctx, tmp_path, monkeypatch):
 
 
 @pytest.mark.parametrize("p_junk", [0.0, 0.01])
-@pytest.mark.parametrize("n,L,force", [(129, 1500, True), (2049, 900, True), (21000, 240, False), (13000, 303, False)])
-def test_streaming_scan_kernels(ctx, monkeypatch, n, L, force, p_junk):
-    """alignments with more rows than the register-resident kernels hold (K2: 20,480, K4: 12,288) go through the streaming
-    two-pass kernels; PFA_GENERIC_SCAN=1 forces them for smaller shapes.  Same checks as test_against_c_oracle, plus the
-    exchange epilogue (world = 1) on this path."""
-    if force:
-        monkeypatch.setenv("PFA_GENERIC_SCAN", "1")
+@pytest.mark.parametrize("n,L", [(21000, 240), (13000, 303)])
+def test_streaming_scan_kernels(ctx, n, L, p_junk):
+    """alignments with more rows than the TMA kernels take (K2: 20,480, K4: 12,288) go through the streaming two-pass
+    kernels, one warp per site or codon column.  Same checks as test_against_c_oracle, plus the exchange epilogue
+    (world = 1) on this path."""
     rng = np.random.default_rng(n + 7 * L)
     text = _random_text(rng, n, L, p_junk=p_junk)
     up = _upper(text)
