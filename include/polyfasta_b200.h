@@ -112,6 +112,7 @@ int pfa_synth_text_device(pfa_ctx* ctx, uint8_t* d_text, int64_t ld, int64_t n, 
 int pfa_aln_free(pfa_aln* a);
 int64_t pfa_aln_nseq(const pfa_aln* a);
 int64_t pfa_aln_nsites(const pfa_aln* a);        /* sites in this shard */
+int64_t pfa_aln_total_sites(const pfa_aln* a);   /* sites of the whole alignment the shard belongs to */
 int64_t pfa_aln_num_escapes(const pfa_aln* a);   /* entries in the exception list */
 int64_t pfa_aln_packed_bytes(const pfa_aln* a);  /* bytes of the three planes */
 int pfa_aln_has_invalid(const pfa_aln* a);       /* any non-ACGT symbol in the shard */
@@ -147,6 +148,11 @@ int64_t pfa_site_offset(const pfa_aln* a, int pop);
 int pfa_site_stats_device(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar);
 /* synchronous convenience: same, copied to host memory */
 int pfa_site_stats(pfa_aln* a, int64_t* out, uint8_t* isvar /* host, optional */);
+/* the same with the per-site H: d_hsite (optional, may be NULL) int64 [k][nsites], n^2 - sum_a c_a^2 of the column in that
+ * population where it is variable, 0 elsewhere (so isvar == (hsite > 0)); zero-filled by the call.  The kernels and launch
+ * plan are those of pfa_site_stats_device. */
+int pfa_site_stats_hsite_device(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, int64_t* d_hsite);
+int pfa_site_stats_hsite(pfa_aln* a, int64_t* out, uint8_t* isvar /* host, optional */, int64_t* hsite /* host, optional */);
 
 /* ---- K4 codon scan: replaces getvarCDSsites + get_syn_nonsyn_cod_sites + the var-site matching
  *      (PolyFastA.py:165-170, 284-434) ------------------------------------------------------------------ */
@@ -285,6 +291,22 @@ typedef struct pfa_final_out {
 int pfa_finalize(pfa_ctx* ctx, const pfa_final_in* in, pfa_final_out* out, int count);
 /* synonymous-site count from the integer accumulators: sum_l sum3_by_len[l] / (3 l), fp64 on the device */
 int pfa_cds_ssites(pfa_ctx* ctx, const int64_t* cds_out /* [count][PFA_CDS_LEN] host */, double* ssites, int count);
+
+/* ---- sliding windows along the alignment (beyond the reference: pi, theta and D per window) -------------------------------
+ * Window i covers the global columns [i*step, min(i*step + window, L)), i = 0 .. pfa_window_count(L, window, step) - 1:
+ * windows start at 0, step, 2*step, ...; the first one that reaches the end of the alignment is truncated to L and is the last;
+ * step > window skips the columns between windows.  A window's (S, H) are what pfa_site_stats returns for the alignment cut to
+ * the window's columns, and its pi / theta / D what K5 returns for (n, S, H, seqlen = window length, jc). */
+/* number of windows (no GPU needed): min(1 + ceil(max(0, L - window) / step), ceil(L / step)), 0 for L = 0; -1 when
+ * L < 0, window < 1 or step < 1 */
+int64_t pfa_window_count(int64_t L, int64_t window, int64_t step);
+/* asynchronous: d_counts (device) = int64 [k][nwin][2], (S, H) of THIS SHARD's columns of every window, in global window
+ * coordinates (nwin from the whole alignment's length): the vectors of the column shards of an alignment add up to the whole
+ * alignment's (pfa_xchg_allreduce).  Runs the site scan with the per-site H into scratch memory of the device pool. */
+int pfa_site_windows_device(pfa_aln* a, int64_t window, int64_t step, int64_t* d_counts);
+/* synchronous: counts (host) = int64 [k][nwin][2] as above; fin (host, optional) = pfa_final_out [k][nwin], the K5 outputs of
+ * every (population, window).  window < 1 or step < 1: PFA_ERR_ARG. */
+int pfa_site_windows(pfa_aln* a, int64_t window, int64_t step, int jc, int64_t* counts, pfa_final_out* fin /* optional */);
 
 #ifdef __cplusplus
 }

@@ -20,9 +20,10 @@ EXPORTS = [
     "pfa_fasta_parse_file", "pfa_fasta_parse_buffer", "pfa_fasta_free", "pfa_fasta_nseq", "pfa_fasta_seqlen",
     "pfa_fasta_row_len", "pfa_fasta_header", "pfa_fasta_copy_row",
     "pfa_aln_from_fasta", "pfa_aln_from_rows", "pfa_aln_from_device_rows", "pfa_aln_synthetic", "pfa_synth_text_device", "pfa_aln_poke_gaps", "pfa_aln_force_validity", "pfa_aln_free",
-    "pfa_aln_nseq", "pfa_aln_nsites", "pfa_aln_num_escapes", "pfa_aln_packed_bytes", "pfa_aln_has_invalid", "pfa_aln_plane_alloc",
+    "pfa_aln_nseq", "pfa_aln_nsites", "pfa_aln_total_sites", "pfa_aln_num_escapes", "pfa_aln_packed_bytes", "pfa_aln_has_invalid", "pfa_aln_plane_alloc",
     "pfa_aln_copy_plane", "pfa_aln_read_probe", "pfa_aln_mask_words", "pfa_aln_set_pops", "pfa_aln_num_pops", "pfa_aln_pop_size",
-    "pfa_site_len", "pfa_site_offset", "pfa_site_stats_device", "pfa_site_stats",
+    "pfa_site_len", "pfa_site_offset", "pfa_site_stats_device", "pfa_site_stats", "pfa_site_stats_hsite_device", "pfa_site_stats_hsite",
+    "pfa_window_count", "pfa_site_windows_device", "pfa_site_windows",
     "pfa_cds_stats_device", "pfa_cds_stats", "pfa_codon_pair_labels", "pfa_codon_set_labels", "pfa_codon_syn3",
     "pfa_codon_class", "pfa_pairwise_device", "pfa_pairwise", "pfa_finalize", "pfa_cds_ssites",
     "pfa_mask_words_for", "pfa_batch_create", "pfa_batch_destroy", "pfa_batch_clear", "pfa_batch_size", "pfa_batch_text_bytes",
@@ -95,6 +96,7 @@ def lib():
         "pfa_aln_free": (c.c_int, [p]),
         "pfa_aln_nseq": (i64, [p]),
         "pfa_aln_nsites": (i64, [p]),
+        "pfa_aln_total_sites": (i64, [p]),
         "pfa_aln_num_escapes": (i64, [p]),
         "pfa_aln_packed_bytes": (i64, [p]),
         "pfa_aln_has_invalid": (c.c_int, [p]),
@@ -110,6 +112,11 @@ def lib():
         "pfa_site_offset": (i64, [p, c.c_int]),
         "pfa_site_stats_device": (c.c_int, [p, p, p]),
         "pfa_site_stats": (c.c_int, [p, p, p]),
+        "pfa_site_stats_hsite_device": (c.c_int, [p, p, p, p]),
+        "pfa_site_stats_hsite": (c.c_int, [p, p, p, p]),
+        "pfa_window_count": (i64, [i64, i64, i64]),
+        "pfa_site_windows_device": (c.c_int, [p, i64, i64, p]),
+        "pfa_site_windows": (c.c_int, [p, i64, i64, c.c_int, p, p]),
         "pfa_cds_stats_device": (c.c_int, [p, p, p]),
         "pfa_cds_stats": (c.c_int, [p, p, p]),
         "pfa_codon_pair_labels": (c.c_int, [c.c_int, c.c_int]),

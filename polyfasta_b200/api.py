@@ -101,6 +101,15 @@ def synth_text_device(ctx, d_ptr, ld, n, seed, p_seg_ppm=50000, tri_ppm=10000, c
           ctx.handle)
 
 
+def window_count(L, window, step):
+    """number of windows of `window` columns every `step` along L columns (pfa_window_count; no GPU needed): windows start at
+    0, step, 2 step, ... and the first one that reaches the end of the alignment is the last"""
+    n = int(lib().pfa_window_count(int(L), int(window), int(step)))
+    if n < 0:
+        raise ValueError("window_count: need L >= 0, window >= 1, step >= 1 (got %r, %r, %r)" % (L, window, step))
+    return n
+
+
 def default_context(device=0):
     ctx = _default_ctx.get(device)
     if ctx is None or not ctx._h:
@@ -227,6 +236,7 @@ class Alignment:
         L = lib()
         self.n = int(L.pfa_aln_nseq(handle))
         self.nsites = int(L.pfa_aln_nsites(handle))
+        self.total_len = int(L.pfa_aln_total_sites(handle))   # columns of the whole alignment (this may be a shard of it)
 
     # ---- constructors ----
     @classmethod
@@ -380,18 +390,59 @@ class Alignment:
         return [{"n": sizes[q], "S": int(vec[off[q]]), "H": int(vec[off[q] + 1]),
                  "sfs": [int(x) for x in vec[off[q] + 2: off[q + 1]]]} for q in range(len(sizes))]
 
-    def site_stats(self, want_isvar=False):
-        """K2 -> list of dict(n, S, H, sfs[, isvar]) per population"""
+    def site_stats(self, want_isvar=False, want_hsite=False):
+        """K2 -> list of dict(n, S, H, sfs[, isvar][, hsite]) per population; hsite: int64 per site of this shard, the column's
+        n^2 - sum_a c_a^2 where it is variable in the population, 0 elsewhere"""
         out = np.zeros(max(self.site_len(), 1), dtype=np.int64)
         k = self.num_pops
         isvar = np.zeros((k, max(self.nsites, 1)), dtype=np.uint8) if want_isvar else None
-        check(lib().pfa_site_stats(self.handle, out.ctypes.data, isvar.ctypes.data if want_isvar else None), self.ctx.handle)
+        hsite = np.zeros((k, max(self.nsites, 1)), dtype=np.int64) if want_hsite else None
+        if want_hsite:
+            check(lib().pfa_site_stats_hsite(self.handle, out.ctypes.data, isvar.ctypes.data if want_isvar else None, hsite.ctypes.data),
+                  self.ctx.handle)
+        else:
+            check(lib().pfa_site_stats(self.handle, out.ctypes.data, isvar.ctypes.data if want_isvar else None), self.ctx.handle)
         res = self.unpack_site(out)
-        if want_isvar:
-            flat = isvar.reshape(-1)[: k * self.nsites].reshape(k, self.nsites) if self.nsites else isvar[:, :0]
-            for q in range(k):
-                res[q]["isvar"] = flat[q]
+        for name, arr in (("isvar", isvar), ("hsite", hsite)):
+            if arr is not None:
+                flat = arr.reshape(-1)[: k * self.nsites].reshape(k, self.nsites) if self.nsites else arr[:, :0]
+                for q in range(k):
+                    res[q][name] = flat[q]
         return res
+
+    def window_count(self, window, step=None):
+        return window_count(self.total_len, window, window if step is None else step)
+
+    def site_windows(self, window, step=None, jc=False):
+        """pi, theta and Tajima's D in windows of `window` columns every `step` (default: `window`) along the alignment ->
+        list of dict(start, end, seqlen, pops=[dict(n, S, H, poly)]), start 0-based, end exclusive; poly is the tuple
+        Context.finalize returns.  For a column shard the counts are the shard's part (see site_windows_device)."""
+        step = window if step is None else step
+        if window < 1 or step < 1:
+            raise ValueError("window and step must be >= 1")
+        nwin = self.window_count(window, step)
+        k = self.num_pops
+        counts = np.zeros((k, max(nwin, 1), 2), dtype=np.int64)
+        fin = (FinalOut * max(k * nwin, 1))()
+        check(lib().pfa_site_windows(self.handle, int(window), int(step), int(bool(jc)), counts.ctypes.data, fin), self.ctx.handle)
+        sizes = self.pop_sizes()
+        res = []
+        for i in range(nwin):
+            start = i * step
+            end = min(start + window, self.total_len)
+            pops = []
+            for q in range(k):
+                S, H = int(counts[q, i, 0]), int(counts[q, i, 1])
+                o = fin[q * nwin + i]
+                poly = (0, 0, 0, "NA") if o.no_var else (S, o.pi_site, o.theta_site, "NA" if o.D_is_NA else o.D)
+                pops.append({"n": sizes[q], "S": S, "H": H, "poly": poly})
+            res.append({"start": start, "end": end, "seqlen": end - start, "pops": pops})
+        return res
+
+    def site_windows_device(self, window, step, d_ptr):
+        """asynchronous: int64 [k][nwin][2] (S, H) of this shard's columns of every window into caller device memory; the
+        vectors of the column shards add up to the whole alignment's (Exchange.allreduce)"""
+        check(lib().pfa_site_windows_device(self.handle, int(window), int(step), ctypes.c_void_p(d_ptr)), self.ctx.handle)
 
     def site_stats_device(self, d_out_ptr, d_isvar_ptr=None):
         """asynchronous K2 into caller device memory (int64[site_len]); for the multi-GPU all-reduce"""

@@ -62,6 +62,7 @@ FLAGS = [
 ]
 
 HEADER_NONCDS = "file,seqlen,pop,N,seg_sites,pi,theta,tajimasD"
+HEADER_WINDOWS = "file,window_start,window_end,seqlen,pop,N,seg_sites,pi,theta,tajimasD"
 HEADER_CDS = ("file,sites_S,sites_N,pop,N,seg_sites_S,seg_sites_N,pi_S,pi_N,theta_S,theta_N,"
               "tajimasD_S,tajimasD_N,nstops")
 
@@ -72,7 +73,27 @@ def build_parser():
     for long, short, kw in FLAGS:
         names = [long] if short is None else [long, short]
         parser.add_argument(*names, **kw)
+    # beyond the reference: sliding windows along the alignment
+    parser.add_argument("--window", type=int, default=None, metavar="W",
+                        help="pi, theta and Tajima's D in windows of W alignment columns (one row per window and population;\n"
+                             "window_start / window_end are 1-based and inclusive). Not with --cds.")
+    parser.add_argument("--step", type=int, default=None, metavar="S",
+                        help="start a window every S columns (default: W). S > W skips the columns between windows.")
     return parser
+
+
+def check_window_args(parser, args):
+    """the --window / --step combinations that are errors"""
+    if args.step is not None and args.window is None:
+        parser.error("--step needs --window")
+    if args.window is None:
+        return None
+    if args.cds:
+        parser.error("--window does not work with --cds")
+    step = args.window if args.step is None else args.step
+    if args.window < 1 or step < 1:
+        parser.error("--window and --step must be positive")
+    return args.window, step
 
 
 class Sink:
@@ -82,8 +103,8 @@ class Sink:
         self.out = out
         self.silent = silent
 
-    def header(self, cds):
-        line = HEADER_CDS if cds else HEADER_NONCDS
+    def header(self, cds, windows=False):
+        line = HEADER_WINDOWS if windows else HEADER_CDS if cds else HEADER_NONCDS
         if self.out:
             with open(self.out, "w") as o:
                 o.write(line + "\n")
@@ -140,6 +161,21 @@ def format_rows(ctx, file, seqlen, cds, jc, pops, site, cdsst):
         else:
             r = next(fin)
             lines.append(f"{file},{seqlen},{label},{n},{r[0]},{r[1]},{r[2]},{r[3]}")           # :196/:198
+    return lines
+
+
+def window_rows(file, found, wins):
+    """rows of one alignment in windows: wins = [(start, end, [(S, poly) per population])], start 0-based, end exclusive.
+    Window by window, the populations in order; each row is the row format_rows gives for the window's columns alone, with
+    the window's 1-based inclusive coordinates in front of seqlen (the window's length)."""
+    lines = []
+    for start, end, per_pop in wins:
+        for (label, _, n), (S, r) in zip(found, per_pop):
+            head = f"{file},{start + 1},{end},{end - start},{label},{n}"
+            if S == 0:
+                lines.append(head + ",0,0,0,NA")                                                   # :187/:189
+            else:
+                lines.append(head + f",{r[0]},{r[1]},{r[2]},{r[3]}")                               # :196/:198
     return lines
 
 
@@ -201,7 +237,46 @@ class RankGroup:
             self.xchg = None
 
 
-def sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found):
+XCHG_MAX_WORDS = 1 << 28   # the longest vector an exchange takes (pfa_xchg_create); longer window vectors go through the host
+
+
+def sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window):
+    """--window over column shards: every rank computes its shard's (S, H) per (population, window), the vectors are summed
+    over the ranks (the exchange, or the host collective when the group is not fused or the vector is longer than an exchange
+    takes), rank 0 finalises and formats"""
+    import torch
+    W, step = window
+    k, L = len(found), fasta.seqlen
+    nwin = api.window_count(L, W, step)
+    words = max(2 * k * nwin, 1)
+    d_cnt = torch.zeros(words, dtype=torch.int64, device="cuda:%d" % ctx.device)
+    torch.cuda.synchronize(ctx.device)
+    if group.fused and words <= XCHG_MAX_WORDS:
+        x = group.exchange(ctx, words)
+        ctx.sync()
+        group.dist.barrier()
+        aln.site_windows_device(W, step, d_cnt.data_ptr())
+        x.allreduce(d_cnt.data_ptr(), words)
+        ctx.sync()
+        if x.timed_out():
+            raise api.PolyFastaError(1, "a rank did not arrive at the exchange")
+        h = d_cnt.cpu()
+    else:
+        aln.site_windows_device(W, step, d_cnt.data_ptr())
+        ctx.sync()
+        h = d_cnt.cpu()
+        group.dist.all_reduce(h)
+    if group.rank != 0:
+        return None
+    cnt = h.numpy()[: 2 * k * nwin].reshape(k, nwin, 2) if nwin else None
+    items = [(rows, int(cnt[q, i, 0]), int(cnt[q, i, 1]), min(i * step + W, L) - i * step, jc)
+             for i in range(nwin) for q, (_, _, rows) in enumerate(found)]
+    fin = iter(ctx.finalize(items))
+    return window_rows(file, found, [(i * step, min(i * step + W, L), [(int(cnt[q, i, 0]), next(fin)) for q in range(k)])
+                                     for i in range(nwin)])
+
+
+def sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window=None):
     """rows of one large alignment whose COLUMNS are split over the ranks (SURVEY.md 8e.1): every rank uploads and scans its
     codon-aligned range, the scan kernels sum the integer vectors over all ranks, rank 0 formats the rows"""
     import numpy as np
@@ -213,6 +288,8 @@ def sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found):
         if found[0][1] is not None:
             m = np.stack([mask for _, mask, _ in found])
             api.check(api.lib().pfa_aln_set_pops(aln.handle, m.ctypes.data, len(found)), ctx.handle)
+        if window is not None:
+            return sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window)
         k = len(found)
         ns, nc = aln.site_len(), api.PFA_CDS_LEN * k
         d_site = torch.zeros(ns, dtype=torch.int64, device="cuda:%d" % ctx.device)
@@ -280,14 +357,17 @@ def plan_populations(fasta, popkeys):
     return plan
 
 
-def single_alignment_rows(ctx, fasta, file, cds, jc, found):
-    """rows of one alignment through the single-alignment kernels (large alignments, and --cds)"""
+def single_alignment_rows(ctx, fasta, file, cds, jc, found, window=None):
+    """rows of one alignment through the single-alignment kernels (large alignments, --cds and --window)"""
     import numpy as np
     aln = api.Alignment.from_fasta(ctx, fasta)
     try:
         if found[0][1] is not None:
             m = np.stack([mask for _, mask, _ in found])
             api.check(api.lib().pfa_aln_set_pops(aln.handle, m.ctypes.data, len(found)), ctx.handle)
+        if window is not None:
+            wins = aln.site_windows(window[0], window[1], jc)
+            return window_rows(file, found, [(w["start"], w["end"], [(p["S"], p["poly"]) for p in w["pops"]]) for w in wins])
         site = aln.site_stats()
         cdsst = aln.cds_stats() if cds else None
     finally:
@@ -295,9 +375,11 @@ def single_alignment_rows(ctx, fasta, file, cds, jc, found):
     return format_rows(ctx, file, fasta.seqlen, cds, jc, [(label, rows) for label, _, rows in found], site, cdsst)
 
 
-def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None):
+def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None):
     """items: [(path, Fasta | exception)] in output order -> ordered actions ('stdout' | 'note' | 'row', ...).
-    Small non-CDS loci of the chunk share ONE batched GPU pass; everything else goes through the single-alignment path."""
+    Small non-CDS loci of the chunk share ONE batched GPU pass; everything else goes through the single-alignment path.
+    window = (W, step): every alignment goes through the single-alignment path (or the column shards of `group`) and gives
+    its window rows after its '# Pop ... not found' notes."""
     actions = []
     pending = []   # (position in actions, locus, pop, file, seqlen, label, n)
     own_batch = None
@@ -319,6 +401,16 @@ def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None):
         plan = plan_populations(fasta, popkeys)
         found = [p for p in plan if p[2] > 0]
         rows = iter(())
+        if window is not None:
+            for label, mask, hits in plan:
+                if hits == 0:
+                    actions.append(("note", f"# Pop {label} string was not found in fasta headers."))   # :126-132
+            if found:
+                lines = (sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window) if group is not None
+                         else single_alignment_rows(ctx, fasta, file, cds, jc, found, window))
+                for i, line in enumerate(lines or ()):
+                    actions.append(("row", line, file, found[i % len(found)][0]))
+            continue
         if found and group is not None:
             rows = iter(sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found))
         elif found and (cds or not api.Batch.fits(fasta)):
@@ -478,13 +570,18 @@ def devices_from_env():
 _SLOTS = {}
 
 
-def run_files(paths, cds, jc, popkeys, sink):
+def run_files(paths, cds, jc, popkeys, sink, window=None):
     """the per-file loop of PolyFastA.py:104-140 over sorted paths, in chunks; chunk i runs on device i mod G and the
     rows are emitted in the reference's order"""
     from concurrent.futures import ThreadPoolExecutor
     from . import parallel
     devs = devices_from_env()
     chunks = [ps for _, ps in parallel.plan_units(paths, [_file_size(p) for p in paths], None, BATCH_FILES, BATCH_BYTES)]
+    if window is not None:   # windows: file by file through the single-alignment path on the first listed device
+        ctx = api.default_context(devs[0])
+        for ps in chunks:
+            emit(process_chunk(ctx, None, list(zip(ps, api.parse_files(ps))), cds, jc, popkeys, window=window), sink)
+        return
     if len(chunks) > 1 and os.environ.get("POLYFASTA_DOUBLE_BUFFER", "1") != "0":
         devs = [d for d in devs for _ in (0, 1)]   # two slots per GPU: host staging of chunk i+1 overlaps the GPU pass of chunk i
     state = _SLOTS   # contexts and pinned staging buffers outlive one call (a process that runs several directories reuses them)
@@ -512,7 +609,7 @@ def run_files(paths, cds, jc, popkeys, sink):
             pl.shutdown()
 
 
-def run_files_ranks(paths, cds, jc, popkeys, sink, group):
+def run_files_ranks(paths, cds, jc, popkeys, sink, group, window=None):
     """the same loop under torchrun (one process per GPU).  Units in the reference's order: a file of at least
     SHARD_MIN_BYTES is ONE alignment scanned by ALL ranks in column shards (exchange fused into the kernels); the other
     files are grouped in chunks and chunk j goes to rank j mod world with no collective (SURVEY.md 8e.2).  Rank 0 gathers the
@@ -527,12 +624,15 @@ def run_files_ranks(paths, cds, jc, popkeys, sink, group):
     for ui, (kind, ps) in enumerate(units):
         if kind == "all":
             fasta = group.parse_once(ps[0], threads)
-            acts = process_chunk(ctx, None, [(ps[0], fasta)], cds, jc, popkeys, group=group)
+            acts = process_chunk(ctx, None, [(ps[0], fasta)], cds, jc, popkeys, group=group, window=window)
             if group.rank == 0:
                 mine.append((ui, acts))
             continue
         if parallel.chunk_owner(j, group.world) == group.rank:
-            mine.append((ui, process_chunk_native(ctx, batch, ps, jc, popkeys, threads, cds)))
+            if window is not None:
+                mine.append((ui, process_chunk(ctx, None, list(zip(ps, api.parse_files(ps, threads))), cds, jc, popkeys, window=window)))
+            else:
+                mine.append((ui, process_chunk_native(ctx, batch, ps, jc, popkeys, threads, cds)))
         j += 1
     group.close(ctx)
     gathered = parallel.gather_rows(mine)
@@ -544,6 +644,7 @@ def run_files_ranks(paths, cds, jc, popkeys, sink, group):
 def main(argv=None):
     parser = build_parser()
     args = parser.parse_args(argv)
+    window = check_window_args(parser, args)
     if args.file == "" and args.dir == "." and not args.pipe:
         print("Both --file/-f and --dir/-d were not found.")
         r = input("Do you wish to run polySFS on all files in the current directory? [y|n]: ")
@@ -562,7 +663,7 @@ def main(argv=None):
     if group is not None and args.pipe:
         group = None
     if not args.silent and (group is None or group.rank == 0):
-        sink.header(args.cds)
+        sink.header(args.cds, window is not None)
     popkeys = args.pops.split(",") if args.pops else None
     paths = sorted(args.file)
     if paths and args.pipe:
@@ -576,12 +677,12 @@ def main(argv=None):
                 fasta = api.Fasta.from_bytes(data)
             except api.NotFasta as e:
                 fasta = e
-            emit(process_chunk(ctx, batch, [(path, fasta)], args.cds, args.jc, popkeys), sink)
+            emit(process_chunk(ctx, batch, [(path, fasta)], args.cds, args.jc, popkeys, window=window), sink)
             data = b""
     elif paths and group is not None:
-        run_files_ranks(paths, args.cds, args.jc, popkeys, sink, group)
+        run_files_ranks(paths, args.cds, args.jc, popkeys, sink, group, window)
     elif paths:
-        run_files(paths, args.cds, args.jc, popkeys, sink)
+        run_files(paths, args.cds, args.jc, popkeys, sink, window)
     if len(args.out) != 0 and not args.silent and (group is None or group.rank == 0):
         print("")
     return 0

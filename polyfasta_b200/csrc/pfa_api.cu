@@ -418,6 +418,7 @@ int pfa_aln_synthetic(pfa_ctx* ctx, int64_t n, int64_t L, uint64_t seed, uint32_
 
 int64_t pfa_aln_nseq(const pfa_aln* a) { return a ? a->n : 0; }
 int64_t pfa_aln_nsites(const pfa_aln* a) { return a ? a->ns : 0; }
+int64_t pfa_aln_total_sites(const pfa_aln* a) { return a ? a->L_total : 0; }
 int64_t pfa_aln_num_escapes(const pfa_aln* a) { return a ? a->n_exc : 0; }
 int64_t pfa_aln_packed_bytes(const pfa_aln* a) { return a ? 3 * a->ns * (int64_t)a->Wq * 16 : 0; }
 int pfa_aln_has_invalid(const pfa_aln* a) { return a ? a->has_invalid : 0; }
@@ -509,6 +510,34 @@ int pfa_site_stats(pfa_aln* a, int64_t* out, uint8_t* isvar) {
     if (!a || !out) return PFA_ERR_ARG;
     return run_to_host(a, sizeof(int64_t) * (size_t)pfa_site_len(a), out, (size_t)(a->k * a->ns), isvar,
                        [&](void* d_out, void* d_aux) { return pfa_launch_site_scan(a, (int64_t*)d_out, (uint8_t*)d_aux); });
+}
+
+int pfa_site_stats_hsite_device(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, int64_t* d_hsite) {
+    if (!a || !d_out) return PFA_ERR_ARG;
+    PFA_CUDA(a->ctx, cudaSetDevice(a->ctx->device));
+    return pfa_launch_site_scan(a, d_out, d_isvar, nullptr, false, d_hsite);
+}
+
+int pfa_site_stats_hsite(pfa_aln* a, int64_t* out, uint8_t* isvar, int64_t* hsite) {
+    if (!a || !out) return PFA_ERR_ARG;
+    if (!hsite) return pfa_site_stats(a, out, isvar);
+    pfa_ctx* ctx = a->ctx;
+    PFA_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t hbytes = sizeof(int64_t) * (size_t)a->k * (size_t)a->ns;
+    int64_t* d_hsite = nullptr;
+    PFA_CUDA(ctx, pfa_dmalloc(ctx, &d_hsite, std::max<size_t>(hbytes, 8)));
+    int rc = run_to_host(a, sizeof(int64_t) * (size_t)pfa_site_len(a), out, (size_t)(a->k * a->ns), isvar, [&](void* d_out, void* d_aux) {
+        return pfa_launch_site_scan(a, (int64_t*)d_out, (uint8_t*)d_aux, nullptr, false, d_hsite);
+    });
+    cudaError_t e = cudaSuccess;
+    if (!rc && hbytes) {
+        e = cudaMemcpyAsync(hsite, d_hsite, hbytes, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    }
+    pfa_dfree(ctx, d_hsite);
+    if (rc) return rc;
+    if (e != cudaSuccess) return pfa_fail(ctx, PFA_ERR_CUDA, "result copy failed: %s", cudaGetErrorString(e));
+    return PFA_OK;
 }
 
 int pfa_cds_stats_device(pfa_aln* a, int64_t* d_out, uint8_t* d_labels) {
@@ -655,7 +684,7 @@ int pfa_aln_flagged_sites(pfa_aln* a, int64_t* out) {
     return PFA_OK;
 }
 
-void pfa_fill_site_args(const pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, PfaSiteArgs* args) {
+void pfa_fill_site_args(const pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, PfaSiteArgs* args, int64_t* d_hsite) {
     memset(&args->x, 0, sizeof args->x);
     args->work = a->ctx->d_work;
     args->b0 = a->b0;
@@ -668,6 +697,7 @@ void pfa_fill_site_args(const pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, PfaS
     args->sfs_off = a->d_pop_n + 2 * a->k;
     args->out = d_out;
     args->isvar = d_isvar;
+    args->hsite = d_hsite;
     args->ns = a->ns;
     args->vflag = nullptr;  // the launchers switch the sparse validity fetch on
     args->gc = a->gc;

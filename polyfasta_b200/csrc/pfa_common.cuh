@@ -129,7 +129,12 @@ struct pfa_xchg;
 struct PfaXchgDev;
 // x != nullptr: fused with the sum over the column shards of all ranks (pfa_xchg.cu); d_out receives the reduced vector
 // defer (with x): the shard's vector stays in the exchange's partial buffer and travels with the next exchange (the codon scan's)
-int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg* x = nullptr, bool defer = false);
+// d_hsite (optional): int64 [k][ns], H of every variable (site, population), 0 elsewhere (pfa_site_stats_hsite_device)
+int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg* x = nullptr, bool defer = false,
+                         int64_t* d_hsite = nullptr);
+// windowed (S, H) of this shard from the per-site H of the site scan (pfa_windows.cu)
+int pfa_launch_site_windows(pfa_aln* a, const int64_t* d_hsite, int64_t window, int64_t step, int64_t* d_counts);
+int pfa_launch_window_final_in(pfa_aln* a, const int64_t* d_counts, int64_t window, int64_t step, int jc, pfa_final_in* d_in);
 int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg* x = nullptr);
 int pfa_xchg_fill(pfa_xchg* x, int64_t len, int64_t* d_out, PfaXchgDev* dev, bool coresident = false);
 unsigned long long* pfa_xchg_partial(pfa_xchg* x);

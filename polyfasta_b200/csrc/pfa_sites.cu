@@ -75,6 +75,7 @@ __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_site_scan_kernel(const P
             if (r.has_escape) continue;  // finished by pfa_escape_sites_kernel
             if (a.isvar) a.isvar[(int64_t)q * a.ns + s] = (uint8_t)r.isvar;
             if (r.isvar) {
+                if (a.hsite) a.hsite[(int64_t)q * a.ns + s] = (int64_t)r.h;
                 atomicAdd(&sm_SH[2 * q], 1ull);
                 atomicAdd(&sm_SH[2 * q + 1], r.h);
                 if (r.sfs_bin >= 0) {
@@ -173,6 +174,7 @@ __device__ __forceinline__ void pfa_site_finish_regs(const PfaSiteArgs& a, int64
         if (r.has_escape) return;
         if (a.isvar) a.isvar[(int64_t)q * a.ns + s] = (uint8_t)r.isvar;
         if (r.isvar) {
+            if (a.hsite) a.hsite[(int64_t)q * a.ns + s] = (int64_t)r.h;
             atomicAdd(&sm_SH[2 * q], 1ull);
             atomicAdd(&sm_SH[2 * q + 1], r.h);
             if (r.sfs_bin >= 0) {
@@ -350,6 +352,7 @@ __global__ void __launch_bounds__(256) pfa_escape_sites_kernel(const PfaSiteArgs
             PfaSiteResult r = pfa_site_result(c, a.pop_n[q], distinct, sq);
             if (a.isvar) a.isvar[(int64_t)q * a.ns + s] = (uint8_t)r.isvar;
             if (r.isvar) {
+                if (a.hsite) a.hsite[(int64_t)q * a.ns + s] = (int64_t)r.h;
                 atomicAdd(reinterpret_cast<unsigned long long*>(a.out + a.out_off[q]), 1ull);
                 atomicAdd(reinterpret_cast<unsigned long long*>(a.out + a.out_off[q] + 1), r.h);
                 if (r.sfs_bin >= 0)
@@ -375,6 +378,7 @@ __device__ __forceinline__ void pfa_site_coop(const PfaSiteArgs& a, int64_t s, c
         if (r.has_escape) continue;  // finished by pfa_escape_sites_kernel
         if (a.isvar && lane == 0) a.isvar[(int64_t)q * a.ns + s] = (uint8_t)r.isvar;
         if (!r.isvar) continue;
+        if (a.hsite && lane == 0) a.hsite[(int64_t)q * a.ns + s] = (int64_t)r.h;
         if (q < LPS) {
             if (lane == q) {
                 S_mine += 1u;
@@ -426,7 +430,10 @@ __device__ __forceinline__ void pfa_site_gap_counts(const PfaSiteArgs& a, int q,
     }
 }
 
-template <int LPS>
+// STORE_H: store the site's H into a.hsite (the single-population call; with several populations a gap site goes to the
+// whole-warp pass when the per-site H is wanted: the store inside the population loop cost the validity-aware multi-population
+// kernels 8-18 bytes of spills)
+template <int LPS, bool STORE_H>
 __device__ __forceinline__ void pfa_site_gap_apply(const PfaSiteArgs& a, int64_t s, int q, uint32_t pa, uint32_t pb, int sub, unsigned gmask,
                                                    unsigned long long* sm_SH, uint32_t& S_mine, unsigned long long& H_mine) {
     pa = pfa_group_add<LPS>(pa, gmask);
@@ -439,6 +446,7 @@ __device__ __forceinline__ void pfa_site_gap_apply(const PfaSiteArgs& a, int64_t
     if (!isvar) return;
     const unsigned long long h = (unsigned long long)nq * nq - ((unsigned long long)valid * valid + (unsigned long long)cg * cg +
                                                                  (unsigned long long)cn * cn + (unsigned long long)cq * cq);
+    if (STORE_H && a.hsite && sub == 0) a.hsite[(int64_t)q * a.ns + s] = (int64_t)h;
     if (q < LPS) {
         if (sub == q) {
             S_mine += 1u;
@@ -602,13 +610,17 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
                     const bool bmono = pfa_flags_bases_mono(f);
                     var = s < a.ns && !bmono;
                     gapsite = s < a.ns && bmono && (f & 32u);  // its valid rows show one base, but not all rows are valid
+                    if (MULTI && gapsite && a.hsite) {  // per-site H wanted: the whole-warp pass counts and stores it (see pfa_site_gap_apply)
+                        var = true;
+                        gapsite = false;
+                    }
                     if (gapsite) {
                         if (!MULTI) {
                             pfa_site_gap_counts<LPS, ITER, false>(a, 0, x0, x1, mv, um, cell, fw, sub, pa, pb);
                         } else {
                             for (int q = 0; q < a.k; ++q) {
                                 pfa_site_gap_counts<LPS, ITER, true>(a, q, x0, x1, mv, um, cell, fw, sub, pa, pb);
-                                pfa_site_gap_apply<LPS>(a, s, q, pa, pb, sub, gmask, sm_SH, S_mine, H_mine);
+                                pfa_site_gap_apply<LPS, false>(a, s, q, pa, pb, sub, gmask, sm_SH, S_mine, H_mine);
                             }
                         }
                     }
@@ -631,7 +643,7 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
                 // the slot's last pass no longer needs it: fetch the next block; what is left of a gap site runs on registers
                 // while that block is on its way
                 if (t == m - 1) refill();
-                if (HAS_V && !MULTI && gapsite) pfa_site_gap_apply<LPS>(a, s, 0, pa, pb, sub, gmask, sm_SH, S_mine, H_mine);
+                if (HAS_V && !MULTI && gapsite) pfa_site_gap_apply<LPS, true>(a, s, 0, pa, pb, sub, gmask, sm_SH, S_mine, H_mine);
             } else {
                 const int idx = t * GW + grp;  // site of this group inside the slot
                 const int64_t s = blk * SPS + idx;
@@ -725,10 +737,12 @@ int pfa_tma_plan(pfa_aln* a, const PfaTmaShape& s, PfaTmaPlan* p) {
     return PFA_OK;
 }
 
-int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg* x, bool defer) {
+int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg* x, bool defer, int64_t* d_hsite) {
     pfa_ctx* ctx = a->ctx;
     const int64_t out_len = a->site_off[a->k];
     if (!x) PFA_CUDA(ctx, cudaMemsetAsync(d_out, 0, sizeof(int64_t) * (size_t)out_len, ctx->stream));
+    // per-site H: the kernels store only variable (site, population) pairs, everything else stays zero
+    if (d_hsite && a->ns > 0) PFA_CUDA(ctx, cudaMemsetAsync(d_hsite, 0, sizeof(int64_t) * (size_t)a->k * (size_t)a->ns, ctx->stream));
     if (x && defer) {
         if (pfa_xchg_carry(x) != 0 || out_len > pfa_xchg_cap(x)) return pfa_fail(ctx, PFA_ERR_ARG, "deferred exchange: buffer in use or too small");
         pfa_xchg_set_carry(x, out_len);  // the next exchange pushes these words along
@@ -738,7 +752,7 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
     PfaSiteArgs args;
     unsigned int* work = nullptr;
     if (int rc = pfa_ctx_work(ctx, &work)) return rc;
-    pfa_fill_site_args(a, d_out, d_isvar, &args);
+    pfa_fill_site_args(a, d_out, d_isvar, &args, d_hsite);
     if (x) {
         // the blocks add into the exchange's partial vector (zero between launches); the escape kernel goes FIRST so that
         // the scan kernel's last block sees the complete shard vector when it runs the exchange

@@ -28,6 +28,7 @@ struct PfaSiteArgs {
     const int64_t* sfs_off;  // [k] offset of pop q's bins in the shared-memory histogram
     int64_t* out;
     uint8_t* isvar;  // optional [k][ns]
+    int64_t* hsite;  // optional [k][ns], zero-filled by the launch: H of every variable (site, population), left 0 elsewhere
     int64_t ns;
     int Wq;
     int k;
@@ -379,7 +380,7 @@ __device__ __forceinline__ bool pfa_slot_issue(unsigned char* slot, uint64_t* ba
     return true;
 }
 
-void pfa_fill_site_args(const pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, PfaSiteArgs* args);
+void pfa_fill_site_args(const pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, PfaSiteArgs* args, int64_t* d_hsite = nullptr);
 int pfa_aln_flagged_sites(pfa_aln* a, int64_t* out);
 
 // ---- launch plan of the TMA scans (K2, K4) -----------------------------------------------------------------------------------
