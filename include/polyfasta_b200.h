@@ -308,6 +308,42 @@ int pfa_site_windows_device(pfa_aln* a, int64_t window, int64_t step, int64_t* d
  * every (population, window).  window < 1 or step < 1: PFA_ERR_ARG. */
 int pfa_site_windows(pfa_aln* a, int64_t window, int64_t step, int jc, int64_t* counts, pfa_final_out* fin /* optional */);
 
+/* ---- divergence between populations (beyond the reference: d_xy, d_a and Hudson's F_ST) ---------------------------------
+ * Pairs are the unordered pairs x < y of the populations in pfa_aln_set_pops order: p = 0 .. P-1 for (0,1), (0,2), ...,
+ * (0,k-1), (1,2), ..., P = k(k-1)/2; 2 <= k <= 64 (else PFA_ERR_ARG).  Every character is an allele (A, C, G, T, '-', 'N',
+ * '?' and each distinct other byte).  For a column c, Dxy_site(c) = n_x n_y - sum_a c_{x,a} c_{y,a}: the ordered pairs of
+ * rows (i in x, j in y) whose characters differ at c (a row in both populations compares equal to itself).  D_xy = the sum
+ * of Dxy_site over the columns, an exact int64; for the whole alignment it equals sum_{i in x, j in y} d_ij of pfa_pairwise's
+ * matrix.  Windows are those of pfa_window_count above. */
+typedef struct pfa_div_in {
+    int64_t n_x, n_y, D; /* population sizes and D_xy over the columns */
+    double seqlen;       /* number of columns (the window's length in a window) */
+    double pi_x, pi_y;   /* pi_site of K5 for the two populations over the same columns: 0 when S == 0, JC-corrected with jc */
+    int32_t jc;
+    int32_t pad;
+} pfa_div_in;
+typedef struct pfa_div_out {
+    double dxy, da, fst;
+    int32_t fst_is_NA; /* dxy == 0 */
+    int32_t undefined; /* n_x n_y == 0 or seqlen <= 0: every field is undefined */
+} pfa_div_out;
+/* asynchronous: d_out (device) = int64 [P], THIS SHARD's D_xy of every pair (the vectors of the column shards add up) */
+int pfa_divergence_device(pfa_aln* a, int64_t* d_out);
+/* asynchronous: d_counts (device) = int64 [P][nwin][2], this shard's (columns with Dxy_site > 0, D_xy) of every (pair, window),
+ * in global window coordinates; the vectors of the column shards add up.  Needs P * nsites * 8 bytes of device scratch for the
+ * per-site values (PFA_ERR_CUDA with a message when that allocation fails). */
+int pfa_divergence_windows_device(pfa_aln* a, int64_t window, int64_t step, int64_t* d_counts);
+/* fp64 on the device, in this operation order: dxy = (D / (n_x n_y)) / seqlen; with jc, x = 1 - (4/3) dxy and dxy = -0.75 log(x)
+ * when x > 0 (K5's rule for pi); hw = 0.5 (pi_x + pi_y); da = dxy - hw; fst = 1 - hw / dxy (Hudson, Slatkin & Maddison 1992,
+ * the estimator of Bhatia et al. 2013), fst_is_NA when dxy == 0 */
+int pfa_div_finalize(pfa_ctx* ctx, const pfa_div_in* in, pfa_div_out* out, int count);
+/* synchronous: counts (host) = int64 [P] D_xy of the whole alignment (of this shard for a column shard); out (host, optional) =
+ * pfa_div_out [P], with pi of every population from the site scan and K5 (seqlen = the alignment's length) */
+int pfa_divergence(pfa_aln* a, int jc, int64_t* counts, pfa_div_out* out /* optional */);
+/* synchronous: counts (host) = int64 [P][nwin] D_xy of every (pair, window); out (host, optional) = pfa_div_out [P][nwin], with
+ * pi of every (population, window) from pfa_site_windows.  window < 1 or step < 1: PFA_ERR_ARG. */
+int pfa_divergence_windows(pfa_aln* a, int64_t window, int64_t step, int jc, int64_t* counts, pfa_div_out* out /* optional */);
+
 #ifdef __cplusplus
 }
 #endif

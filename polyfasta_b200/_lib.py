@@ -24,6 +24,7 @@ EXPORTS = [
     "pfa_aln_copy_plane", "pfa_aln_read_probe", "pfa_aln_mask_words", "pfa_aln_set_pops", "pfa_aln_num_pops", "pfa_aln_pop_size",
     "pfa_site_len", "pfa_site_offset", "pfa_site_stats_device", "pfa_site_stats", "pfa_site_stats_hsite_device", "pfa_site_stats_hsite",
     "pfa_window_count", "pfa_site_windows_device", "pfa_site_windows",
+    "pfa_divergence_device", "pfa_divergence_windows_device", "pfa_div_finalize", "pfa_divergence", "pfa_divergence_windows",
     "pfa_cds_stats_device", "pfa_cds_stats", "pfa_codon_pair_labels", "pfa_codon_set_labels", "pfa_codon_syn3",
     "pfa_codon_class", "pfa_pairwise_device", "pfa_pairwise", "pfa_finalize", "pfa_cds_ssites",
     "pfa_mask_words_for", "pfa_batch_create", "pfa_batch_destroy", "pfa_batch_clear", "pfa_batch_size", "pfa_batch_text_bytes",
@@ -44,6 +45,16 @@ class FinalIn(ctypes.Structure):
 class FinalOut(ctypes.Structure):
     _fields_ = [("pi_site", ctypes.c_double), ("theta_site", ctypes.c_double), ("D", ctypes.c_double),
                 ("D_is_NA", ctypes.c_int32), ("no_var", ctypes.c_int32)]
+
+
+class DivIn(ctypes.Structure):
+    _fields_ = [("n_x", ctypes.c_int64), ("n_y", ctypes.c_int64), ("D", ctypes.c_int64), ("seqlen", ctypes.c_double),
+                ("pi_x", ctypes.c_double), ("pi_y", ctypes.c_double), ("jc", ctypes.c_int32), ("pad", ctypes.c_int32)]
+
+
+class DivOut(ctypes.Structure):
+    _fields_ = [("dxy", ctypes.c_double), ("da", ctypes.c_double), ("fst", ctypes.c_double),
+                ("fst_is_NA", ctypes.c_int32), ("undefined", ctypes.c_int32)]
 
 
 class PolyFastaError(RuntimeError):
@@ -117,6 +128,11 @@ def lib():
         "pfa_window_count": (i64, [i64, i64, i64]),
         "pfa_site_windows_device": (c.c_int, [p, i64, i64, p]),
         "pfa_site_windows": (c.c_int, [p, i64, i64, c.c_int, p, p]),
+        "pfa_divergence_device": (c.c_int, [p, p]),
+        "pfa_divergence_windows_device": (c.c_int, [p, i64, i64, p]),
+        "pfa_div_finalize": (c.c_int, [p, c.POINTER(DivIn), c.POINTER(DivOut), c.c_int]),
+        "pfa_divergence": (c.c_int, [p, c.c_int, p, p]),
+        "pfa_divergence_windows": (c.c_int, [p, i64, i64, c.c_int, p, p]),
         "pfa_cds_stats_device": (c.c_int, [p, p, p]),
         "pfa_cds_stats": (c.c_int, [p, p, p]),
         "pfa_codon_pair_labels": (c.c_int, [c.c_int, c.c_int]),

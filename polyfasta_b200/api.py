@@ -6,7 +6,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from ._lib import FinalIn, FinalOut, PFA_CDS_LEN, PolyFastaError, check, lib
+from ._lib import DivIn, DivOut, FinalIn, FinalOut, PFA_CDS_LEN, PolyFastaError, check, lib
 
 _default_ctx = {}
 
@@ -87,6 +87,19 @@ class Context:
                 res.append((int(S), o.pi_site, o.theta_site, "NA" if o.D_is_NA else o.D))
         return res
 
+    def div_finalize(self, items):
+        """items: iterable of (n_x, n_y, D, seqlen, pi_x, pi_y, jc) -> list of (dxy, da, fst | "NA") per item, fp64 on the device
+        (pfa_div_finalize); ("NA", "NA", "NA") where n_x n_y == 0 or seqlen <= 0"""
+        items = list(items)
+        if not items:
+            return []
+        inp = (DivIn * len(items))()
+        for i, (nx, ny, D, seqlen, pi_x, pi_y, jc) in enumerate(items):
+            inp[i] = DivIn(int(nx), int(ny), int(D), float(seqlen), float(pi_x), float(pi_y), int(bool(jc)), 0)
+        out = (DivOut * len(items))()
+        check(lib().pfa_div_finalize(self.handle, inp, out, len(items)), self.handle)
+        return [("NA", "NA", "NA") if o.undefined else (o.dxy, o.da, "NA" if o.fst_is_NA else o.fst) for o in out]
+
     def cds_ssites(self, cds_rows):
         """[k][PFA_CDS_LEN] int64 -> synonymous-site counts (fp64 on the device)"""
         arr = np.ascontiguousarray(cds_rows, dtype=np.int64).reshape(-1, PFA_CDS_LEN)
@@ -108,6 +121,11 @@ def window_count(L, window, step):
     if n < 0:
         raise ValueError("window_count: need L >= 0, window >= 1, step >= 1 (got %r, %r, %r)" % (L, window, step))
     return n
+
+
+def pop_pairs(k):
+    """the population pairs of the divergence statistics, in their order: (0, 1), (0, 2), ..., (0, k-1), (1, 2), ..."""
+    return [(x, y) for x in range(k) for y in range(x + 1, k)]
 
 
 def default_context(device=0):
@@ -443,6 +461,57 @@ class Alignment:
         """asynchronous: int64 [k][nwin][2] (S, H) of this shard's columns of every window into caller device memory; the
         vectors of the column shards add up to the whole alignment's (Exchange.allreduce)"""
         check(lib().pfa_site_windows_device(self.handle, int(window), int(step), ctypes.c_void_p(d_ptr)), self.ctx.handle)
+
+    def divergence(self, jc=False):
+        """d_xy, net divergence d_a and Hudson's F_ST of every population pair (pop_pairs order) over the whole alignment ->
+        list of dict(x, y, n_x, n_y, D, pi_x, pi_y, dxy, da, fst).  D is the exact number of (row of x, row of y, column)
+        triples whose characters differ; pi_x / pi_y are pi_site of the two populations (0 without variable sites); fst is "NA"
+        where dxy == 0 (dxy, da and fst are all "NA" for an empty population).  For a column shard D is the shard's part."""
+        k = self.num_pops
+        pairs = pop_pairs(k)
+        D = np.zeros(max(len(pairs), 1), dtype=np.int64)
+        check(lib().pfa_divergence(self.handle, int(bool(jc)), D.ctypes.data, None), self.ctx.handle)
+        sizes = self.pop_sizes()
+        pis = [p[1] for p in self.ctx.finalize((s["n"], s["S"], s["H"], self.total_len, jc) for s in self.site_stats())]
+        fin = self.ctx.div_finalize((sizes[x], sizes[y], int(D[p]), self.total_len, pis[x], pis[y], jc) for p, (x, y) in enumerate(pairs))
+        return [{"x": x, "y": y, "n_x": sizes[x], "n_y": sizes[y], "D": int(D[p]), "pi_x": pis[x], "pi_y": pis[y],
+                 "dxy": fin[p][0], "da": fin[p][1], "fst": fin[p][2]} for p, (x, y) in enumerate(pairs)]
+
+    def divergence_windows(self, window, step=None, jc=False):
+        """divergence in windows of `window` columns every `step` (default: `window`), as site_windows ->
+        list of dict(start, end, seqlen, pairs=[dict(x, y, D, dxy, da, fst)]), start 0-based, end exclusive; a window's entry is
+        what divergence() returns for the alignment cut to the window's columns"""
+        step = window if step is None else step
+        if window < 1 or step < 1:
+            raise ValueError("window and step must be >= 1")
+        nwin = self.window_count(window, step)
+        pairs = pop_pairs(self.num_pops)
+        D = np.zeros((max(len(pairs), 1), max(nwin, 1)), dtype=np.int64)
+        check(lib().pfa_divergence_windows(self.handle, int(window), int(step), int(bool(jc)), D.ctypes.data, None), self.ctx.handle)
+        D = D.reshape(-1)[: len(pairs) * nwin].reshape(len(pairs), nwin)
+        sizes = self.pop_sizes()
+        wins = self.site_windows(window, step, jc)
+        items = [(sizes[x], sizes[y], int(D[p, i]), w["seqlen"], w["pops"][x]["poly"][1], w["pops"][y]["poly"][1], jc)
+                 for i, w in enumerate(wins) for p, (x, y) in enumerate(pairs)]
+        fin = iter(self.ctx.div_finalize(items))
+        res = []
+        for i, w in enumerate(wins):
+            row = []
+            for p, (x, y) in enumerate(pairs):
+                dxy, da, fst = next(fin)
+                row.append({"x": x, "y": y, "D": int(D[p, i]), "dxy": dxy, "da": da, "fst": fst})
+            res.append({"start": w["start"], "end": w["end"], "seqlen": w["seqlen"], "pairs": row})
+        return res
+
+    def divergence_device(self, d_ptr):
+        """asynchronous: int64 [P] D_xy of this shard of every pair into caller device memory; the vectors of the column shards
+        add up to the whole alignment's (Exchange.allreduce)"""
+        check(lib().pfa_divergence_device(self.handle, ctypes.c_void_p(d_ptr)), self.ctx.handle)
+
+    def divergence_windows_device(self, window, step, d_ptr):
+        """asynchronous: int64 [P][nwin][2] (columns with a difference, D_xy) of this shard's columns of every (pair, window)
+        into caller device memory; the vectors of the column shards add up"""
+        check(lib().pfa_divergence_windows_device(self.handle, int(window), int(step), ctypes.c_void_p(d_ptr)), self.ctx.handle)
 
     def site_stats_device(self, d_out_ptr, d_isvar_ptr=None):
         """asynchronous K2 into caller device memory (int64[site_len]); for the multi-GPU all-reduce"""

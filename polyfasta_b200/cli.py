@@ -63,6 +63,8 @@ FLAGS = [
 
 HEADER_NONCDS = "file,seqlen,pop,N,seg_sites,pi,theta,tajimasD"
 HEADER_WINDOWS = "file,window_start,window_end,seqlen,pop,N,seg_sites,pi,theta,tajimasD"
+HEADER_DXY = "file,seqlen,pop1,pop2,N1,N2,dxy,da,Fst"
+HEADER_DXY_WINDOWS = "file,window_start,window_end,seqlen,pop1,pop2,N1,N2,dxy,da,Fst"
 HEADER_CDS = ("file,sites_S,sites_N,pop,N,seg_sites_S,seg_sites_N,pi_S,pi_N,theta_S,theta_N,"
               "tajimasD_S,tajimasD_N,nstops")
 
@@ -79,7 +81,21 @@ def build_parser():
                              "window_start / window_end are 1-based and inclusive). Not with --cds.")
     parser.add_argument("--step", type=int, default=None, metavar="S",
                         help="start a window every S columns (default: W). S > W skips the columns between windows.")
+    # beyond the reference: divergence between populations
+    parser.add_argument("--dxy", action="store_true", default=False,
+                        help="d_xy, net divergence d_a and Hudson's F_ST between every pair of the -p populations (one row per\n"
+                             "pair instead of the per-population rows; with --window, one row per window and pair). Not with --cds.")
     return parser
+
+
+def check_dxy_args(parser, args):
+    """the --dxy combinations that are errors"""
+    if not args.dxy:
+        return
+    if not args.pops:
+        parser.error("--dxy needs -p/--pops")
+    if args.cds:
+        parser.error("--dxy does not work with --cds")
 
 
 def check_window_args(parser, args):
@@ -103,8 +119,11 @@ class Sink:
         self.out = out
         self.silent = silent
 
-    def header(self, cds, windows=False):
-        line = HEADER_WINDOWS if windows else HEADER_CDS if cds else HEADER_NONCDS
+    def header(self, cds, windows=False, dxy=False):
+        if dxy:
+            line = HEADER_DXY_WINDOWS if windows else HEADER_DXY
+        else:
+            line = HEADER_WINDOWS if windows else HEADER_CDS if cds else HEADER_NONCDS
         if self.out:
             with open(self.out, "w") as o:
                 o.write(line + "\n")
@@ -179,6 +198,18 @@ def window_rows(file, found, wins):
     return lines
 
 
+def dxy_rows(file, found, wins, windowed):
+    """--dxy rows of one alignment: wins = [(start, end, [(dxy, da, fst) per pair])], start 0-based, end exclusive; the pairs in
+    api.pop_pairs order.  windowed: the window's 1-based inclusive coordinates go in front of seqlen (the window's length)"""
+    pairs = api.pop_pairs(len(found))
+    lines = []
+    for start, end, fins in wins:
+        head = f"{file},{start + 1},{end},{end - start}" if windowed else f"{file},{end - start}"
+        for (x, y), (dxy, da, fst) in zip(pairs, fins):
+            lines.append(head + f",{found[x][0]},{found[y][0]},{found[x][2]},{found[y][2]},{dxy},{da},{fst}")
+    return lines
+
+
 class RankGroup:
     """the ranks of a torchrun launch (one process per GPU): rendezvous and row gathering go through torch.distributed
     (gloo, host plumbing only); the per-shard count vectors are summed inside the scan kernels over NVLink (api.Exchange)"""
@@ -240,32 +271,36 @@ class RankGroup:
 XCHG_MAX_WORDS = 1 << 28   # the longest vector an exchange takes (pfa_xchg_create); longer window vectors go through the host
 
 
-def sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window):
-    """--window over column shards: every rank computes its shard's (S, H) per (population, window), the vectors are summed
-    over the ranks (the exchange, or the host collective when the group is not fused or the vector is longer than an exchange
-    takes), rank 0 finalises and formats"""
+def sum_over_ranks(ctx, group, words, launch):
+    """launch(d_ptr) writes this rank's int64 vector of `words` words into device memory; returns the sum over the ranks as a
+    host tensor (the exchange, or the host collective when the group is not fused or the vector is longer than an exchange takes)"""
     import torch
-    W, step = window
-    k, L = len(found), fasta.seqlen
-    nwin = api.window_count(L, W, step)
-    words = max(2 * k * nwin, 1)
     d_cnt = torch.zeros(words, dtype=torch.int64, device="cuda:%d" % ctx.device)
     torch.cuda.synchronize(ctx.device)
     if group.fused and words <= XCHG_MAX_WORDS:
         x = group.exchange(ctx, words)
         ctx.sync()
         group.dist.barrier()
-        aln.site_windows_device(W, step, d_cnt.data_ptr())
+        launch(d_cnt.data_ptr())
         x.allreduce(d_cnt.data_ptr(), words)
         ctx.sync()
         if x.timed_out():
             raise api.PolyFastaError(1, "a rank did not arrive at the exchange")
-        h = d_cnt.cpu()
-    else:
-        aln.site_windows_device(W, step, d_cnt.data_ptr())
-        ctx.sync()
-        h = d_cnt.cpu()
-        group.dist.all_reduce(h)
+        return d_cnt.cpu()
+    launch(d_cnt.data_ptr())
+    ctx.sync()
+    h = d_cnt.cpu()
+    group.dist.all_reduce(h)
+    return h
+
+
+def sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window):
+    """--window over column shards: every rank computes its shard's (S, H) per (population, window), the vectors are summed
+    over the ranks, rank 0 finalises and formats"""
+    W, step = window
+    k, L = len(found), fasta.seqlen
+    nwin = api.window_count(L, W, step)
+    h = sum_over_ranks(ctx, group, max(2 * k * nwin, 1), lambda d: aln.site_windows_device(W, step, d))
     if group.rank != 0:
         return None
     cnt = h.numpy()[: 2 * k * nwin].reshape(k, nwin, 2) if nwin else None
@@ -276,7 +311,38 @@ def sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window):
                                      for i in range(nwin)])
 
 
-def sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window=None):
+def sharded_divergence_rows(ctx, group, aln, fasta, file, jc, found, window):
+    """--dxy over column shards: every rank computes its shard's site vector and D_xy per pair (with --window: (S, H) per
+    (population, window) and D_xy per (pair, window)), ONE vector is summed over the ranks, rank 0 finalises pi and the
+    divergence and formats"""
+    k, L = len(found), fasta.seqlen
+    pairs = api.pop_pairs(k)
+    P = len(pairs)
+    if window is None:
+        ns = aln.site_len()
+        h = sum_over_ranks(ctx, group, ns + P, lambda d: (aln.site_stats_device(d), aln.divergence_device(d + 8 * ns))).numpy()
+        if group.rank != 0:
+            return None
+        pis = [p[1] for p in ctx.finalize((s["n"], s["S"], s["H"], L, jc) for s in aln.unpack_site(h[:ns]))]
+        items = [(found[x][2], found[y][2], int(h[ns + p]), L, pis[x], pis[y], jc) for p, (x, y) in enumerate(pairs)]
+        return dxy_rows(file, found, [(0, L, ctx.div_finalize(items))], False)
+    W, step = window
+    nwin = api.window_count(L, W, step)
+    ws, wd = 2 * k * nwin, 2 * P * nwin
+    h = sum_over_ranks(ctx, group, max(ws + wd, 1),
+                       lambda d: (aln.site_windows_device(W, step, d), aln.divergence_windows_device(W, step, d + 8 * ws))).numpy()
+    if group.rank != 0:
+        return None
+    sc, dc = h[:ws].reshape(k, nwin, 2), h[ws:ws + wd].reshape(P, nwin, 2)
+    span = [(i * step, min(i * step + W, L)) for i in range(nwin)]
+    pis = [p[1] for p in ctx.finalize((found[q][2], int(sc[q, i, 0]), int(sc[q, i, 1]), e - s, jc)
+                                      for i, (s, e) in enumerate(span) for q in range(k))]
+    fin = ctx.div_finalize((found[x][2], found[y][2], int(dc[p, i, 1]), e - s, pis[i * k + x], pis[i * k + y], jc)
+                           for i, (s, e) in enumerate(span) for p, (x, y) in enumerate(pairs))
+    return dxy_rows(file, found, [(s, e, fin[i * P:(i + 1) * P]) for i, (s, e) in enumerate(span)], True)
+
+
+def sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window=None, dxy=False):
     """rows of one large alignment whose COLUMNS are split over the ranks (SURVEY.md 8e.1): every rank uploads and scans its
     codon-aligned range, the scan kernels sum the integer vectors over all ranks, rank 0 formats the rows"""
     import numpy as np
@@ -288,6 +354,8 @@ def sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window=None)
         if found[0][1] is not None:
             m = np.stack([mask for _, mask, _ in found])
             api.check(api.lib().pfa_aln_set_pops(aln.handle, m.ctypes.data, len(found)), ctx.handle)
+        if dxy:
+            return sharded_divergence_rows(ctx, group, aln, fasta, file, jc, found, window)
         if window is not None:
             return sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window)
         k = len(found)
@@ -357,14 +425,19 @@ def plan_populations(fasta, popkeys):
     return plan
 
 
-def single_alignment_rows(ctx, fasta, file, cds, jc, found, window=None):
-    """rows of one alignment through the single-alignment kernels (large alignments, --cds and --window)"""
+def single_alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False):
+    """rows of one alignment through the single-alignment kernels (large alignments, --cds, --window and --dxy)"""
     import numpy as np
     aln = api.Alignment.from_fasta(ctx, fasta)
     try:
         if found[0][1] is not None:
             m = np.stack([mask for _, mask, _ in found])
             api.check(api.lib().pfa_aln_set_pops(aln.handle, m.ctypes.data, len(found)), ctx.handle)
+        if dxy and window is not None:
+            wins = aln.divergence_windows(window[0], window[1], jc)
+            return dxy_rows(file, found, [(w["start"], w["end"], [(p["dxy"], p["da"], p["fst"]) for p in w["pairs"]]) for w in wins], True)
+        if dxy:
+            return dxy_rows(file, found, [(0, fasta.seqlen, [(d["dxy"], d["da"], d["fst"]) for d in aln.divergence(jc)])], False)
         if window is not None:
             wins = aln.site_windows(window[0], window[1], jc)
             return window_rows(file, found, [(w["start"], w["end"], [(p["S"], p["poly"]) for p in w["pops"]]) for w in wins])
@@ -375,11 +448,12 @@ def single_alignment_rows(ctx, fasta, file, cds, jc, found, window=None):
     return format_rows(ctx, file, fasta.seqlen, cds, jc, [(label, rows) for label, _, rows in found], site, cdsst)
 
 
-def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None):
+def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None, dxy=False):
     """items: [(path, Fasta | exception)] in output order -> ordered actions ('stdout' | 'note' | 'row', ...).
     Small non-CDS loci of the chunk share ONE batched GPU pass; everything else goes through the single-alignment path.
     window = (W, step): every alignment goes through the single-alignment path (or the column shards of `group`) and gives
-    its window rows after its '# Pop ... not found' notes."""
+    its window rows after its '# Pop ... not found' notes.  dxy: the same, with one row per population pair (and window); a file
+    with fewer than two populations found gives one more '#' note instead."""
     actions = []
     pending = []   # (position in actions, locus, pop, file, seqlen, label, n)
     own_batch = None
@@ -401,15 +475,19 @@ def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None):
         plan = plan_populations(fasta, popkeys)
         found = [p for p in plan if p[2] > 0]
         rows = iter(())
-        if window is not None:
+        if window is not None or dxy:
             for label, mask, hits in plan:
                 if hits == 0:
                     actions.append(("note", f"# Pop {label} string was not found in fasta headers."))   # :126-132
-            if found:
-                lines = (sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window) if group is not None
-                         else single_alignment_rows(ctx, fasta, file, cds, jc, found, window))
+            if dxy and len(found) < 2:
+                actions.append(("note", f"# Fewer than two populations found in {file}: no divergence rows."))
+            elif found:
+                lines = (sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window, dxy) if group is not None
+                         else single_alignment_rows(ctx, fasta, file, cds, jc, found, window, dxy))
+                keys = ([f"{found[x][0]},{found[y][0]}" for x, y in api.pop_pairs(len(found))] if dxy
+                        else [label for label, _, _ in found])
                 for i, line in enumerate(lines or ()):
-                    actions.append(("row", line, file, found[i % len(found)][0]))
+                    actions.append(("row", line, file, keys[i % len(keys)]))
             continue
         if found and group is not None:
             rows = iter(sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found))
@@ -570,17 +648,17 @@ def devices_from_env():
 _SLOTS = {}
 
 
-def run_files(paths, cds, jc, popkeys, sink, window=None):
+def run_files(paths, cds, jc, popkeys, sink, window=None, dxy=False):
     """the per-file loop of PolyFastA.py:104-140 over sorted paths, in chunks; chunk i runs on device i mod G and the
     rows are emitted in the reference's order"""
     from concurrent.futures import ThreadPoolExecutor
     from . import parallel
     devs = devices_from_env()
     chunks = [ps for _, ps in parallel.plan_units(paths, [_file_size(p) for p in paths], None, BATCH_FILES, BATCH_BYTES)]
-    if window is not None:   # windows: file by file through the single-alignment path on the first listed device
+    if window is not None or dxy:   # windows, divergence: file by file through the single-alignment path on the first listed device
         ctx = api.default_context(devs[0])
         for ps in chunks:
-            emit(process_chunk(ctx, None, list(zip(ps, api.parse_files(ps))), cds, jc, popkeys, window=window), sink)
+            emit(process_chunk(ctx, None, list(zip(ps, api.parse_files(ps))), cds, jc, popkeys, window=window, dxy=dxy), sink)
         return
     if len(chunks) > 1 and os.environ.get("POLYFASTA_DOUBLE_BUFFER", "1") != "0":
         devs = [d for d in devs for _ in (0, 1)]   # two slots per GPU: host staging of chunk i+1 overlaps the GPU pass of chunk i
@@ -609,7 +687,7 @@ def run_files(paths, cds, jc, popkeys, sink, window=None):
             pl.shutdown()
 
 
-def run_files_ranks(paths, cds, jc, popkeys, sink, group, window=None):
+def run_files_ranks(paths, cds, jc, popkeys, sink, group, window=None, dxy=False):
     """the same loop under torchrun (one process per GPU).  Units in the reference's order: a file of at least
     SHARD_MIN_BYTES is ONE alignment scanned by ALL ranks in column shards (exchange fused into the kernels); the other
     files are grouped in chunks and chunk j goes to rank j mod world with no collective (SURVEY.md 8e.2).  Rank 0 gathers the
@@ -624,13 +702,14 @@ def run_files_ranks(paths, cds, jc, popkeys, sink, group, window=None):
     for ui, (kind, ps) in enumerate(units):
         if kind == "all":
             fasta = group.parse_once(ps[0], threads)
-            acts = process_chunk(ctx, None, [(ps[0], fasta)], cds, jc, popkeys, group=group, window=window)
+            acts = process_chunk(ctx, None, [(ps[0], fasta)], cds, jc, popkeys, group=group, window=window, dxy=dxy)
             if group.rank == 0:
                 mine.append((ui, acts))
             continue
         if parallel.chunk_owner(j, group.world) == group.rank:
-            if window is not None:
-                mine.append((ui, process_chunk(ctx, None, list(zip(ps, api.parse_files(ps, threads))), cds, jc, popkeys, window=window)))
+            if window is not None or dxy:
+                mine.append((ui, process_chunk(ctx, None, list(zip(ps, api.parse_files(ps, threads))), cds, jc, popkeys, window=window,
+                                               dxy=dxy)))
             else:
                 mine.append((ui, process_chunk_native(ctx, batch, ps, jc, popkeys, threads, cds)))
         j += 1
@@ -645,6 +724,7 @@ def main(argv=None):
     parser = build_parser()
     args = parser.parse_args(argv)
     window = check_window_args(parser, args)
+    check_dxy_args(parser, args)
     if args.file == "" and args.dir == "." and not args.pipe:
         print("Both --file/-f and --dir/-d were not found.")
         r = input("Do you wish to run polySFS on all files in the current directory? [y|n]: ")
@@ -663,7 +743,7 @@ def main(argv=None):
     if group is not None and args.pipe:
         group = None
     if not args.silent and (group is None or group.rank == 0):
-        sink.header(args.cds, window is not None)
+        sink.header(args.cds, window is not None, args.dxy)
     popkeys = args.pops.split(",") if args.pops else None
     paths = sorted(args.file)
     if paths and args.pipe:
@@ -677,12 +757,12 @@ def main(argv=None):
                 fasta = api.Fasta.from_bytes(data)
             except api.NotFasta as e:
                 fasta = e
-            emit(process_chunk(ctx, batch, [(path, fasta)], args.cds, args.jc, popkeys, window=window), sink)
+            emit(process_chunk(ctx, batch, [(path, fasta)], args.cds, args.jc, popkeys, window=window, dxy=args.dxy), sink)
             data = b""
     elif paths and group is not None:
-        run_files_ranks(paths, args.cds, args.jc, popkeys, sink, group, window)
+        run_files_ranks(paths, args.cds, args.jc, popkeys, sink, group, window, args.dxy)
     elif paths:
-        run_files(paths, args.cds, args.jc, popkeys, sink, window)
+        run_files(paths, args.cds, args.jc, popkeys, sink, window, args.dxy)
     if len(args.out) != 0 and not args.silent and (group is None or group.rank == 0):
         print("")
     return 0

@@ -134,6 +134,11 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
                          int64_t* d_hsite = nullptr);
 // windowed (S, H) of this shard from the per-site H of the site scan (pfa_windows.cu)
 int pfa_launch_site_windows(pfa_aln* a, const int64_t* d_hsite, int64_t window, int64_t step, int64_t* d_counts);
+// the same reduction for `rows` rows of per-site values d_persite [rows][ns]: d_counts [rows][nwin][2] = (non-zero sites, sum)
+// (the divergence windows feed it the per-pair Dxy_site)
+int pfa_launch_row_windows(pfa_aln* a, int rows, const int64_t* d_persite, int64_t window, int64_t step, int64_t* d_counts);
+// K3's first step alone: flags[s] = 1 where two of the n rows differ in the planes (pfa_pairwise.cu)
+int pfa_launch_var_flags(pfa_aln* a, uint8_t* flags);
 int pfa_launch_window_final_in(pfa_aln* a, const int64_t* d_counts, int64_t window, int64_t step, int jc, pfa_final_in* d_in);
 int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg* x = nullptr);
 int pfa_xchg_fill(pfa_xchg* x, int64_t len, int64_t* d_out, PfaXchgDev* dev, bool coresident = false);

@@ -235,6 +235,18 @@ __global__ void __launch_bounds__(256) pfa_pairwise_popsum_kernel(const int32_t*
     }
 }
 
+// step 0 alone, for the divergence scan (pfa_divergence.cu): flags[s] = 1 where two rows differ in the planes; the two-plane
+// instantiation for a pure-ACGT shard, as below
+int pfa_launch_var_flags(pfa_aln* a, uint8_t* flags) {
+    pfa_ctx* ctx = a->ctx;
+    if (a->ns == 0) return PFA_OK;
+    const unsigned g = (unsigned)((a->ns + 7) / 8);
+    if (a->has_invalid) pfa_var_flags_kernel<3><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, a->n, flags);
+    else pfa_var_flags_kernel<2><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, a->n, flags);
+    PFA_LAUNCH_CHECK(ctx);
+    return PFA_OK;
+}
+
 int pfa_launch_pairwise(pfa_aln* a, int64_t* d_out, int32_t* d_matrix) {
     pfa_ctx* ctx = a->ctx;
     PFA_CUDA(ctx, cudaMemsetAsync(d_out, 0, sizeof(int64_t) * (size_t)a->k, ctx->stream));

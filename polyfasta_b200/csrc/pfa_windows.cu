@@ -132,12 +132,16 @@ static unsigned pfa_win_grid(pfa_ctx* ctx, int64_t threads) {
 }
 
 int pfa_launch_site_windows(pfa_aln* a, const int64_t* d_hsite, int64_t window, int64_t step, int64_t* d_counts) {
+    return pfa_launch_row_windows(a, a->k, d_hsite, window, step, d_counts);
+}
+
+int pfa_launch_row_windows(pfa_aln* a, int rows, const int64_t* d_persite, int64_t window, int64_t step, int64_t* d_counts) {
     pfa_ctx* ctx = a->ctx;
     const int64_t nwin = pfa_window_count(a->L_total, window, step);
-    const int64_t nout = (int64_t)a->k * nwin;
+    const int64_t nout = (int64_t)rows * nwin;
     if (nout == 0) return PFA_OK;
     const PfaWinGeom w = pfa_win_geom(a, window, step);
-    const int64_t nbins = (int64_t)a->k * w.nb;
+    const int64_t nbins = (int64_t)rows * w.nb;
     if (nbins == 0) {  // an empty shard contributes nothing
         PFA_CUDA(ctx, cudaMemsetAsync(d_counts, 0, sizeof(int64_t) * 2 * (size_t)nout, ctx->stream));
         return PFA_OK;
@@ -154,8 +158,8 @@ int pfa_launch_site_windows(pfa_aln* a, const int64_t* d_hsite, int64_t window, 
     int G = 1;
     while (G < 32 && G < w.g) G *= 2;
     if (e == cudaSuccess) {
-        pfa_window_bins_kernel<<<pfa_win_grid(ctx, nbins * mpb * G), 256, 0, ctx->stream>>>(d_hsite, a->ns, a->col_begin, w.g, w.b0, w.nb, mpb,
-                                                                                           a->k, G, bins);
+        pfa_window_bins_kernel<<<pfa_win_grid(ctx, nbins * mpb * G), 256, 0, ctx->stream>>>(d_persite, a->ns, a->col_begin, w.g, w.b0, w.nb, mpb,
+                                                                                           rows, G, bins);
         ctx->launches++;
         e = cudaGetLastError();
     }
@@ -164,7 +168,7 @@ int pfa_launch_site_windows(pfa_aln* a, const int64_t* d_hsite, int64_t window, 
     if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveScan(tmp, tmp_bytes, bins, pre, PfaSHAdd(), PfaSH{0, 0}, (int)(nbins + 1), ctx->stream);
     if (e == cudaSuccess) {
         ctx->launches++;
-        pfa_window_counts_kernel<<<pfa_win_grid(ctx, nout), 256, 0, ctx->stream>>>(pre, a->L_total, window, step, w.g, w.b0, w.nb, a->k, nwin, d_counts);
+        pfa_window_counts_kernel<<<pfa_win_grid(ctx, nout), 256, 0, ctx->stream>>>(pre, a->L_total, window, step, w.g, w.b0, w.nb, rows, nwin, d_counts);
         ctx->launches++;
         e = cudaGetLastError();
     }
