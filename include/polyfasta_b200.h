@@ -308,6 +308,23 @@ int pfa_site_windows_device(pfa_aln* a, int64_t window, int64_t step, int64_t* d
  * every (population, window).  window < 1 or step < 1: PFA_ERR_ARG. */
 int pfa_site_windows(pfa_aln* a, int64_t window, int64_t step, int jc, int64_t* counts, pfa_final_out* fin /* optional */);
 
+/* ---- synonymous and nonsynonymous statistics in sliding windows (beyond the reference: --cds --window) --------------------
+ * Windows as above; window and step must be multiples of 3, so that no codon column straddles a window boundary, and a column
+ * shard must start on a codon boundary (else PFA_ERR_ARG).  The vector of a (population, window) has PFA_CDS_WIN_LEN words:
+ * words 0..70 are what pfa_cds_stats returns for the alignment cut to the window's columns (PFA_CDS_* layout; the trailing
+ * partial codon column of an alignment whose length is not a multiple of 3 adds 3 to `missing` of the window that holds it),
+ * word PFA_CDS_WIN_S is the S of pfa_site_stats for the same cut. */
+#define PFA_CDS_WIN_LEN 72
+#define PFA_CDS_WIN_S 71
+/* asynchronous: d_counts (device) = int64 [k][nwin][PFA_CDS_WIN_LEN] of THIS SHARD's columns, in global window coordinates: the
+ * vectors of the column shards add up to the whole alignment's.  Runs the site scan with the per-site H and the codon scan with
+ * the labels, then one pass over the shard's codon columns into bins of gcd(window, step) columns and a prefix sum over the
+ * bins.  Device scratch from the pool: k * nsites * 9 bytes (labels and per-site H) plus k * 72 * (nbins + 1) * 8 bytes, nbins =
+ * the shard's bins of gcd(window, step) columns. */
+int pfa_cds_windows_device(pfa_aln* a, int64_t window, int64_t step, int64_t* d_counts);
+/* synchronous: counts (host) = int64 [k][nwin][PFA_CDS_WIN_LEN] as above */
+int pfa_cds_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* counts);
+
 /* ---- divergence between populations (beyond the reference: d_xy, d_a and Hudson's F_ST) ---------------------------------
  * Pairs are the unordered pairs x < y of the populations in pfa_aln_set_pops order: p = 0 .. P-1 for (0,1), (0,2), ...,
  * (0,k-1), (1,2), ..., P = k(k-1)/2; 2 <= k <= 64 (else PFA_ERR_ARG).  Every character is an allele (A, C, G, T, '-', 'N',

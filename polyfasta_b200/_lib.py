@@ -10,6 +10,7 @@ SO_PATH = os.path.join(_HERE, "libpolyfasta_b200.so")
 
 PFA_OK, PFA_ERR_CUDA, PFA_ERR_ARG, PFA_ERR_NOT_FASTA, PFA_ERR_RAGGED, PFA_ERR_IO, PFA_ERR_NOMEM, PFA_ERR_NON_ASCII = range(8)
 PFA_CDS_LEN = 71
+PFA_CDS_WIN_LEN = 72   # a codon window vector: the PFA_CDS_LEN words, then the site scan's S
 PFA_BATCH_TOO_BIG = 100
 
 # every symbol include/polyfasta_b200.h declares (tests check that the library exports all of them)
@@ -23,7 +24,7 @@ EXPORTS = [
     "pfa_aln_nseq", "pfa_aln_nsites", "pfa_aln_total_sites", "pfa_aln_num_escapes", "pfa_aln_packed_bytes", "pfa_aln_has_invalid", "pfa_aln_plane_alloc",
     "pfa_aln_copy_plane", "pfa_aln_read_probe", "pfa_aln_mask_words", "pfa_aln_set_pops", "pfa_aln_num_pops", "pfa_aln_pop_size",
     "pfa_site_len", "pfa_site_offset", "pfa_site_stats_device", "pfa_site_stats", "pfa_site_stats_hsite_device", "pfa_site_stats_hsite",
-    "pfa_window_count", "pfa_site_windows_device", "pfa_site_windows",
+    "pfa_window_count", "pfa_site_windows_device", "pfa_site_windows", "pfa_cds_windows_device", "pfa_cds_windows",
     "pfa_divergence_device", "pfa_divergence_windows_device", "pfa_div_finalize", "pfa_divergence", "pfa_divergence_windows",
     "pfa_cds_stats_device", "pfa_cds_stats", "pfa_codon_pair_labels", "pfa_codon_set_labels", "pfa_codon_syn3",
     "pfa_codon_class", "pfa_pairwise_device", "pfa_pairwise", "pfa_finalize", "pfa_cds_ssites",
@@ -128,6 +129,8 @@ def lib():
         "pfa_window_count": (i64, [i64, i64, i64]),
         "pfa_site_windows_device": (c.c_int, [p, i64, i64, p]),
         "pfa_site_windows": (c.c_int, [p, i64, i64, c.c_int, p, p]),
+        "pfa_cds_windows_device": (c.c_int, [p, i64, i64, p]),
+        "pfa_cds_windows": (c.c_int, [p, i64, i64, p]),
         "pfa_divergence_device": (c.c_int, [p, p]),
         "pfa_divergence_windows_device": (c.c_int, [p, i64, i64, p]),
         "pfa_div_finalize": (c.c_int, [p, c.POINTER(DivIn), c.POINTER(DivOut), c.c_int]),

@@ -6,7 +6,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from ._lib import DivIn, DivOut, FinalIn, FinalOut, PFA_CDS_LEN, PolyFastaError, check, lib
+from ._lib import DivIn, DivOut, FinalIn, FinalOut, PFA_CDS_LEN, PFA_CDS_WIN_LEN, PolyFastaError, check, lib
 
 _default_ctx = {}
 
@@ -121,6 +121,33 @@ def window_count(L, window, step):
     if n < 0:
         raise ValueError("window_count: need L >= 0, window >= 1, step >= 1 (got %r, %r, %r)" % (L, window, step))
     return n
+
+
+def cds_window_results(ctx, counts, sizes, L, window, step, jc):
+    """codon window vectors int64 [k][nwin][PFA_CDS_WIN_LEN] of an alignment of L columns (pfa_cds_windows, or the sum over its
+    column shards) -> the list Alignment.cds_windows returns; ssites and the K5 entries come from Context.cds_ssites and
+    Context.finalize exactly as for the --cds row of the window's columns"""
+    counts = np.asarray(counts, dtype=np.int64)
+    k, nwin = counts.shape[0], counts.shape[1]
+    ss = ctx.cds_ssites(counts[:, :, :PFA_CDS_LEN].reshape(-1, PFA_CDS_LEN)).reshape(k, nwin) if k * nwin else None
+    res, items = [], []
+    for i in range(nwin):
+        start, end = i * step, min(i * step + window, L)
+        pops = []
+        for q in range(k):
+            row = counts[q, i]
+            c = Alignment.unpack_cds(row)
+            c["ssites"] = float(ss[q, i])
+            c["nsites"] = ((end - start) - c["missing"]) - c["ssites"]
+            c["raw"] = row.copy()
+            items += [(sizes[q], c["S_s"], c["H_s"], c["ssites"], jc), (sizes[q], c["S_n"], c["H_n"], c["nsites"], jc)]
+            pops.append({"n": sizes[q], "S": int(row[PFA_CDS_LEN]), "cds": c})
+        res.append({"start": start, "end": end, "pops": pops})
+    fin = iter(ctx.finalize(items))
+    for w in res:
+        for p in w["pops"]:
+            p["poly_s"], p["poly_n"] = next(fin), next(fin)
+    return res
 
 
 def pop_pairs(k):
@@ -461,6 +488,26 @@ class Alignment:
         """asynchronous: int64 [k][nwin][2] (S, H) of this shard's columns of every window into caller device memory; the
         vectors of the column shards add up to the whole alignment's (Exchange.allreduce)"""
         check(lib().pfa_site_windows_device(self.handle, int(window), int(step), ctypes.c_void_p(d_ptr)), self.ctx.handle)
+
+    def cds_windows(self, window, step=None, jc=False):
+        """synonymous and nonsynonymous pi, theta and Tajima's D in windows of `window` columns every `step` (default: `window`),
+        both multiples of 3 -> list of dict(start, end, pops=[dict(n, S, cds, poly_s, poly_n)]), start 0-based, end exclusive.
+        A window's entry is what site_stats() and cds_stats() give for the alignment cut to the window's columns: S is the site
+        scan's S, cds the unpacked codon vector with ssites, nsites = (window length - missing) - ssites and raw (the
+        PFA_CDS_WIN_LEN words), poly_s / poly_n the tuples Context.finalize returns for (n, S_s, H_s, ssites) and
+        (n, S_n, H_n, nsites).  For a column shard the counts are the shard's part (see cds_windows_device)."""
+        step = window if step is None else step
+        if window < 1 or step < 1 or window % 3 or step % 3:
+            raise ValueError("cds windows: window and step must be positive multiples of 3")
+        nwin = self.window_count(window, step)
+        counts = np.zeros((self.num_pops, max(nwin, 1), PFA_CDS_WIN_LEN), dtype=np.int64)
+        check(lib().pfa_cds_windows(self.handle, int(window), int(step), counts.ctypes.data), self.ctx.handle)
+        return cds_window_results(self.ctx, counts[:, :nwin], self.pop_sizes(), self.total_len, window, step, jc)
+
+    def cds_windows_device(self, window, step, d_ptr):
+        """asynchronous: int64 [k][nwin][PFA_CDS_WIN_LEN] codon window vectors of this shard's columns into caller device memory;
+        the vectors of the column shards add up to the whole alignment's (Exchange.allreduce)"""
+        check(lib().pfa_cds_windows_device(self.handle, int(window), int(step), ctypes.c_void_p(d_ptr)), self.ctx.handle)
 
     def divergence(self, jc=False):
         """d_xy, net divergence d_a and Hudson's F_ST of every population pair (pop_pairs order) over the whole alignment ->

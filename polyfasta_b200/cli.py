@@ -67,6 +67,8 @@ HEADER_DXY = "file,seqlen,pop1,pop2,N1,N2,dxy,da,Fst"
 HEADER_DXY_WINDOWS = "file,window_start,window_end,seqlen,pop1,pop2,N1,N2,dxy,da,Fst"
 HEADER_CDS = ("file,sites_S,sites_N,pop,N,seg_sites_S,seg_sites_N,pi_S,pi_N,theta_S,theta_N,"
               "tajimasD_S,tajimasD_N,nstops")
+HEADER_CDS_WINDOWS = ("file,window_start,window_end,sites_S,sites_N,pop,N,seg_sites_S,seg_sites_N,pi_S,pi_N,theta_S,theta_N,"
+                      "tajimasD_S,tajimasD_N,nstops")
 
 
 def build_parser():
@@ -78,7 +80,8 @@ def build_parser():
     # beyond the reference: sliding windows along the alignment
     parser.add_argument("--window", type=int, default=None, metavar="W",
                         help="pi, theta and Tajima's D in windows of W alignment columns (one row per window and population;\n"
-                             "window_start / window_end are 1-based and inclusive). Not with --cds.")
+                             "window_start / window_end are 1-based and inclusive). With --cds: the synonymous and\n"
+                             "nonsynonymous statistics per window; W and S must then be multiples of 3.")
     parser.add_argument("--step", type=int, default=None, metavar="S",
                         help="start a window every S columns (default: W). S > W skips the columns between windows.")
     # beyond the reference: divergence between populations
@@ -104,11 +107,11 @@ def check_window_args(parser, args):
         parser.error("--step needs --window")
     if args.window is None:
         return None
-    if args.cds:
-        parser.error("--window does not work with --cds")
     step = args.window if args.step is None else args.step
     if args.window < 1 or step < 1:
         parser.error("--window and --step must be positive")
+    if args.cds and (args.window % 3 or step % 3):
+        parser.error("with --cds, --window and --step must be multiples of 3 (a window holds whole codons)")
     return args.window, step
 
 
@@ -123,7 +126,7 @@ class Sink:
         if dxy:
             line = HEADER_DXY_WINDOWS if windows else HEADER_DXY
         else:
-            line = HEADER_WINDOWS if windows else HEADER_CDS if cds else HEADER_NONCDS
+            line = (HEADER_CDS_WINDOWS if cds else HEADER_WINDOWS) if windows else HEADER_CDS if cds else HEADER_NONCDS
         if self.out:
             with open(self.out, "w") as o:
                 o.write(line + "\n")
@@ -195,6 +198,23 @@ def window_rows(file, found, wins):
                 lines.append(head + ",0,0,0,NA")                                                   # :187/:189
             else:
                 lines.append(head + f",{r[0]},{r[1]},{r[2]},{r[3]}")                               # :196/:198
+    return lines
+
+
+def cds_window_rows(file, found, wins):
+    """--cds rows of one alignment in windows: wins = the list Alignment.cds_windows returns.  Window by window, the populations
+    in order; each row is the --cds row format_rows gives for the window's columns alone, with the window's 1-based inclusive
+    coordinates after the file's name"""
+    lines = []
+    for w in wins:
+        for (label, _, n), p in zip(found, w["pops"]):
+            c = p["cds"]
+            head = f"{file},{w['start'] + 1},{w['end']},{round(c['ssites'], 2)},{round(c['nsites'], 2)},{label},{n}"
+            if p["S"] == 0:
+                lines.append(head + ",0,0,0,NA,0,0,0,NA,0")                                     # :160/:162
+            else:
+                s, m = p["poly_s"], p["poly_n"]
+                lines.append(head + f",{s[0]},{m[0]},{s[1]},{m[1]},{s[2]},{m[2]},{s[3]},{m[3]},{c['nstops']}")  # :178/:180
     return lines
 
 
@@ -311,6 +331,20 @@ def sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window):
                                      for i in range(nwin)])
 
 
+def sharded_cds_window_rows(ctx, group, aln, fasta, file, jc, found, window):
+    """--cds --window over column shards (codon-aligned by parallel.shard_columns): every rank computes its shard's codon window
+    vectors, the vectors are summed over the ranks, rank 0 finalises and formats"""
+    W, step = window
+    k, L = len(found), fasta.seqlen
+    nwin = api.window_count(L, W, step)
+    words = k * nwin * api.PFA_CDS_WIN_LEN
+    h = sum_over_ranks(ctx, group, max(words, 1), lambda d: aln.cds_windows_device(W, step, d))
+    if group.rank != 0:
+        return None
+    cnt = h.numpy()[:words].reshape(k, nwin, api.PFA_CDS_WIN_LEN)
+    return cds_window_rows(file, found, api.cds_window_results(ctx, cnt, [rows for _, _, rows in found], L, W, step, jc))
+
+
 def sharded_divergence_rows(ctx, group, aln, fasta, file, jc, found, window):
     """--dxy over column shards: every rank computes its shard's site vector and D_xy per pair (with --window: (S, H) per
     (population, window) and D_xy per (pair, window)), ONE vector is summed over the ranks, rank 0 finalises pi and the
@@ -356,6 +390,8 @@ def sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window=None,
             api.check(api.lib().pfa_aln_set_pops(aln.handle, m.ctypes.data, len(found)), ctx.handle)
         if dxy:
             return sharded_divergence_rows(ctx, group, aln, fasta, file, jc, found, window)
+        if window is not None and cds:
+            return sharded_cds_window_rows(ctx, group, aln, fasta, file, jc, found, window)
         if window is not None:
             return sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window)
         k = len(found)
@@ -426,7 +462,7 @@ def plan_populations(fasta, popkeys):
 
 
 def single_alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False):
-    """rows of one alignment through the single-alignment kernels (large alignments, --cds, --window and --dxy)"""
+    """rows of one alignment through the single-alignment kernels (large alignments, --cds, --window, --cds --window and --dxy)"""
     import numpy as np
     aln = api.Alignment.from_fasta(ctx, fasta)
     try:
@@ -438,6 +474,8 @@ def single_alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=Fal
             return dxy_rows(file, found, [(w["start"], w["end"], [(p["dxy"], p["da"], p["fst"]) for p in w["pairs"]]) for w in wins], True)
         if dxy:
             return dxy_rows(file, found, [(0, fasta.seqlen, [(d["dxy"], d["da"], d["fst"]) for d in aln.divergence(jc)])], False)
+        if window is not None and cds:
+            return cds_window_rows(file, found, aln.cds_windows(window[0], window[1], jc))
         if window is not None:
             wins = aln.site_windows(window[0], window[1], jc)
             return window_rows(file, found, [(w["start"], w["end"], [(p["S"], p["poly"]) for p in w["pops"]]) for w in wins])

@@ -552,6 +552,44 @@ int pfa_cds_stats(pfa_aln* a, int64_t* out, uint8_t* labels) {
                        [&](void* d_out, void* d_aux) { return pfa_launch_cds_scan(a, (int64_t*)d_out, (uint8_t*)d_aux); });
 }
 
+int pfa_cds_windows_device(pfa_aln* a, int64_t window, int64_t step, int64_t* d_counts) {
+    if (!a) return PFA_ERR_ARG;
+    pfa_ctx* ctx = a->ctx;
+    if (window < 1 || step < 1 || window % 3 != 0 || step % 3 != 0)
+        return pfa_fail(ctx, PFA_ERR_ARG, "cds windows: window and step must be positive multiples of 3 (got %lld, %lld)", (long long)window,
+                        (long long)step);
+    if (a->col_begin % 3 != 0) return pfa_fail(ctx, PFA_ERR_ARG, "cds windows: the shard must start on a codon boundary");
+    const int64_t nwin = pfa_window_count(a->L_total, window, step);
+    if (nwin == 0) return PFA_OK;
+    if (!d_counts) return pfa_fail(ctx, PFA_ERR_ARG, "cds windows: null output");
+    PFA_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t per_site = (size_t)a->k * (size_t)a->ns;
+    int64_t *d_site = nullptr, *d_cds = nullptr, *d_hsite = nullptr;
+    uint8_t* d_labels = nullptr;
+    cudaError_t e = pfa_dmalloc(ctx, &d_site, sizeof(int64_t) * (size_t)std::max<int64_t>(pfa_site_len(a), 1));
+    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &d_cds, sizeof(int64_t) * PFA_CDS_LEN * (size_t)a->k);
+    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &d_hsite, sizeof(int64_t) * std::max<size_t>(per_site, 1));
+    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &d_labels, std::max<size_t>(per_site, 1));
+    int rc = e == cudaSuccess ? PFA_OK : pfa_fail(ctx, PFA_ERR_CUDA, "cds windows: cudaMallocAsync failed: %s", cudaGetErrorString(e));
+    if (!rc) rc = pfa_launch_site_scan(a, d_site, nullptr, nullptr, false, d_hsite);
+    if (!rc) rc = pfa_launch_cds_scan(a, d_cds, d_labels);
+    if (!rc) rc = pfa_launch_cds_windows(a, d_hsite, d_labels, window, step, d_counts);
+    pfa_dfree(ctx, d_labels);
+    pfa_dfree(ctx, d_hsite);
+    pfa_dfree(ctx, d_cds);
+    pfa_dfree(ctx, d_site);
+    return rc;
+}
+
+int pfa_cds_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* counts) {
+    if (!a) return PFA_ERR_ARG;
+    const int64_t nwin = pfa_window_count(a->L_total, window, step);
+    if (nwin <= 0) return pfa_cds_windows_device(a, window, step, nullptr);  // argument errors, or nothing to do
+    if (!counts) return pfa_fail(a->ctx, PFA_ERR_ARG, "cds windows: null output");
+    return run_to_host(a, sizeof(int64_t) * PFA_CDS_WIN_LEN * (size_t)(a->k * nwin), counts, 0, nullptr,
+                       [&](void* d_out, void*) { return pfa_cds_windows_device(a, window, step, (int64_t*)d_out); });
+}
+
 int pfa_site_stats_xchg(pfa_aln* a, pfa_xchg* x, int64_t* d_out, uint8_t* d_isvar) {
     if (!a || !x || !d_out) return PFA_ERR_ARG;
     PFA_CUDA(a->ctx, cudaSetDevice(a->ctx->device));

@@ -1387,3 +1387,171 @@ int pfa_launch_batch_cds(pfa_ctx* ctx, const PfaBatchArgs& args, int max_Wq, con
     }
     return PFA_OK;
 }
+
+// ---- codon windows (pfa_cds_windows_device): the PFA_CDS_WIN_LEN-word vector of every (population, bin) ------------------
+// Bins of g = gcd(W, step) columns as in pfa_windows.cu (g is a multiple of 3 and the shard starts on a codon boundary, so
+// every codon column lies in ONE bin).  A bin's vector is what K4 + K2 return for its columns alone:
+//   S_s, H_s, S_n, H_n: sums over the bin's sites of K4's labels and K2's per-site H (H of a labelled position is the
+//     population's H of the column, :169-170); word PFA_CDS_WIN_S is K2's S (sites with H > 0);
+//   nstops, missing, sum3_by_len: functions of the presence mask P of every (codon column, population), as in
+//     pfa_cds_contribute.  A column whose three sites are monomorphic over the union and all valid (no flagged cell, or the
+//     validity plane says so) shows one codon to every population: its terms stay in registers until the piece ends.
+// One warp per piece of at most PFA_CDS_WIN_PIECE sites of a bin (so the number of warps follows ns, not W); every piece adds
+// into its bins with one atomic per non-zero word.  bins = [k][PFA_CDS_WIN_LEN][nb], zeroed by the caller.
+#define PFA_CDS_WIN_PIECE 96  // sites (32 codon columns) per piece
+
+struct PfaCdsWinArgs {
+    PfaSiteArgs s;          // planes, masks, k, Wq, ns, vflag (nullptr: read the validity plane of every column)
+    const int64_t* hsite;   // [k][ns] (K2)
+    const uint8_t* labels;  // [k][ns] (K4)
+    int64_t* bins;
+    int64_t c0, g, b0, nb, mpb, ncf;
+    int has_partial;  // the shard ends with a partial codon column: +3 missing in its bin
+};
+
+__device__ __forceinline__ void pfa_cds_win_add(const PfaCdsWinArgs& a, int q, int w, int64_t j, unsigned long long x) {
+    if (x) atomicAdd(reinterpret_cast<unsigned long long*>(a.bins + ((int64_t)q * PFA_CDS_WIN_LEN + w) * a.nb + j), x);
+}
+
+__device__ __forceinline__ unsigned long long pfa_warp_sum64(unsigned long long x) {
+#pragma unroll
+    for (int off = 16; off; off >>= 1) x += __shfl_xor_sync(0xffffffffu, x, off);
+    return x;
+}
+
+template <bool HAS_V>
+__global__ void __launch_bounds__(256) pfa_cds_window_bins_kernel(const PfaCdsWinArgs a) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int Wq = a.s.Wq, k = a.s.k;
+    const int64_t ns = a.s.ns, total = a.nb * a.mpb;
+    for (int64_t e = warp; e < total; e += nwarps) {  // warp-uniform
+        const int64_t j = e / a.mpb, m = e - j * a.mpb;
+        const int64_t bs = (a.b0 + j) * a.g + m * PFA_CDS_WIN_PIECE;  // global columns of the piece, clipped to the bin and the shard
+        const int64_t lo = max(a.c0, bs) - a.c0, hi = min(min(a.c0 + ns, (a.b0 + j + 1) * a.g), bs + PFA_CDS_WIN_PIECE) - a.c0;
+        if (hi <= lo) continue;
+        // ---- per-site words ----
+        for (int q = 0; q < k; ++q) {
+            const int64_t* hq = a.hsite + (int64_t)q * ns;
+            const uint8_t* lq = a.labels + (int64_t)q * ns;
+            unsigned long long hs = 0, hn = 0, cnt = 0;  // cnt: S at bits 0-15, S_s at 16-31, S_n at 32-47 (a piece < 65,536 sites)
+            for (int64_t i = lo + lane; i < hi; i += 32) {
+                const int64_t h = hq[i];
+                const int l = lq[i];
+                cnt += (h != 0 ? 1ull : 0ull) + (l == 1 ? 1ull << 16 : 0ull) + (l == 2 ? 1ull << 32 : 0ull);
+                hs += l == 1 ? (unsigned long long)h : 0ull;
+                hn += l == 2 ? (unsigned long long)h : 0ull;
+            }
+            cnt = pfa_warp_sum64(cnt);
+            hs = pfa_warp_sum64(hs);
+            hn = pfa_warp_sum64(hn);
+            if (lane == 0) {
+                pfa_cds_win_add(a, q, PFA_CDS_WIN_S, j, cnt & 0xffffull);
+                pfa_cds_win_add(a, q, PFA_CDS_SS, j, (cnt >> 16) & 0xffffull);
+                pfa_cds_win_add(a, q, PFA_CDS_HS, j, hs);
+                pfa_cds_win_add(a, q, PFA_CDS_SN, j, (cnt >> 32) & 0xffffull);
+                pfa_cds_win_add(a, q, PFA_CDS_HN, j, hn);
+            }
+        }
+        // ---- codon words ----
+        unsigned u_nstops = 0, u_missing = 0, u_sum3 = 0;  // identical for every population
+        const int64_t cend = min(hi / 3, a.ncf);
+        for (int64_t cc = lo / 3; cc < cend; ++cc) {
+            const int64_t site0 = cc * 3;
+            bool hv = HAS_V;  // this column's validity plane must be read
+            if (HAS_V && a.s.vflag) hv = (__ldg(a.s.vflag + site0) | __ldg(a.s.vflag + site0 + 1) | __ldg(a.s.vflag + site0 + 2)) != 0u;
+            unsigned f = 0;  // 6 bits per site as in pfa_cds_scan_kernel: b0 one / zero, b1 one / zero, valid / not valid
+            for (int jj = lane; jj < Wq; jj += 32) {
+                const uint4 um = __ldg(a.s.umask + jj);
+#pragma unroll
+                for (int t = 0; t < 3; ++t) {
+                    const uint4 x0 = pfa_ld_stream(a.s.b0 + (site0 + t) * Wq + jj);
+                    const uint4 x1 = pfa_ld_stream(a.s.b1 + (site0 + t) * Wq + jj);
+                    const uint32_t o0 = (x0.x & um.x) | (x0.y & um.y) | (x0.z & um.z) | (x0.w & um.w);
+                    const uint32_t z0 = (~x0.x & um.x) | (~x0.y & um.y) | (~x0.z & um.z) | (~x0.w & um.w);
+                    const uint32_t o1 = (x1.x & um.x) | (x1.y & um.y) | (x1.z & um.z) | (x1.w & um.w);
+                    const uint32_t z1 = (~x1.x & um.x) | (~x1.y & um.y) | (~x1.z & um.z) | (~x1.w & um.w);
+                    uint32_t ov = um.x | um.y | um.z | um.w, zv = 0;
+                    if (HAS_V && hv) {
+                        const uint4 xv = pfa_ld_stream(a.s.v + (site0 + t) * Wq + jj);
+                        ov = (xv.x & um.x) | (xv.y & um.y) | (xv.z & um.z) | (xv.w & um.w);
+                        zv = (~xv.x & um.x) | (~xv.y & um.y) | (~xv.z & um.z) | (~xv.w & um.w);
+                    }
+                    f |= ((o0 ? 1u : 0u) | (z0 ? 2u : 0u) | (o1 ? 4u : 0u) | (z1 ? 8u : 0u) | (ov ? 16u : 0u) | (zv ? 32u : 0u)) << (6 * t);
+                }
+            }
+            f = __reduce_or_sync(0xffffffffu, f);
+            bool uniform = true, clean = true;
+            int codon = 0;
+#pragma unroll
+            for (int t = 0; t < 3; ++t) {
+                const unsigned ft = (f >> (6 * t)) & 63u;
+                const bool mono = ((ft & 3u) != 3u) && ((ft & 12u) != 12u) && ((ft & 48u) != 48u);
+                const bool all_escape = (ft & 1u) && (ft & 4u) && !(ft & 16u);
+                uniform = uniform && mono && !all_escape;
+                clean = clean && (ft & 16u) && !(ft & 32u);
+                codon = (codon << 2) | ((ft & 4u) ? 2 : 0) | ((ft & 1u) ? 1 : 0);
+            }
+            if (uniform) {
+                if (clean) {
+                    u_nstops += (unsigned)((c_stop_mask >> codon) & 1ull);
+                    u_sum3 += c_syn3[codon];
+                } else {
+                    u_missing += 3;
+                }
+                continue;
+            }
+            for (int q = 0; q < k; ++q) {
+                const uint4* mq = a.s.masks + (int64_t)q * Wq;
+                const unsigned long long P = hv ? pfa_codon_presence<true>(a.s.b0, a.s.b1, a.s.v, site0, Wq, mq, lane)
+                                                : pfa_codon_presence<false>(a.s.b0, a.s.b1, a.s.v, site0, Wq, mq, lane);
+                if (lane != 0) continue;
+                const int len = __popcll(P);
+                pfa_cds_win_add(a, q, PFA_CDS_NSTOPS, j, (P & c_stop_mask) ? 1ull : 0ull);
+                if (len == 0) {
+                    pfa_cds_win_add(a, q, PFA_CDS_MISSING, j, 3ull);
+                } else {
+                    const unsigned tot3 = (unsigned)__popcll(P & c_syn3_bits[0]) + 2u * (unsigned)__popcll(P & c_syn3_bits[1]) +
+                                          4u * (unsigned)__popcll(P & c_syn3_bits[2]);
+                    pfa_cds_win_add(a, q, PFA_CDS_SUM3 + len, j, tot3);
+                }
+            }
+        }
+        if (a.has_partial && lo <= a.ncf * 3 && a.ncf * 3 < hi) u_missing += 3;  // :305 for the trailing 1-2 sites
+        for (int q = lane; q < k; q += 32) {
+            pfa_cds_win_add(a, q, PFA_CDS_NSTOPS, j, u_nstops);
+            pfa_cds_win_add(a, q, PFA_CDS_MISSING, j, u_missing);
+            pfa_cds_win_add(a, q, PFA_CDS_SUM3 + 1, j, u_sum3);
+        }
+    }
+}
+
+int pfa_launch_cds_window_bins(pfa_aln* a, const int64_t* d_hsite, const uint8_t* d_labels, int64_t g, int64_t b0, int64_t nb, int64_t* d_bins) {
+    pfa_ctx* ctx = a->ctx;
+    if (!ctx->codon_tables_ready) {
+        int rc = pfa_upload_codon_tables(ctx);
+        if (rc) return rc;
+        ctx->codon_tables_ready = true;
+    }
+    if (a->ns == 0 || nb == 0) return PFA_OK;
+    PfaCdsWinArgs args;
+    pfa_fill_site_args(a, nullptr, nullptr, &args.s);
+    args.s.vflag = a->vflag;  // a column whose three sites have no flagged cell is all valid: its validity records are not read
+    args.hsite = d_hsite;
+    args.labels = d_labels;
+    args.bins = d_bins;
+    args.c0 = a->col_begin;
+    args.g = g;
+    args.b0 = b0;
+    args.nb = nb;
+    args.mpb = (g + PFA_CDS_WIN_PIECE - 1) / PFA_CDS_WIN_PIECE;
+    args.ncf = a->ns / 3;
+    args.has_partial = (a->ns % 3) != 0;
+    const int64_t warps = nb * args.mpb;
+    const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((warps + 7) / 8, (int64_t)ctx->sm_count * 8));
+    if (a->has_invalid) pfa_cds_window_bins_kernel<true><<<grid, 256, 0, ctx->stream>>>(args);
+    else pfa_cds_window_bins_kernel<false><<<grid, 256, 0, ctx->stream>>>(args);
+    PFA_LAUNCH_CHECK(ctx);
+    return PFA_OK;
+}

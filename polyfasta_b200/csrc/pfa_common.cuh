@@ -141,6 +141,10 @@ int pfa_launch_row_windows(pfa_aln* a, int rows, const int64_t* d_persite, int64
 int pfa_launch_var_flags(pfa_aln* a, uint8_t* flags);
 int pfa_launch_window_final_in(pfa_aln* a, const int64_t* d_counts, int64_t window, int64_t step, int jc, pfa_final_in* d_in);
 int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg* x = nullptr);
+// codon windows: bins [k][PFA_CDS_WIN_LEN][nb] (zeroed) of this shard from K2's per-site H and K4's labels (pfa_codon.cu), and
+// the window vectors [k][nwin][PFA_CDS_WIN_LEN] from them (pfa_windows.cu)
+int pfa_launch_cds_window_bins(pfa_aln* a, const int64_t* d_hsite, const uint8_t* d_labels, int64_t g, int64_t b0, int64_t nb, int64_t* d_bins);
+int pfa_launch_cds_windows(pfa_aln* a, const int64_t* d_hsite, const uint8_t* d_labels, int64_t window, int64_t step, int64_t* d_counts);
 int pfa_xchg_fill(pfa_xchg* x, int64_t len, int64_t* d_out, PfaXchgDev* dev, bool coresident = false);
 unsigned long long* pfa_xchg_partial(pfa_xchg* x);
 void pfa_xchg_commit(pfa_xchg* x);

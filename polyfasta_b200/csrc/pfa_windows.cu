@@ -12,6 +12,9 @@
 //   3. each window is the difference of two prefix sums.
 // Only the columns of this shard contribute (bins are clipped to the shard), so the vectors of the column shards of an
 // alignment add up to the whole alignment's.  All arithmetic is exact int64.
+// The codon windows (pfa_cds_windows_device) reduce the same way: pfa_cds_window_bins_kernel (pfa_codon.cu, next to the codon
+// tables) fills PFA_CDS_WIN_LEN words per (population, bin), one exclusive sum runs over all of them and every window word is
+// the difference of two prefix sums: O(k ns + k 72 nwin) work whatever W and step are.
 #include <algorithm>
 #include <climits>
 
@@ -187,6 +190,56 @@ int pfa_launch_window_final_in(pfa_aln* a, const int64_t* d_counts, int64_t wind
     pfa_window_final_in_kernel<<<pfa_win_grid(ctx, nout), 256, 0, ctx->stream>>>(d_counts, a->d_pop_n, a->L_total, window, step, jc ? 1 : 0, a->k,
                                                                                   nwin, d_in);
     PFA_LAUNCH_CHECK(ctx);
+    return PFA_OK;
+}
+
+// codon windows: counts[(q nwin + i) PFA_CDS_WIN_LEN + w] = word w of this shard's columns of window i; pre = exclusive prefix
+// sums of the bins [k][PFA_CDS_WIN_LEN][nb] (one row of nb bins per (population, word))
+__global__ void __launch_bounds__(256) pfa_cds_window_counts_kernel(const long long* __restrict__ pre, int64_t L, int64_t W, int64_t step, int64_t g,
+                                                                    int64_t b0, int64_t nb, int k, int64_t nwin, int64_t* __restrict__ counts) {
+    const int64_t total = (int64_t)k * nwin * PFA_CDS_WIN_LEN;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t qi = e / PFA_CDS_WIN_LEN, w = e - qi * PFA_CDS_WIN_LEN, q = qi / nwin, i = qi - q * nwin;
+        const int64_t ws = i * step, we = min(ws + W, L);
+        const int64_t lo = min(max(ws / g - b0, (int64_t)0), nb), hi = min(max((we + g - 1) / g - b0, (int64_t)0), nb);
+        const long long* row = pre + (q * PFA_CDS_WIN_LEN + w) * nb;
+        counts[e] = hi > lo ? row[hi] - row[lo] : 0;
+    }
+}
+
+int pfa_launch_cds_windows(pfa_aln* a, const int64_t* d_hsite, const uint8_t* d_labels, int64_t window, int64_t step, int64_t* d_counts) {
+    pfa_ctx* ctx = a->ctx;
+    const int64_t nwin = pfa_window_count(a->L_total, window, step);
+    const int64_t nout = (int64_t)a->k * nwin;
+    if (nout == 0) return PFA_OK;
+    const PfaWinGeom w = pfa_win_geom(a, window, step);
+    const int64_t nbins = (int64_t)a->k * PFA_CDS_WIN_LEN * w.nb;
+    if (nbins == 0) {  // an empty shard contributes nothing
+        PFA_CUDA(ctx, cudaMemsetAsync(d_counts, 0, sizeof(int64_t) * PFA_CDS_WIN_LEN * (size_t)nout, ctx->stream));
+        return PFA_OK;
+    }
+    if (nbins + 1 > INT_MAX)
+        return pfa_fail(ctx, PFA_ERR_ARG, "cds windows: %lld bin words of %lld columns exceed the scan's range", (long long)nbins, (long long)w.g);
+    long long* bins = nullptr;  // scanned in place; the word past the last bin becomes the total
+    void* tmp = nullptr;
+    size_t tmp_bytes = 0;
+    cudaError_t e = pfa_dmalloc(ctx, &bins, sizeof(long long) * (size_t)(nbins + 1));
+    if (e == cudaSuccess) e = cudaMemsetAsync(bins, 0, sizeof(long long) * (size_t)(nbins + 1), ctx->stream);
+    int rc = e == cudaSuccess ? pfa_launch_cds_window_bins(a, d_hsite, d_labels, w.g, w.b0, w.nb, reinterpret_cast<int64_t*>(bins)) : PFA_OK;
+    if (!rc && e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, bins, (int)(nbins + 1), ctx->stream);
+    if (!rc && e == cudaSuccess) e = pfa_dmalloc(ctx, &tmp, tmp_bytes);
+    if (!rc && e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, bins, (int)(nbins + 1), ctx->stream);
+    if (!rc && e == cudaSuccess) {
+        ctx->launches++;
+        pfa_cds_window_counts_kernel<<<pfa_win_grid(ctx, nout * PFA_CDS_WIN_LEN), 256, 0, ctx->stream>>>(bins, a->L_total, window, step, w.g, w.b0,
+                                                                                                          w.nb, a->k, nwin, d_counts);
+        ctx->launches++;
+        e = cudaGetLastError();
+    }
+    pfa_dfree(ctx, tmp);
+    pfa_dfree(ctx, bins);
+    if (rc) return rc;
+    if (e != cudaSuccess) return pfa_fail(ctx, PFA_ERR_CUDA, "cds windows: %s", cudaGetErrorString(e));
     return PFA_OK;
 }
 
