@@ -304,9 +304,8 @@ int64_t pfa_window_count(int64_t L, int64_t window, int64_t step);
  * coordinates (nwin from the whole alignment's length): the vectors of the column shards of an alignment add up to the whole
  * alignment's (pfa_xchg_allreduce).  Runs the site scan with the per-site H into scratch memory of the device pool. */
 int pfa_site_windows_device(pfa_aln* a, int64_t window, int64_t step, int64_t* d_counts);
-/* synchronous: counts (host) = int64 [k][nwin][2] as above; fin (host, optional) = pfa_final_out [k][nwin], the K5 outputs of
- * every (population, window).  window < 1 or step < 1: PFA_ERR_ARG. */
-int pfa_site_windows(pfa_aln* a, int64_t window, int64_t step, int jc, int64_t* counts, pfa_final_out* fin /* optional */);
+/* synchronous: counts (host) = int64 [k][nwin][2] as above.  window < 1 or step < 1: PFA_ERR_ARG. */
+int pfa_site_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* counts);
 
 /* ---- synonymous and nonsynonymous statistics in sliding windows (beyond the reference: --cds --window) --------------------
  * Windows as above; window and step must be multiples of 3, so that no codon column straddles a window boundary, and a column
@@ -319,7 +318,7 @@ int pfa_site_windows(pfa_aln* a, int64_t window, int64_t step, int jc, int64_t* 
 /* asynchronous: d_counts (device) = int64 [k][nwin][PFA_CDS_WIN_LEN] of THIS SHARD's columns, in global window coordinates: the
  * vectors of the column shards add up to the whole alignment's.  Runs the site scan with the per-site H and the codon scan with
  * the labels, then one pass over the shard's codon columns into bins of gcd(window, step) columns and a prefix sum over the
- * bins.  Device scratch from the pool: k * nsites * 9 bytes (labels and per-site H) plus k * 72 * (nbins + 1) * 8 bytes, nbins =
+ * bins.  Device scratch from the pool: k * nsites * 9 bytes (labels and per-site H) plus (k * 72 * nbins + 1) * 8 bytes, nbins =
  * the shard's bins of gcd(window, step) columns. */
 int pfa_cds_windows_device(pfa_aln* a, int64_t window, int64_t step, int64_t* d_counts);
 /* synchronous: counts (host) = int64 [k][nwin][PFA_CDS_WIN_LEN] as above */
@@ -354,12 +353,11 @@ int pfa_divergence_windows_device(pfa_aln* a, int64_t window, int64_t step, int6
  * when x > 0 (K5's rule for pi); hw = 0.5 (pi_x + pi_y); da = dxy - hw; fst = 1 - hw / dxy (Hudson, Slatkin & Maddison 1992,
  * the estimator of Bhatia et al. 2013), fst_is_NA when dxy == 0 */
 int pfa_div_finalize(pfa_ctx* ctx, const pfa_div_in* in, pfa_div_out* out, int count);
-/* synchronous: counts (host) = int64 [P] D_xy of the whole alignment (of this shard for a column shard); out (host, optional) =
- * pfa_div_out [P], with pi of every population from the site scan and K5 (seqlen = the alignment's length) */
-int pfa_divergence(pfa_aln* a, int jc, int64_t* counts, pfa_div_out* out /* optional */);
-/* synchronous: counts (host) = int64 [P][nwin] D_xy of every (pair, window); out (host, optional) = pfa_div_out [P][nwin], with
- * pi of every (population, window) from pfa_site_windows.  window < 1 or step < 1: PFA_ERR_ARG. */
-int pfa_divergence_windows(pfa_aln* a, int64_t window, int64_t step, int jc, int64_t* counts, pfa_div_out* out /* optional */);
+/* synchronous: counts (host) = int64 [P] D_xy of the whole alignment (of this shard for a column shard) */
+int pfa_divergence(pfa_aln* a, int64_t* counts);
+/* synchronous: counts (host) = int64 [P][nwin][2] as pfa_divergence_windows_device gives it.  window < 1 or step < 1:
+ * PFA_ERR_ARG. */
+int pfa_divergence_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* counts);
 
 #ifdef __cplusplus
 }

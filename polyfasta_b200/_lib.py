@@ -128,14 +128,14 @@ def lib():
         "pfa_site_stats_hsite": (c.c_int, [p, p, p, p]),
         "pfa_window_count": (i64, [i64, i64, i64]),
         "pfa_site_windows_device": (c.c_int, [p, i64, i64, p]),
-        "pfa_site_windows": (c.c_int, [p, i64, i64, c.c_int, p, p]),
+        "pfa_site_windows": (c.c_int, [p, i64, i64, p]),
         "pfa_cds_windows_device": (c.c_int, [p, i64, i64, p]),
         "pfa_cds_windows": (c.c_int, [p, i64, i64, p]),
         "pfa_divergence_device": (c.c_int, [p, p]),
         "pfa_divergence_windows_device": (c.c_int, [p, i64, i64, p]),
         "pfa_div_finalize": (c.c_int, [p, c.POINTER(DivIn), c.POINTER(DivOut), c.c_int]),
-        "pfa_divergence": (c.c_int, [p, c.c_int, p, p]),
-        "pfa_divergence_windows": (c.c_int, [p, i64, i64, c.c_int, p, p]),
+        "pfa_divergence": (c.c_int, [p, p]),
+        "pfa_divergence_windows": (c.c_int, [p, i64, i64, p]),
         "pfa_cds_stats_device": (c.c_int, [p, p, p]),
         "pfa_cds_stats": (c.c_int, [p, p, p]),
         "pfa_codon_pair_labels": (c.c_int, [c.c_int, c.c_int]),

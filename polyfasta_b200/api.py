@@ -123,30 +123,82 @@ def window_count(L, window, step):
     return n
 
 
+def cds_results(ctx, rows):
+    """codon vectors int64 [m][>= PFA_CDS_LEN] (pfa_cds_stats' [k][PFA_CDS_LEN], codon window vectors, or their sums over column
+    shards) -> list of dict(nstops, missing, S_s, H_s, S_n, H_n, sum3_by_len, ssites, raw) per row; raw is the row as given"""
+    rows = np.asarray(rows, dtype=np.int64)
+    res = []
+    for row, ss in zip(rows, ctx.cds_ssites(rows[:, :PFA_CDS_LEN])):
+        d = Alignment.unpack_cds(row)
+        d["ssites"] = float(ss)
+        d["raw"] = row.copy()
+        res.append(d)
+    return res
+
+
+def site_window_results(ctx, counts, sizes, L, window, step, jc):
+    """(S, H) vectors int64 [k][nwin][2] of an alignment of L columns (pfa_site_windows, or the sum over its column shards) ->
+    the list Alignment.site_windows returns; every window is finalised by K5 (Context.finalize) with seqlen = its length"""
+    counts = np.asarray(counts, dtype=np.int64)
+    k, nwin = counts.shape[0], counts.shape[1]
+    spans = [(i * step, min(i * step + window, L)) for i in range(nwin)]
+    fin = iter(ctx.finalize((sizes[q], counts[q, i, 0], counts[q, i, 1], end - start, jc)
+                            for i, (start, end) in enumerate(spans) for q in range(k)))
+    return [{"start": start, "end": end, "seqlen": end - start,
+             "pops": [{"n": sizes[q], "S": int(counts[q, i, 0]), "H": int(counts[q, i, 1]), "poly": next(fin)} for q in range(k)]}
+            for i, (start, end) in enumerate(spans)]
+
+
 def cds_window_results(ctx, counts, sizes, L, window, step, jc):
     """codon window vectors int64 [k][nwin][PFA_CDS_WIN_LEN] of an alignment of L columns (pfa_cds_windows, or the sum over its
-    column shards) -> the list Alignment.cds_windows returns; ssites and the K5 entries come from Context.cds_ssites and
+    column shards) -> the list Alignment.cds_windows returns; ssites and the K5 entries come from cds_results and
     Context.finalize exactly as for the --cds row of the window's columns"""
     counts = np.asarray(counts, dtype=np.int64)
     k, nwin = counts.shape[0], counts.shape[1]
-    ss = ctx.cds_ssites(counts[:, :, :PFA_CDS_LEN].reshape(-1, PFA_CDS_LEN)).reshape(k, nwin) if k * nwin else None
+    cds = cds_results(ctx, counts.reshape(k * nwin, PFA_CDS_WIN_LEN))
     res, items = [], []
     for i in range(nwin):
         start, end = i * step, min(i * step + window, L)
         pops = []
         for q in range(k):
-            row = counts[q, i]
-            c = Alignment.unpack_cds(row)
-            c["ssites"] = float(ss[q, i])
+            c = cds[q * nwin + i]
             c["nsites"] = ((end - start) - c["missing"]) - c["ssites"]
-            c["raw"] = row.copy()
             items += [(sizes[q], c["S_s"], c["H_s"], c["ssites"], jc), (sizes[q], c["S_n"], c["H_n"], c["nsites"], jc)]
-            pops.append({"n": sizes[q], "S": int(row[PFA_CDS_LEN]), "cds": c})
+            pops.append({"n": sizes[q], "S": int(c["raw"][PFA_CDS_LEN]), "cds": c})
         res.append({"start": start, "end": end, "pops": pops})
     fin = iter(ctx.finalize(items))
     for w in res:
         for p in w["pops"]:
             p["poly_s"], p["poly_n"] = next(fin), next(fin)
+    return res
+
+
+def divergence_results(ctx, site, D, sizes, L, jc):
+    """the site scan's results per population (Alignment.site_stats / unpack_site) and D_xy int64 [P] of an alignment of L
+    columns (pfa_divergence, or the sums over its column shards) -> the list Alignment.divergence returns"""
+    pairs = pop_pairs(len(sizes))
+    pis = [p[1] for p in ctx.finalize((sizes[q], s["S"], s["H"], L, jc) for q, s in enumerate(site))]
+    fin = ctx.div_finalize((sizes[x], sizes[y], int(D[p]), L, pis[x], pis[y], jc) for p, (x, y) in enumerate(pairs))
+    return [{"x": x, "y": y, "n_x": sizes[x], "n_y": sizes[y], "D": int(D[p]), "pi_x": pis[x], "pi_y": pis[y],
+             "dxy": fin[p][0], "da": fin[p][1], "fst": fin[p][2]} for p, (x, y) in enumerate(pairs)]
+
+
+def divergence_window_results(ctx, site_counts, div_counts, sizes, L, window, step, jc):
+    """(S, H) int64 [k][nwin][2] and (columns, D_xy) int64 [P][nwin][2] of an alignment of L columns (pfa_site_windows and
+    pfa_divergence_windows, or their sums over column shards) -> the list Alignment.divergence_windows returns; pi of every
+    (population, window) comes from site_window_results"""
+    wins = site_window_results(ctx, site_counts, sizes, L, window, step, jc)
+    pairs = pop_pairs(len(sizes))
+    D = np.asarray(div_counts, dtype=np.int64)[:, :, 1]
+    fin = iter(ctx.div_finalize((sizes[x], sizes[y], int(D[p, i]), w["seqlen"], w["pops"][x]["poly"][1], w["pops"][y]["poly"][1], jc)
+                                for i, w in enumerate(wins) for p, (x, y) in enumerate(pairs)))
+    res = []
+    for i, w in enumerate(wins):
+        row = []
+        for p, (x, y) in enumerate(pairs):
+            dxy, da, fst = next(fin)
+            row.append({"x": x, "y": y, "D": int(D[p, i]), "dxy": dxy, "da": da, "fst": fst})
+        res.append({"start": w["start"], "end": w["end"], "seqlen": w["seqlen"], "pairs": row})
     return res
 
 
@@ -435,6 +487,12 @@ class Alignment:
         return [{"n": sizes[q], "S": int(vec[off[q]]), "H": int(vec[off[q] + 1]),
                  "sfs": [int(x) for x in vec[off[q] + 2: off[q + 1]]]} for q in range(len(sizes))]
 
+    def site_counts(self):
+        """int64 [site_len()]: the site scan's vector (pfa_site_stats; unpack_site reads it)"""
+        out = np.zeros(max(self.site_len(), 1), dtype=np.int64)
+        check(lib().pfa_site_stats(self.handle, out.ctypes.data, None), self.ctx.handle)
+        return out
+
     def site_stats(self, want_isvar=False, want_hsite=False):
         """K2 -> list of dict(n, S, H, sfs[, isvar][, hsite]) per population; hsite: int64 per site of this shard, the column's
         n^2 - sum_a c_a^2 where it is variable in the population, 0 elsewhere"""
@@ -465,24 +523,14 @@ class Alignment:
         step = window if step is None else step
         if window < 1 or step < 1:
             raise ValueError("window and step must be >= 1")
+        return site_window_results(self.ctx, self.site_window_counts(window, step), self.pop_sizes(), self.total_len, window, step, jc)
+
+    def site_window_counts(self, window, step):
+        """int64 [k][nwin][2]: (S, H) of this shard's columns of every (population, window) (pfa_site_windows)"""
         nwin = self.window_count(window, step)
-        k = self.num_pops
-        counts = np.zeros((k, max(nwin, 1), 2), dtype=np.int64)
-        fin = (FinalOut * max(k * nwin, 1))()
-        check(lib().pfa_site_windows(self.handle, int(window), int(step), int(bool(jc)), counts.ctypes.data, fin), self.ctx.handle)
-        sizes = self.pop_sizes()
-        res = []
-        for i in range(nwin):
-            start = i * step
-            end = min(start + window, self.total_len)
-            pops = []
-            for q in range(k):
-                S, H = int(counts[q, i, 0]), int(counts[q, i, 1])
-                o = fin[q * nwin + i]
-                poly = (0, 0, 0, "NA") if o.no_var else (S, o.pi_site, o.theta_site, "NA" if o.D_is_NA else o.D)
-                pops.append({"n": sizes[q], "S": S, "H": H, "poly": poly})
-            res.append({"start": start, "end": end, "seqlen": end - start, "pops": pops})
-        return res
+        counts = np.zeros((self.num_pops, max(nwin, 1), 2), dtype=np.int64)
+        check(lib().pfa_site_windows(self.handle, int(window), int(step), counts.ctypes.data), self.ctx.handle)
+        return counts[:, :nwin]
 
     def site_windows_device(self, window, step, d_ptr):
         """asynchronous: int64 [k][nwin][2] (S, H) of this shard's columns of every window into caller device memory; the
@@ -499,10 +547,14 @@ class Alignment:
         step = window if step is None else step
         if window < 1 or step < 1 or window % 3 or step % 3:
             raise ValueError("cds windows: window and step must be positive multiples of 3")
+        return cds_window_results(self.ctx, self.cds_window_counts(window, step), self.pop_sizes(), self.total_len, window, step, jc)
+
+    def cds_window_counts(self, window, step):
+        """int64 [k][nwin][PFA_CDS_WIN_LEN]: the codon window vectors of this shard's columns (pfa_cds_windows)"""
         nwin = self.window_count(window, step)
         counts = np.zeros((self.num_pops, max(nwin, 1), PFA_CDS_WIN_LEN), dtype=np.int64)
         check(lib().pfa_cds_windows(self.handle, int(window), int(step), counts.ctypes.data), self.ctx.handle)
-        return cds_window_results(self.ctx, counts[:, :nwin], self.pop_sizes(), self.total_len, window, step, jc)
+        return counts[:, :nwin]
 
     def cds_windows_device(self, window, step, d_ptr):
         """asynchronous: int64 [k][nwin][PFA_CDS_WIN_LEN] codon window vectors of this shard's columns into caller device memory;
@@ -514,15 +566,13 @@ class Alignment:
         list of dict(x, y, n_x, n_y, D, pi_x, pi_y, dxy, da, fst).  D is the exact number of (row of x, row of y, column)
         triples whose characters differ; pi_x / pi_y are pi_site of the two populations (0 without variable sites); fst is "NA"
         where dxy == 0 (dxy, da and fst are all "NA" for an empty population).  For a column shard D is the shard's part."""
-        k = self.num_pops
-        pairs = pop_pairs(k)
-        D = np.zeros(max(len(pairs), 1), dtype=np.int64)
-        check(lib().pfa_divergence(self.handle, int(bool(jc)), D.ctypes.data, None), self.ctx.handle)
-        sizes = self.pop_sizes()
-        pis = [p[1] for p in self.ctx.finalize((s["n"], s["S"], s["H"], self.total_len, jc) for s in self.site_stats())]
-        fin = self.ctx.div_finalize((sizes[x], sizes[y], int(D[p]), self.total_len, pis[x], pis[y], jc) for p, (x, y) in enumerate(pairs))
-        return [{"x": x, "y": y, "n_x": sizes[x], "n_y": sizes[y], "D": int(D[p]), "pi_x": pis[x], "pi_y": pis[y],
-                 "dxy": fin[p][0], "da": fin[p][1], "fst": fin[p][2]} for p, (x, y) in enumerate(pairs)]
+        return divergence_results(self.ctx, self.site_stats(), self.divergence_counts(), self.pop_sizes(), self.total_len, jc)
+
+    def divergence_counts(self):
+        """int64 [P]: D_xy of this shard's columns of every pair (pfa_divergence)"""
+        D = np.zeros(max(len(pop_pairs(self.num_pops)), 1), dtype=np.int64)
+        check(lib().pfa_divergence(self.handle, D.ctypes.data), self.ctx.handle)
+        return D
 
     def divergence_windows(self, window, step=None, jc=False):
         """divergence in windows of `window` columns every `step` (default: `window`), as site_windows ->
@@ -531,24 +581,16 @@ class Alignment:
         step = window if step is None else step
         if window < 1 or step < 1:
             raise ValueError("window and step must be >= 1")
-        nwin = self.window_count(window, step)
-        pairs = pop_pairs(self.num_pops)
-        D = np.zeros((max(len(pairs), 1), max(nwin, 1)), dtype=np.int64)
-        check(lib().pfa_divergence_windows(self.handle, int(window), int(step), int(bool(jc)), D.ctypes.data, None), self.ctx.handle)
-        D = D.reshape(-1)[: len(pairs) * nwin].reshape(len(pairs), nwin)
-        sizes = self.pop_sizes()
-        wins = self.site_windows(window, step, jc)
-        items = [(sizes[x], sizes[y], int(D[p, i]), w["seqlen"], w["pops"][x]["poly"][1], w["pops"][y]["poly"][1], jc)
-                 for i, w in enumerate(wins) for p, (x, y) in enumerate(pairs)]
-        fin = iter(self.ctx.div_finalize(items))
-        res = []
-        for i, w in enumerate(wins):
-            row = []
-            for p, (x, y) in enumerate(pairs):
-                dxy, da, fst = next(fin)
-                row.append({"x": x, "y": y, "D": int(D[p, i]), "dxy": dxy, "da": da, "fst": fst})
-            res.append({"start": w["start"], "end": w["end"], "seqlen": w["seqlen"], "pairs": row})
-        return res
+        return divergence_window_results(self.ctx, self.site_window_counts(window, step), self.divergence_window_counts(window, step),
+                                         self.pop_sizes(), self.total_len, window, step, jc)
+
+    def divergence_window_counts(self, window, step):
+        """int64 [P][nwin][2]: (columns with a difference, D_xy) of this shard's columns of every (pair, window)
+        (pfa_divergence_windows)"""
+        P, nwin = len(pop_pairs(self.num_pops)), self.window_count(window, step)
+        counts = np.zeros((max(P, 1), max(nwin, 1), 2), dtype=np.int64)
+        check(lib().pfa_divergence_windows(self.handle, int(window), int(step), counts.ctypes.data), self.ctx.handle)
+        return counts[:P, :nwin]
 
     def divergence_device(self, d_ptr):
         """asynchronous: int64 [P] D_xy of this shard of every pair into caller device memory; the vectors of the column shards
@@ -591,16 +633,17 @@ class Alignment:
         out = np.zeros((k, PFA_CDS_LEN), dtype=np.int64)
         labels = np.zeros((k, max(self.nsites, 1)), dtype=np.uint8) if want_labels else None
         check(lib().pfa_cds_stats(self.handle, out.ctypes.data, labels.ctypes.data if want_labels else None), self.ctx.handle)
-        ss = self.ctx.cds_ssites(out)
-        res = []
-        for q in range(k):
-            d = self.unpack_cds(out[q])
-            d["ssites"] = float(ss[q])
-            d["raw"] = out[q].copy()
-            if want_labels:
+        res = cds_results(self.ctx, out)
+        if want_labels:
+            for q, d in enumerate(res):
                 d["labels"] = labels.reshape(-1)[: k * self.nsites].reshape(k, self.nsites)[q] if self.nsites else labels[q, :0]
-            res.append(d)
         return res
+
+    def cds_counts(self):
+        """int64 [k][PFA_CDS_LEN]: the codon scan's vectors (pfa_cds_stats; cds_results reads them)"""
+        out = np.zeros((self.num_pops, PFA_CDS_LEN), dtype=np.int64)
+        check(lib().pfa_cds_stats(self.handle, out.ctypes.data, None), self.ctx.handle)
+        return out
 
     def cds_stats_device(self, d_out_ptr, d_labels_ptr=None):
         check(lib().pfa_cds_stats_device(self.handle, ctypes.c_void_p(d_out_ptr), ctypes.c_void_p(d_labels_ptr or 0)),

@@ -151,6 +151,21 @@ class Sink:
             print(line)
 
 
+def poly_tail(S, poly):
+    """the tail of a default or window row: S of the site scan, poly the tuple Context.finalize returns"""
+    if S == 0:
+        return ",0,0,0,NA"                                                                     # PolyFastA.py:187/:189
+    return f",{poly[0]},{poly[1]},{poly[2]},{poly[3]}"                                         # :196/:198
+
+
+def cds_tail(S, poly_s, poly_n, nstops):
+    """the tail of a --cds or codon-window row: S of the site scan, poly_s / poly_n the synonymous / nonsynonymous tuples"""
+    if S == 0:
+        return ",0,0,0,NA,0,0,0,NA,0"                                                          # PolyFastA.py:160/:162
+    s, m = poly_s, poly_n
+    return f",{s[0]},{m[0]},{s[1]},{m[1]},{s[2]},{m[2]},{s[3]},{m[3]},{nstops}"                 # :178/:180
+
+
 def format_rows(ctx, file, seqlen, cds, jc, pops, site, cdsst):
     """rows of print_result.no_header (PolyFastA.py:148-198) for the populations of one alignment.
     pops: list of (label, n); site: K2 results per population; cdsst: K4 results per population or None."""
@@ -158,51 +173,34 @@ def format_rows(ctx, file, seqlen, cds, jc, pops, site, cdsst):
     for q, (label, n) in enumerate(pops):
         if cds:
             c = cdsst[q]
-            ssites = c["ssites"]
-            nsites = (seqlen - c["missing"]) - ssites
+            nsites = (seqlen - c["missing"]) - c["ssites"]
             if site[q]["S"]:
-                todo.append((n, c["S_s"], c["H_s"], ssites, jc))
+                todo.append((n, c["S_s"], c["H_s"], c["ssites"], jc))
                 todo.append((n, c["S_n"], c["H_n"], nsites, jc))
         elif site[q]["S"]:
             todo.append((n, site[q]["S"], site[q]["H"], seqlen, jc))
     fin = iter(ctx.finalize(todo))
     lines = []
     for q, (label, n) in enumerate(pops):
+        S = site[q]["S"]
         if cds:
-            c = cdsst[q]
-            ssites = c["ssites"]
-            nsites = (seqlen - c["missing"]) - ssites
-            head = f"{file},{round(ssites, 2)},{round(nsites, 2)},{label},{n}"
-            if site[q]["S"] == 0:
-                lines.append(head + ",0,0,0,NA,0,0,0,NA,0")                                   # :160/:162
-            else:
-                s, m = next(fin), next(fin)
-                lines.append(head + f",{s[0]},{m[0]},{s[1]},{m[1]},{s[2]},{m[2]},{s[3]},{m[3]},{c['nstops']}")  # :178/:180
-        elif site[q]["S"] == 0:
-            lines.append(f"{file},{seqlen},{label},{n},0,0,0,NA")                              # :187/:189
+            s, m = (next(fin), next(fin)) if S else (None, None)
+            lines.append(cds_line(file, seqlen, label, n, S, cdsst[q], s, m))
         else:
-            r = next(fin)
-            lines.append(f"{file},{seqlen},{label},{n},{r[0]},{r[1]},{r[2]},{r[3]}")           # :196/:198
+            lines.append(f"{file},{seqlen},{label},{n}" + poly_tail(S, next(fin) if S else None))
     return lines
 
 
 def window_rows(file, found, wins):
-    """rows of one alignment in windows: wins = [(start, end, [(S, poly) per population])], start 0-based, end exclusive.
-    Window by window, the populations in order; each row is the row format_rows gives for the window's columns alone, with
-    the window's 1-based inclusive coordinates in front of seqlen (the window's length)."""
-    lines = []
-    for start, end, per_pop in wins:
-        for (label, _, n), (S, r) in zip(found, per_pop):
-            head = f"{file},{start + 1},{end},{end - start},{label},{n}"
-            if S == 0:
-                lines.append(head + ",0,0,0,NA")                                                   # :187/:189
-            else:
-                lines.append(head + f",{r[0]},{r[1]},{r[2]},{r[3]}")                               # :196/:198
-    return lines
+    """rows of one alignment in windows: wins = the list api.site_window_results returns.  Window by window, the populations in
+    order; each row is the row format_rows gives for the window's columns alone, with the window's 1-based inclusive
+    coordinates in front of seqlen (the window's length)."""
+    return [f"{file},{w['start'] + 1},{w['end']},{w['seqlen']},{label},{n}" + poly_tail(p["S"], p["poly"])
+            for w in wins for (label, _, n), p in zip(found, w["pops"])]
 
 
 def cds_window_rows(file, found, wins):
-    """--cds rows of one alignment in windows: wins = the list Alignment.cds_windows returns.  Window by window, the populations
+    """--cds rows of one alignment in windows: wins = the list api.cds_window_results returns.  Window by window, the populations
     in order; each row is the --cds row format_rows gives for the window's columns alone, with the window's 1-based inclusive
     coordinates after the file's name"""
     lines = []
@@ -210,23 +208,22 @@ def cds_window_rows(file, found, wins):
         for (label, _, n), p in zip(found, w["pops"]):
             c = p["cds"]
             head = f"{file},{w['start'] + 1},{w['end']},{round(c['ssites'], 2)},{round(c['nsites'], 2)},{label},{n}"
-            if p["S"] == 0:
-                lines.append(head + ",0,0,0,NA,0,0,0,NA,0")                                     # :160/:162
-            else:
-                s, m = p["poly_s"], p["poly_n"]
-                lines.append(head + f",{s[0]},{m[0]},{s[1]},{m[1]},{s[2]},{m[2]},{s[3]},{m[3]},{c['nstops']}")  # :178/:180
+            lines.append(head + cds_tail(p["S"], p["poly_s"], p["poly_n"], c["nstops"]))
     return lines
 
 
 def dxy_rows(file, found, wins, windowed):
-    """--dxy rows of one alignment: wins = [(start, end, [(dxy, da, fst) per pair])], start 0-based, end exclusive; the pairs in
-    api.pop_pairs order.  windowed: the window's 1-based inclusive coordinates go in front of seqlen (the window's length)"""
+    """--dxy rows of one alignment: wins = [dict(start, end, pairs=[dict(dxy, da, fst)])] (the list
+    api.divergence_window_results returns, or the whole alignment's api.divergence_results as one window), start 0-based, end
+    exclusive; the pairs in api.pop_pairs order.  windowed: the window's 1-based inclusive coordinates go in front of seqlen
+    (the window's length)"""
     pairs = api.pop_pairs(len(found))
     lines = []
-    for start, end, fins in wins:
+    for w in wins:
+        start, end = w["start"], w["end"]
         head = f"{file},{start + 1},{end},{end - start}" if windowed else f"{file},{end - start}"
-        for (x, y), (dxy, da, fst) in zip(pairs, fins):
-            lines.append(head + f",{found[x][0]},{found[y][0]},{found[x][2]},{found[y][2]},{dxy},{da},{fst}")
+        for (x, y), d in zip(pairs, w["pairs"]):
+            lines.append(head + f",{found[x][0]},{found[y][0]},{found[x][2]},{found[y][2]},{d['dxy']},{d['da']},{d['fst']}")
     return lines
 
 
@@ -291,158 +288,46 @@ class RankGroup:
 XCHG_MAX_WORDS = 1 << 28   # the longest vector an exchange takes (pfa_xchg_create); longer window vectors go through the host
 
 
-def sum_over_ranks(ctx, group, words, launch):
-    """launch(d_ptr) writes this rank's int64 vector of `words` words into device memory; returns the sum over the ranks as a
-    host tensor (the exchange, or the host collective when the group is not fused or the vector is longer than an exchange takes)"""
+def sum_over_ranks(ctx, group, parts, fused=None):
+    """parts: [(words, launch(d_ptr))], each launch writing this rank's int64 vector of `words` words into device memory;
+    returns the sums over the ranks as host arrays, one per part.  The vectors travel in one exchange, or through the host
+    collective when the group is not fused or they are longer than an exchange takes.  fused(xchg, d_ptr): one launch that
+    computes every part and sums it over the ranks itself (the scan kernels' own exchange)."""
     import torch
+    offs = [0]
+    for n, _ in parts:
+        offs.append(offs[-1] + n)
+    words = max(offs[-1], 1)
     d_cnt = torch.zeros(words, dtype=torch.int64, device="cuda:%d" % ctx.device)
+    d = d_cnt.data_ptr()
+
+    def launch():
+        for off, (_, part) in zip(offs, parts):
+            part(d + 8 * off)
+
     torch.cuda.synchronize(ctx.device)
     if group.fused and words <= XCHG_MAX_WORDS:
         x = group.exchange(ctx, words)
+        # the ranks meet on the host AFTER their uploads (parse + ingest times differ by seconds on cold files), so the wait
+        # inside the kernels only has to cover launch skew
         ctx.sync()
         group.dist.barrier()
-        launch(d_cnt.data_ptr())
-        x.allreduce(d_cnt.data_ptr(), words)
+        if fused is not None:
+            fused(x, d)
+        else:
+            launch()
+            x.allreduce(d, words)
         ctx.sync()
         if x.timed_out():
             raise api.PolyFastaError(1, "a rank did not arrive at the exchange")
-        return d_cnt.cpu()
-    launch(d_cnt.data_ptr())
-    ctx.sync()
-    h = d_cnt.cpu()
-    group.dist.all_reduce(h)
-    return h
-
-
-def sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window):
-    """--window over column shards: every rank computes its shard's (S, H) per (population, window), the vectors are summed
-    over the ranks, rank 0 finalises and formats"""
-    W, step = window
-    k, L = len(found), fasta.seqlen
-    nwin = api.window_count(L, W, step)
-    h = sum_over_ranks(ctx, group, max(2 * k * nwin, 1), lambda d: aln.site_windows_device(W, step, d))
-    if group.rank != 0:
-        return None
-    cnt = h.numpy()[: 2 * k * nwin].reshape(k, nwin, 2) if nwin else None
-    items = [(rows, int(cnt[q, i, 0]), int(cnt[q, i, 1]), min(i * step + W, L) - i * step, jc)
-             for i in range(nwin) for q, (_, _, rows) in enumerate(found)]
-    fin = iter(ctx.finalize(items))
-    return window_rows(file, found, [(i * step, min(i * step + W, L), [(int(cnt[q, i, 0]), next(fin)) for q in range(k)])
-                                     for i in range(nwin)])
-
-
-def sharded_cds_window_rows(ctx, group, aln, fasta, file, jc, found, window):
-    """--cds --window over column shards (codon-aligned by parallel.shard_columns): every rank computes its shard's codon window
-    vectors, the vectors are summed over the ranks, rank 0 finalises and formats"""
-    W, step = window
-    k, L = len(found), fasta.seqlen
-    nwin = api.window_count(L, W, step)
-    words = k * nwin * api.PFA_CDS_WIN_LEN
-    h = sum_over_ranks(ctx, group, max(words, 1), lambda d: aln.cds_windows_device(W, step, d))
-    if group.rank != 0:
-        return None
-    cnt = h.numpy()[:words].reshape(k, nwin, api.PFA_CDS_WIN_LEN)
-    return cds_window_rows(file, found, api.cds_window_results(ctx, cnt, [rows for _, _, rows in found], L, W, step, jc))
-
-
-def sharded_divergence_rows(ctx, group, aln, fasta, file, jc, found, window):
-    """--dxy over column shards: every rank computes its shard's site vector and D_xy per pair (with --window: (S, H) per
-    (population, window) and D_xy per (pair, window)), ONE vector is summed over the ranks, rank 0 finalises pi and the
-    divergence and formats"""
-    k, L = len(found), fasta.seqlen
-    pairs = api.pop_pairs(k)
-    P = len(pairs)
-    if window is None:
-        ns = aln.site_len()
-        h = sum_over_ranks(ctx, group, ns + P, lambda d: (aln.site_stats_device(d), aln.divergence_device(d + 8 * ns))).numpy()
-        if group.rank != 0:
-            return None
-        pis = [p[1] for p in ctx.finalize((s["n"], s["S"], s["H"], L, jc) for s in aln.unpack_site(h[:ns]))]
-        items = [(found[x][2], found[y][2], int(h[ns + p]), L, pis[x], pis[y], jc) for p, (x, y) in enumerate(pairs)]
-        return dxy_rows(file, found, [(0, L, ctx.div_finalize(items))], False)
-    W, step = window
-    nwin = api.window_count(L, W, step)
-    ws, wd = 2 * k * nwin, 2 * P * nwin
-    h = sum_over_ranks(ctx, group, max(ws + wd, 1),
-                       lambda d: (aln.site_windows_device(W, step, d), aln.divergence_windows_device(W, step, d + 8 * ws))).numpy()
-    if group.rank != 0:
-        return None
-    sc, dc = h[:ws].reshape(k, nwin, 2), h[ws:ws + wd].reshape(P, nwin, 2)
-    span = [(i * step, min(i * step + W, L)) for i in range(nwin)]
-    pis = [p[1] for p in ctx.finalize((found[q][2], int(sc[q, i, 0]), int(sc[q, i, 1]), e - s, jc)
-                                      for i, (s, e) in enumerate(span) for q in range(k))]
-    fin = ctx.div_finalize((found[x][2], found[y][2], int(dc[p, i, 1]), e - s, pis[i * k + x], pis[i * k + y], jc)
-                           for i, (s, e) in enumerate(span) for p, (x, y) in enumerate(pairs))
-    return dxy_rows(file, found, [(s, e, fin[i * P:(i + 1) * P]) for i, (s, e) in enumerate(span)], True)
-
-
-def sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window=None, dxy=False):
-    """rows of one large alignment whose COLUMNS are split over the ranks (SURVEY.md 8e.1): every rank uploads and scans its
-    codon-aligned range, the scan kernels sum the integer vectors over all ranks, rank 0 formats the rows"""
-    import numpy as np
-    import torch
-    from . import parallel
-    c0, c1 = parallel.shard_columns(fasta.seqlen, group.world, group.rank)
-    aln = api.Alignment.from_fasta(ctx, fasta, c0, c1)
-    try:
-        if found[0][1] is not None:
-            m = np.stack([mask for _, mask, _ in found])
-            api.check(api.lib().pfa_aln_set_pops(aln.handle, m.ctypes.data, len(found)), ctx.handle)
-        if dxy:
-            return sharded_divergence_rows(ctx, group, aln, fasta, file, jc, found, window)
-        if window is not None and cds:
-            return sharded_cds_window_rows(ctx, group, aln, fasta, file, jc, found, window)
-        if window is not None:
-            return sharded_window_rows(ctx, group, aln, fasta, file, jc, found, window)
-        k = len(found)
-        ns, nc = aln.site_len(), api.PFA_CDS_LEN * k
-        d_site = torch.zeros(ns, dtype=torch.int64, device="cuda:%d" % ctx.device)
-        d_cds = torch.zeros(nc, dtype=torch.int64, device="cuda:%d" % ctx.device)
-        torch.cuda.synchronize(ctx.device)
-        if group.fused:
-            x = group.exchange(ctx, ns + nc)
-            # the ranks meet on the host AFTER their uploads (parse + ingest times differ by seconds on cold files), so the
-            # wait inside the kernels only has to cover launch skew
-            ctx.sync()
-            group.dist.barrier()
-            if cds:   # K2 leaves its vector in the exchange's buffer, K4's epilogue pushes both: ONE exchange per alignment
-                d_both = torch.zeros(ns + nc, dtype=torch.int64, device="cuda:%d" % ctx.device)
-                torch.cuda.synchronize(ctx.device)
-                aln.site_cds_stats_xchg(x, d_both.data_ptr())
-            else:
-                aln.site_stats_xchg(x, d_site.data_ptr())
-            ctx.sync()
-            if x.timed_out():
-                raise api.PolyFastaError(1, "a rank did not arrive at the exchange")
-            if cds:
-                h_both = d_both.cpu()
-                h_site, h_cds = h_both[:ns], h_both[ns:]
-            else:
-                h_site, h_cds = d_site.cpu(), d_cds.cpu()
-        else:
-            aln.site_stats_device(d_site.data_ptr())
-            if cds:
-                aln.cds_stats_device(d_cds.data_ptr())
-            ctx.sync()
-            h_site, h_cds = d_site.cpu(), d_cds.cpu()
-            group.dist.all_reduce(h_site)
-            if cds:
-                group.dist.all_reduce(h_cds)
-        site = aln.unpack_site(h_site.numpy())
-        cdsst = None
-        if cds:
-            raw = h_cds.numpy().reshape(k, api.PFA_CDS_LEN)
-            ss = ctx.cds_ssites(raw)
-            cdsst = []
-            for q in range(k):
-                d = aln.unpack_cds(raw[q])
-                d["ssites"] = float(ss[q])
-                cdsst.append(d)
-    finally:
-        aln.free()
-    if group.rank != 0:
-        return [None] * len(found)
-    return format_rows(ctx, file, fasta.seqlen, cds, jc, [(label, rows) for label, _, rows in found], site, cdsst)
+        h = d_cnt.cpu()
+    else:
+        launch()
+        ctx.sync()
+        h = d_cnt.cpu()
+        group.dist.all_reduce(h)
+    h = h.numpy()
+    return [h[offs[i]:offs[i + 1]] for i in range(len(parts))]
 
 
 BATCH_FILES = int(os.environ.get("POLYFASTA_BATCH_FILES", "512"))   # loci per batched GPU pass
@@ -461,29 +346,68 @@ def plan_populations(fasta, popkeys):
     return plan
 
 
-def single_alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False):
-    """rows of one alignment through the single-alignment kernels (large alignments, --cds, --window, --cds --window and --dxy)"""
+def alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False, group=None):
+    """rows of one alignment through the single-alignment kernels (large alignments, --cds, --window, --cds --window and --dxy).
+    One process scans the whole alignment.  With `group`, every rank scans its codon-aligned column shard (SURVEY.md 8e.1), the
+    integer vectors are summed over the ranks, and rank 0 finalises and formats them as one process does (the other ranks
+    return None)."""
     import numpy as np
-    aln = api.Alignment.from_fasta(ctx, fasta)
+    from functools import partial
+    L, k = fasta.seqlen, len(found)
+    sizes = [rows for _, _, rows in found]
+    if group is None:
+        aln = api.Alignment.from_fasta(ctx, fasta)
+    else:
+        from . import parallel
+        aln = api.Alignment.from_fasta(ctx, fasta, *parallel.shard_columns(L, group.world, group.rank))
     try:
         if found[0][1] is not None:
             m = np.stack([mask for _, mask, _ in found])
-            api.check(api.lib().pfa_aln_set_pops(aln.handle, m.ctypes.data, len(found)), ctx.handle)
-        if dxy and window is not None:
-            wins = aln.divergence_windows(window[0], window[1], jc)
-            return dxy_rows(file, found, [(w["start"], w["end"], [(p["dxy"], p["da"], p["fst"]) for p in w["pairs"]]) for w in wins], True)
+            api.check(api.lib().pfa_aln_set_pops(aln.handle, m.ctypes.data, k), ctx.handle)
+        P = len(api.pop_pairs(k))
+        fused = None
+        # (words, synchronous counts, asynchronous launch into device memory) of every vector the rows need
+        if window is None:
+            parts = [(aln.site_len(), aln.site_counts, aln.site_stats_device)]
+            if cds:   # K2 leaves its vector in the exchange's buffer, K4's epilogue pushes both: ONE exchange per alignment
+                parts.append((k * api.PFA_CDS_LEN, aln.cds_counts, aln.cds_stats_device))
+                fused = aln.site_cds_stats_xchg
+            elif dxy:
+                parts.append((P, aln.divergence_counts, aln.divergence_device))
+            else:
+                fused = aln.site_stats_xchg
+        else:
+            W, step = window
+            nwin = api.window_count(L, W, step)
+            if cds:
+                parts = [(k * nwin * api.PFA_CDS_WIN_LEN, partial(aln.cds_window_counts, W, step), partial(aln.cds_windows_device, W, step))]
+            else:
+                parts = [(2 * k * nwin, partial(aln.site_window_counts, W, step), partial(aln.site_windows_device, W, step))]
+            if dxy:
+                parts.append((2 * P * nwin, partial(aln.divergence_window_counts, W, step), partial(aln.divergence_windows_device, W, step)))
+        if group is None:
+            vecs = [counts() for _, counts, _ in parts]
+        else:
+            vecs = sum_over_ranks(ctx, group, [(words, launch) for words, _, launch in parts], fused)
+            if group.rank != 0:
+                return None
+        if window is None:
+            site = aln.unpack_site(vecs[0])
+            if dxy:
+                return dxy_rows(file, found, [{"start": 0, "end": L, "pairs": api.divergence_results(ctx, site, vecs[1], sizes, L, jc)}],
+                                False)
+            cdsst = api.cds_results(ctx, np.reshape(vecs[1], (k, api.PFA_CDS_LEN))) if cds else None
+            return format_rows(ctx, file, L, cds, jc, [(label, rows) for label, _, rows in found], site, cdsst)
+        if cds:
+            wins = api.cds_window_results(ctx, np.reshape(vecs[0], (k, nwin, api.PFA_CDS_WIN_LEN)), sizes, L, W, step, jc)
+            return cds_window_rows(file, found, wins)
+        site = np.reshape(vecs[0], (k, nwin, 2))
         if dxy:
-            return dxy_rows(file, found, [(0, fasta.seqlen, [(d["dxy"], d["da"], d["fst"]) for d in aln.divergence(jc)])], False)
-        if window is not None and cds:
-            return cds_window_rows(file, found, aln.cds_windows(window[0], window[1], jc))
-        if window is not None:
-            wins = aln.site_windows(window[0], window[1], jc)
-            return window_rows(file, found, [(w["start"], w["end"], [(p["S"], p["poly"]) for p in w["pops"]]) for w in wins])
-        site = aln.site_stats()
-        cdsst = aln.cds_stats() if cds else None
+            wins = api.divergence_window_results(ctx, site, np.reshape(vecs[1], (P, nwin, 2)), sizes, L, W, step, jc)
+            return dxy_rows(file, found, wins, True)
+        return window_rows(file, found, api.site_window_results(ctx, site, sizes, L, W, step, jc))
     finally:
         aln.free()
-    return format_rows(ctx, file, fasta.seqlen, cds, jc, [(label, rows) for label, _, rows in found], site, cdsst)
 
 
 def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None, dxy=False):
@@ -520,17 +444,14 @@ def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None, 
             if dxy and len(found) < 2:
                 actions.append(("note", f"# Fewer than two populations found in {file}: no divergence rows."))
             elif found:
-                lines = (sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found, window, dxy) if group is not None
-                         else single_alignment_rows(ctx, fasta, file, cds, jc, found, window, dxy))
+                lines = alignment_rows(ctx, fasta, file, cds, jc, found, window, dxy, group)
                 keys = ([f"{found[x][0]},{found[y][0]}" for x, y in api.pop_pairs(len(found))] if dxy
                         else [label for label, _, _ in found])
                 for i, line in enumerate(lines or ()):
                     actions.append(("row", line, file, keys[i % len(keys)]))
             continue
-        if found and group is not None:
-            rows = iter(sharded_alignment_rows(ctx, group, fasta, file, cds, jc, found))
-        elif found and (cds or not api.Batch.fits(fasta)):
-            rows = iter(single_alignment_rows(ctx, fasta, file, cds, jc, found))
+        if found and (group is not None or cds or not api.Batch.fits(fasta)):
+            rows = iter(alignment_rows(ctx, fasta, file, cds, jc, found, group=group) or [None] * len(found))
         elif found:
             import numpy as np
             masks = None if found[0][1] is None else np.stack([m for _, m, _ in found])
@@ -550,13 +471,7 @@ def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None, 
     if pending:
         batch.run(jc)
         for pos, locus, q, file, seqlen, label, n in pending:
-            r = batch.result(locus, q)
-            if r["S"] == 0:
-                line = f"{file},{seqlen},{label},{n},0,0,0,NA"                                     # :187/:189
-            else:
-                p = r["poly"]
-                line = f"{file},{seqlen},{label},{n},{p[0]},{p[1]},{p[2]},{p[3]}"                  # :196/:198
-            actions[pos] = ("row", line, file, label)
+            actions[pos] = ("row", noncds_line(file, seqlen, label, n, batch.result(locus, q)), file, label)
     for _, fasta in items:
         if isinstance(fasta, api.Fasta):
             fasta.close()
@@ -566,21 +481,16 @@ def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None, 
 
 
 def noncds_line(file, seqlen, label, n, r):
-    if r["S"] == 0:
-        return f"{file},{seqlen},{label},{n},0,0,0,NA"                                         # PolyFastA.py:187/:189
-    p = r["poly"]
-    return f"{file},{seqlen},{label},{n},{p[0]},{p[1]},{p[2]},{p[3]}"                          # :196/:198
+    """the default row of print_result.no_header (PolyFastA.py:187-198) from the batched results of one (locus, population)"""
+    return f"{file},{seqlen},{label},{n}" + poly_tail(r["S"], r["poly"])
 
 
-def cds_line(file, seqlen, label, n, site, c):
-    """the --cds row of print_result.no_header (PolyFastA.py:160-180) from the batched results of one (locus, population)"""
+def cds_line(file, seqlen, label, n, S, c, poly_s, poly_n):
+    """the --cds row of print_result.no_header (PolyFastA.py:160-180) of one population: S of the site scan, c its codon-scan
+    results, poly_s / poly_n the synonymous / nonsynonymous tuples"""
     ssites = c["ssites"]
     nsites = (seqlen - c["missing"]) - ssites
-    head = f"{file},{round(ssites, 2)},{round(nsites, 2)},{label},{n}"
-    if site["S"] == 0:
-        return head + ",0,0,0,NA,0,0,0,NA,0"                                                   # :160/:162
-    s, m = c["poly_s"], c["poly_n"]
-    return head + f",{s[0]},{m[0]},{s[1]},{m[1]},{s[2]},{m[2]},{s[3]},{m[3]},{c['nstops']}"     # :178/:180
+    return f"{file},{round(ssites, 2)},{round(nsites, 2)},{label},{n}" + cds_tail(S, poly_s, poly_n, c["nstops"])
 
 
 def process_chunk_native(ctx, batch, paths, jc, popkeys, threads, cds=False):
@@ -646,7 +556,8 @@ def process_chunk_native(ctx, batch, paths, jc, popkeys, threads, cds=False):
         t3 = time.perf_counter()
         for pos, locus, q, file, seqlen, label, n in pending:
             if cds:
-                line = cds_line(file, seqlen, label, n, batch.result(locus, q), batch.result_cds(locus, q))
+                c = batch.result_cds(locus, q)
+                line = cds_line(file, seqlen, label, n, batch.result(locus, q)["S"], c, c["poly_s"], c["poly_n"])
             else:
                 line = noncds_line(file, seqlen, label, n, batch.result(locus, q))
             actions[pos] = ("row", line, file, label)

@@ -590,6 +590,31 @@ int pfa_cds_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* counts) {
                        [&](void* d_out, void*) { return pfa_cds_windows_device(a, window, step, (int64_t*)d_out); });
 }
 
+int pfa_site_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* counts) {
+    if (!a) return PFA_ERR_ARG;
+    const int64_t nwin = pfa_window_count(a->L_total, window, step);
+    if (nwin <= 0) return pfa_site_windows_device(a, window, step, nullptr);  // argument errors, or nothing to do
+    if (!counts) return pfa_fail(a->ctx, PFA_ERR_ARG, "windows: null output");
+    return run_to_host(a, sizeof(int64_t) * 2 * (size_t)(a->k * nwin), counts, 0, nullptr,
+                       [&](void* d_out, void*) { return pfa_site_windows_device(a, window, step, (int64_t*)d_out); });
+}
+
+int pfa_divergence(pfa_aln* a, int64_t* counts) {
+    if (!a || !counts) return PFA_ERR_ARG;
+    const int64_t P = (int64_t)a->k * (a->k - 1) / 2;
+    return run_to_host(a, sizeof(int64_t) * (size_t)P, counts, 0, nullptr,
+                       [&](void* d_out, void*) { return pfa_divergence_device(a, (int64_t*)d_out); });
+}
+
+int pfa_divergence_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* counts) {
+    if (!a) return PFA_ERR_ARG;
+    const int64_t nwin = pfa_window_count(a->L_total, window, step), P = (int64_t)a->k * (a->k - 1) / 2;
+    if (nwin <= 0 || P <= 0) return pfa_divergence_windows_device(a, window, step, nullptr);  // argument errors, or nothing to do
+    if (!counts) return pfa_fail(a->ctx, PFA_ERR_ARG, "divergence windows: null output");
+    return run_to_host(a, sizeof(int64_t) * 2 * (size_t)(P * nwin), counts, 0, nullptr,
+                       [&](void* d_out, void*) { return pfa_divergence_windows_device(a, window, step, (int64_t*)d_out); });
+}
+
 int pfa_site_stats_xchg(pfa_aln* a, pfa_xchg* x, int64_t* d_out, uint8_t* d_isvar) {
     if (!a || !x || !d_out) return PFA_ERR_ARG;
     PFA_CUDA(a->ctx, cudaSetDevice(a->ctx->device));

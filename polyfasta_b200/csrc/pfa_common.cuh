@@ -132,14 +132,11 @@ struct PfaXchgDev;
 // d_hsite (optional): int64 [k][ns], H of every variable (site, population), 0 elsewhere (pfa_site_stats_hsite_device)
 int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg* x = nullptr, bool defer = false,
                          int64_t* d_hsite = nullptr);
-// windowed (S, H) of this shard from the per-site H of the site scan (pfa_windows.cu)
-int pfa_launch_site_windows(pfa_aln* a, const int64_t* d_hsite, int64_t window, int64_t step, int64_t* d_counts);
-// the same reduction for `rows` rows of per-site values d_persite [rows][ns]: d_counts [rows][nwin][2] = (non-zero sites, sum)
-// (the divergence windows feed it the per-pair Dxy_site)
+// windows of this shard (pfa_windows.cu) for `rows` rows of per-site values d_persite [rows][ns]: d_counts [rows][nwin][2] =
+// (non-zero sites, sum); the site scan's per-site H gives (S, H) per population, the divergence scan's Dxy_site per pair
 int pfa_launch_row_windows(pfa_aln* a, int rows, const int64_t* d_persite, int64_t window, int64_t step, int64_t* d_counts);
 // K3's first step alone: flags[s] = 1 where two of the n rows differ in the planes (pfa_pairwise.cu)
 int pfa_launch_var_flags(pfa_aln* a, uint8_t* flags);
-int pfa_launch_window_final_in(pfa_aln* a, const int64_t* d_counts, int64_t window, int64_t step, int jc, pfa_final_in* d_in);
 int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg* x = nullptr);
 // codon windows: bins [k][PFA_CDS_WIN_LEN][nb] (zeroed) of this shard from K2's per-site H and K4's labels (pfa_codon.cu), and
 // the window vectors [k][nwin][PFA_CDS_WIN_LEN] from them (pfa_windows.cu)

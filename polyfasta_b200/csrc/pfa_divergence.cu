@@ -17,7 +17,6 @@
 //   4. pfa_div_finalize_kernel: dxy, d_a, F_ST in fp64 with round-to-nearest intrinsics (-fmad=false for the library).
 #include <algorithm>
 #include <climits>
-#include <vector>
 
 #include <cub/device/device_select.cuh>
 #include <cub/iterator/counting_input_iterator.cuh>
@@ -274,9 +273,6 @@ static int pfa_launch_div_finalize(pfa_ctx* ctx, const pfa_div_in* d_in, pfa_div
     return PFA_OK;
 }
 
-// pi_site of a K5 output: 0 when the population has no variable site there
-static double pfa_div_pi(const pfa_final_out& f) { return f.no_var ? 0.0 : f.pi_site; }
-
 extern "C" {
 
 int pfa_divergence_device(pfa_aln* a, int64_t* d_out) {
@@ -291,8 +287,8 @@ int pfa_divergence_windows_device(pfa_aln* a, int64_t window, int64_t step, int6
     pfa_ctx* ctx = a->ctx;
     if (window < 1 || step < 1) return pfa_fail(ctx, PFA_ERR_ARG, "divergence windows: window and step must be >= 1 (got %lld, %lld)", (long long)window, (long long)step);
     if (int rc = pfa_div_check(a)) return rc;
-    const int64_t nwin = pfa_window_count(a->L_total, window, step);
-    if (!d_counts && nwin > 0) return pfa_fail(ctx, PFA_ERR_ARG, "divergence windows: null output");
+    if (pfa_window_count(a->L_total, window, step) == 0) return PFA_OK;
+    if (!d_counts) return pfa_fail(ctx, PFA_ERR_ARG, "divergence windows: null output");
     PFA_CUDA(ctx, cudaSetDevice(ctx->device));
     const int64_t P = pfa_div_pairs(a);
     int64_t *d_tot = nullptr, *d_dsite = nullptr;
@@ -329,83 +325,6 @@ int pfa_div_finalize(pfa_ctx* ctx, const pfa_div_in* in, pfa_div_out* out, int c
     pfa_dfree(ctx, d_out);
     pfa_dfree(ctx, d_in);
     return rc;
-}
-
-int pfa_divergence(pfa_aln* a, int jc, int64_t* counts, pfa_div_out* out) {
-    if (!a || !counts) return PFA_ERR_ARG;
-    if (int rc = pfa_div_check(a)) return rc;
-    pfa_ctx* ctx = a->ctx;
-    PFA_CUDA(ctx, cudaSetDevice(ctx->device));
-    const int64_t P = pfa_div_pairs(a), slen = pfa_site_len(a);
-    int64_t *d_D = nullptr, *d_site = nullptr;
-    std::vector<int64_t> site((size_t)(out ? slen : 0));
-    cudaError_t e = pfa_dmalloc(ctx, &d_D, sizeof(int64_t) * (size_t)P);
-    if (e == cudaSuccess && out) e = pfa_dmalloc(ctx, &d_site, sizeof(int64_t) * (size_t)slen);
-    int rc = e == cudaSuccess ? PFA_OK : pfa_fail(ctx, PFA_ERR_CUDA, "divergence: cudaMallocAsync failed: %s", cudaGetErrorString(e));
-    if (!rc) rc = pfa_launch_divergence(a, d_D, nullptr);
-    if (!rc && out) rc = pfa_launch_site_scan(a, d_site, nullptr);  // pi of every population
-    if (!rc) {
-        e = cudaMemcpyAsync(counts, d_D, sizeof(int64_t) * (size_t)P, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess && out) e = cudaMemcpyAsync(site.data(), d_site, sizeof(int64_t) * (size_t)slen, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = pfa_fail(ctx, PFA_ERR_CUDA, "divergence: result copy failed: %s", cudaGetErrorString(e));
-    }
-    pfa_dfree(ctx, d_site);
-    pfa_dfree(ctx, d_D);
-    if (rc || !out) return rc;
-    std::vector<pfa_final_in> fin_in((size_t)a->k);
-    std::vector<pfa_final_out> fin((size_t)a->k);
-    for (int q = 0; q < a->k; ++q)
-        fin_in[(size_t)q] = pfa_final_in{a->pop_n[(size_t)q], site[(size_t)a->site_off[(size_t)q]], site[(size_t)a->site_off[(size_t)q] + 1],
-                                         (double)a->L_total, jc ? 1 : 0, 0};
-    if ((rc = pfa_finalize(ctx, fin_in.data(), fin.data(), a->k))) return rc;
-    std::vector<pfa_div_in> din((size_t)P);
-    for (int x = 0, p = 0; x < a->k; ++x)
-        for (int y = x + 1; y < a->k; ++y, ++p)
-            din[(size_t)p] = pfa_div_in{a->pop_n[(size_t)x], a->pop_n[(size_t)y], counts[p], (double)a->L_total,
-                                        pfa_div_pi(fin[(size_t)x]), pfa_div_pi(fin[(size_t)y]), jc ? 1 : 0, 0};
-    return pfa_div_finalize(ctx, din.data(), out, (int)P);
-}
-
-int pfa_divergence_windows(pfa_aln* a, int64_t window, int64_t step, int jc, int64_t* counts, pfa_div_out* out) {
-    if (!a) return PFA_ERR_ARG;
-    pfa_ctx* ctx = a->ctx;
-    if (window < 1 || step < 1) return pfa_fail(ctx, PFA_ERR_ARG, "divergence windows: window and step must be >= 1 (got %lld, %lld)", (long long)window, (long long)step);
-    if (int rc = pfa_div_check(a)) return rc;
-    const int64_t nwin = pfa_window_count(a->L_total, window, step), P = pfa_div_pairs(a);
-    if (nwin == 0) return PFA_OK;
-    if (!counts) return pfa_fail(ctx, PFA_ERR_ARG, "divergence windows: null output");
-    if (P * nwin > INT_MAX || (int64_t)a->k * nwin > INT_MAX)
-        return pfa_fail(ctx, PFA_ERR_ARG, "divergence windows: %lld (pair, window) entries exceed the finalisation's range", (long long)(P * nwin));
-    PFA_CUDA(ctx, cudaSetDevice(ctx->device));
-    std::vector<int64_t> dc((size_t)(2 * P * nwin));
-    int64_t* d_counts = nullptr;
-    cudaError_t e = pfa_dmalloc(ctx, &d_counts, sizeof(int64_t) * dc.size());
-    int rc = e == cudaSuccess ? PFA_OK : pfa_fail(ctx, PFA_ERR_CUDA, "divergence windows: cudaMallocAsync failed: %s", cudaGetErrorString(e));
-    if (!rc) rc = pfa_divergence_windows_device(a, window, step, d_counts);
-    if (!rc) {
-        e = cudaMemcpyAsync(dc.data(), d_counts, sizeof(int64_t) * dc.size(), cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = pfa_fail(ctx, PFA_ERR_CUDA, "divergence windows: result copy failed: %s", cudaGetErrorString(e));
-    }
-    pfa_dfree(ctx, d_counts);
-    if (rc) return rc;
-    for (int64_t e2 = 0; e2 < P * nwin; ++e2) counts[e2] = dc[(size_t)(2 * e2 + 1)];  // the D half of (S, D)
-    if (!out) return PFA_OK;
-    // pi of every (population, window): the site scan's windows and K5
-    std::vector<int64_t> sc((size_t)(2 * a->k * nwin));
-    std::vector<pfa_final_out> fin((size_t)(a->k * nwin));
-    if ((rc = pfa_site_windows(a, window, step, jc, sc.data(), fin.data()))) return rc;
-    std::vector<pfa_div_in> din((size_t)(P * nwin));
-    for (int x = 0, p = 0; x < a->k; ++x)
-        for (int y = x + 1; y < a->k; ++y, ++p)
-            for (int64_t i = 0; i < nwin; ++i) {
-                const int64_t ws = i * step, we = std::min(ws + window, a->L_total);
-                din[(size_t)(p * nwin + i)] = pfa_div_in{a->pop_n[(size_t)x], a->pop_n[(size_t)y], counts[p * nwin + i], (double)(we - ws),
-                                                         pfa_div_pi(fin[(size_t)(x * nwin + i)]), pfa_div_pi(fin[(size_t)(y * nwin + i)]),
-                                                         jc ? 1 : 0, 0};
-            }
-    return pfa_div_finalize(ctx, din.data(), out, (int)(P * nwin));
 }
 
 }  // extern "C"

@@ -98,9 +98,9 @@ def test_cli_dxy_headers(tmp_path, capsys):
         assert out.read_text() == want + "\n"
 
 
-def test_cli_dxy_rows_format():
+def test_cli_dxy_rows_from_results():
     found = [("p0", None, 3), ("p1", None, 2), ("p2", None, 4)]
-    fins = [(0.25, 0.125, 0.5), (0.0, 0.0, "NA"), (1.5, -0.25, 0.75)]
-    assert cli.dxy_rows("f.fa", found, [(0, 10, fins)], False) == [
+    fins = [{"dxy": dxy, "da": da, "fst": fst} for dxy, da, fst in ((0.25, 0.125, 0.5), (0.0, 0.0, "NA"), (1.5, -0.25, 0.75))]
+    assert cli.dxy_rows("f.fa", found, [{"start": 0, "end": 10, "pairs": fins}], False) == [
         "f.fa,10,p0,p1,3,2,0.25,0.125,0.5", "f.fa,10,p0,p2,3,4,0.0,0.0,NA", "f.fa,10,p1,p2,2,4,1.5,-0.25,0.75"]
-    assert cli.dxy_rows("f.fa", found[:2], [(5, 9, fins[:1])], True) == ["f.fa,6,9,4,p0,p1,3,2,0.25,0.125,0.5"]
+    assert cli.dxy_rows("f.fa", found[:2], [{"start": 5, "end": 9, "pairs": fins[:1]}], True) == ["f.fa,6,9,4,p0,p1,3,2,0.25,0.125,0.5"]

@@ -190,9 +190,9 @@ def test_windows_against_oracle_slices(ctx, n, L):
     aln.free()
 
 
-def test_whole_alignment_against_python_oracle(ctx):
-    """the Python oracle end to end (pi from the reference's restatement) on a small alignment, and the synchronous C entry
-    point with its finalised output"""
+def test_whole_alignment_counts_against_python_oracle(ctx):
+    """the Python oracle end to end (pi from the reference's restatement) on a small alignment, and D from the synchronous C
+    entry point"""
     rng = np.random.default_rng(5)
     n, L = 24, 120
     text = _random_text(rng, n, L, p_var=0.2, p_junk=0.05)
@@ -203,8 +203,7 @@ def test_whole_alignment_against_python_oracle(ctx):
     for jc in (False, True):
         got = aln.divergence(jc)
         D = np.zeros(3, dtype=np.int64)
-        out = (api.DivOut * 3)()
-        api.check(api.lib().pfa_divergence(aln.handle, int(jc), D.ctypes.data, out), ctx.handle)
+        api.check(api.lib().pfa_divergence(aln.handle, D.ctypes.data), ctx.handle)
         for p, (x, y) in enumerate(pairs(3)):
             rx, ry = [seqs[i] for i in pops[x]], [seqs[i] for i in pops[y]]
             Dw = divergence(rx, ry, L)
@@ -214,9 +213,6 @@ def test_whole_alignment_against_python_oracle(ctx):
             assert g["D"] == Dw == int(D[p])
             assert close(g["pi_x"], px) and close(g["pi_y"], py)
             _check_fin((g["dxy"], g["da"], g["fst"]), want)
-            o = out[p]
-            assert not o.undefined
-            _check_fin((o.dxy, o.da, "NA" if o.fst_is_NA else o.fst), want)
     aln.free()
 
 
