@@ -359,6 +359,20 @@ int pfa_divergence(pfa_aln* a, int64_t* counts);
  * PFA_ERR_ARG. */
 int pfa_divergence_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* counts);
 
+/* ---- haplotype classes (beyond the reference: number of haplotypes and haplotype diversity) -------------------------------
+ * Two rows are the same haplotype over a set of columns iff their (upper-cased) characters are equal at every one of them:
+ * every character is an allele, as in the site scan, so 'A', '-', 'N', '?' and two different other bytes all differ;
+ * equivalently, d_ij of pfa_pairwise is 0 over those columns.  rep[w][r] = the smallest row index (over all rows, whatever the
+ * populations) of row r's class over THIS SHARD's columns of window w; windows are those of pfa_window_count, and window = step
+ * = L gives the whole alignment as the single window.  A window that does not meet the shard is one class (rep = 0).  The rows
+ * are identical over the whole alignment iff they are identical in every column shard: the classes of the alignment are the
+ * common refinement of the shards' classes.  Needs nwin * n <= 2^31-1 and a shard of at most 2^31-1 sites (else PFA_ERR_ARG).
+ * Builds K3's row-major planes of the marked sites and a row-ordered copy of the exception list once per alignment. */
+/* asynchronous: d_rep (device) = int32 [nwin][n] */
+int pfa_haplotypes_device(pfa_aln* a, int64_t window, int64_t step, int32_t* d_rep);
+/* synchronous: rep (host) = int32 [nwin][n] as above */
+int pfa_haplotypes(pfa_aln* a, int64_t window, int64_t step, int32_t* rep);
+
 #ifdef __cplusplus
 }
 #endif

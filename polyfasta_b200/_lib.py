@@ -26,6 +26,7 @@ EXPORTS = [
     "pfa_site_len", "pfa_site_offset", "pfa_site_stats_device", "pfa_site_stats", "pfa_site_stats_hsite_device", "pfa_site_stats_hsite",
     "pfa_window_count", "pfa_site_windows_device", "pfa_site_windows", "pfa_cds_windows_device", "pfa_cds_windows",
     "pfa_divergence_device", "pfa_divergence_windows_device", "pfa_div_finalize", "pfa_divergence", "pfa_divergence_windows",
+    "pfa_haplotypes_device", "pfa_haplotypes",
     "pfa_cds_stats_device", "pfa_cds_stats", "pfa_codon_pair_labels", "pfa_codon_set_labels", "pfa_codon_syn3",
     "pfa_codon_class", "pfa_pairwise_device", "pfa_pairwise", "pfa_finalize", "pfa_cds_ssites",
     "pfa_mask_words_for", "pfa_batch_create", "pfa_batch_destroy", "pfa_batch_clear", "pfa_batch_size", "pfa_batch_text_bytes",
@@ -136,6 +137,8 @@ def lib():
         "pfa_div_finalize": (c.c_int, [p, c.POINTER(DivIn), c.POINTER(DivOut), c.c_int]),
         "pfa_divergence": (c.c_int, [p, p]),
         "pfa_divergence_windows": (c.c_int, [p, i64, i64, p]),
+        "pfa_haplotypes_device": (c.c_int, [p, i64, i64, p]),
+        "pfa_haplotypes": (c.c_int, [p, i64, i64, p]),
         "pfa_cds_stats_device": (c.c_int, [p, p, p]),
         "pfa_cds_stats": (c.c_int, [p, p, p]),
         "pfa_codon_pair_labels": (c.c_int, [c.c_int, c.c_int]),

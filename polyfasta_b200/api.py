@@ -202,6 +202,71 @@ def divergence_window_results(ctx, site_counts, div_counts, sizes, L, window, st
     return res
 
 
+def meet_classes(reps):
+    """the haplotype classes of an alignment from the classes of its column shards: reps = int32 [nwin][n] rep arrays
+    (pfa_haplotypes of each shard, same windows).  Two rows are one haplotype iff they are one in every shard (the common
+    refinement); the result is again canonical: every row's rep is the smallest row index of its class."""
+    reps = [np.asarray(r, dtype=np.int64) for r in reps]
+    if len(reps) == 1:
+        return reps[0].astype(np.int32)
+    nwin, n = reps[0].shape
+    base = (np.arange(nwin, dtype=np.int64) * n)[:, None]
+    cur = reps[0]
+    for nxt in reps[1:]:
+        # (window, class in the meet so far, class in the next shard) -> one int64 key: < nwin n^2 <= 2^31 n
+        key = (base + cur) * n + nxt
+        _, first, inv = np.unique(key.ravel(), return_index=True, return_inverse=True)
+        cur = (first[inv.ravel()] - np.repeat(base.ravel(), n)).reshape(nwin, n)   # the first index of a key is its smallest row
+    return cur.astype(np.int32)
+
+
+def haplotype_results(rep, masks, sizes, L, window, step):
+    """canonical classes int32 [nwin][n] of an alignment of L columns (meet_classes of pfa_haplotypes' arrays) -> list of
+    dict(start, end, seqlen, pops=[dict(n, h, s2, s3, Hd, Hd_var)]), start 0-based, end exclusive.  masks: uint32 [k][words] row
+    masks of the populations (rows_to_masks, match_mask), or None for one population of all rows; sizes: their row counts.
+    For a population of n rows whose classes have c_1 .. c_h rows: s2 = sum c^2, s3 = sum c^3, Hd = (n^2 - s2) / (n (n - 1))
+    (one fp64 division of two exact integers) and Hd_var = Nei (1987) eq. 8.12 evaluated as the exact integer
+    2 [2 (n - 2) (n s3 - s2^2) + n^2 s2 - s2^2] over n^5 (n - 1), rounded once; both "NA" for n = 1.  There is no kernel for
+    this step: Hd and Hd_var are closed forms of four exact integers."""
+    rep = np.asarray(rep, dtype=np.int64)
+    nwin, nrows = rep.shape
+    if masks is None:
+        pops = [np.arange(nrows)]
+    else:
+        bits = np.unpackbits(np.ascontiguousarray(masks, dtype=np.uint32).view(np.uint8).reshape(len(masks), -1), axis=1,
+                             bitorder="little")
+        pops = [np.flatnonzero(b[:nrows]) for b in bits]
+    stats = []
+    for q, rows in enumerate(pops):
+        n = rows.size
+        if n != sizes[q]:
+            raise ValueError("haplotype_results: population %d has %d rows in its mask, %d in sizes" % (q, n, sizes[q]))
+        sub = np.sort(rep[:, rows], axis=1)
+        new = np.ones(sub.shape, dtype=bool)
+        new[:, 1:] = sub[:, 1:] != sub[:, :-1]
+        h = new.sum(axis=1)
+        starts = np.flatnonzero(new.ravel())
+        c = np.diff(np.append(starts, new.size))              # class sizes, window by window
+        first = np.concatenate(([0], np.cumsum(h)[:-1]))       # every window has at least one class
+        s2, s3 = np.add.reduceat(c * c, first), np.add.reduceat(c * c * c, first)
+        s2o, s3o = s2.astype(object), s3.astype(object)
+        if n > 1:
+            Hd = (n * n - s2).astype(np.float64) / float(n * (n - 1))
+            V = 2 * (2 * (n - 2) * (n * s3o - s2o * s2o) + n * n * s2o - s2o * s2o)
+            Hd_var = [int(v) / (n ** 5 * (n - 1)) for v in V]
+        else:
+            Hd = Hd_var = ["NA"] * nwin
+        stats.append((n, h, s2, s3, Hd, Hd_var))
+    res = []
+    for i in range(nwin):
+        start, end = i * step, min(i * step + window, L)
+        res.append({"start": start, "end": end, "seqlen": end - start,
+                    "pops": [{"n": n, "h": int(h[i]), "s2": int(s2[i]), "s3": int(s3[i]),
+                              "Hd": Hd[i] if n == 1 else float(Hd[i]), "Hd_var": Hd_var[i]}
+                             for n, h, s2, s3, Hd, Hd_var in stats]})
+    return res
+
+
 def pop_pairs(k):
     """the population pairs of the divergence statistics, in their order: (0, 1), (0, 2), ..., (0, k-1), (1, 2), ..."""
     return [(x, y) for x in range(k) for y in range(x + 1, k)]
@@ -458,9 +523,11 @@ class Alignment:
         """row_lists: list of row-index iterables (one per population, in output order); None/[] = all rows"""
         if not row_lists:
             check(lib().pfa_aln_set_pops(self.handle, None, 0), self.ctx.handle)
+            self._pop_masks = None
             return
         m = rows_to_masks(self.mask_words, row_lists)
         check(lib().pfa_aln_set_pops(self.handle, m.ctypes.data, len(row_lists)), self.ctx.handle)
+        self._pop_masks = m
 
     @property
     def mask_words(self):
@@ -601,6 +668,39 @@ class Alignment:
         """asynchronous: int64 [P][nwin][2] (columns with a difference, D_xy) of this shard's columns of every (pair, window)
         into caller device memory; the vectors of the column shards add up"""
         check(lib().pfa_divergence_windows_device(self.handle, int(window), int(step), ctypes.c_void_p(d_ptr)), self.ctx.handle)
+
+    def haplotype_classes(self, window=None, step=None):
+        """int32 [nwin][n]: rep[w][r] = the smallest row index of row r's haplotype class over this shard's columns of window w
+        (pfa_haplotypes); window None: the whole alignment as the single window [0, L).  Classes are over all rows, whatever
+        the populations; meet_classes combines the arrays of the column shards of an alignment."""
+        window, step = self._hap_span(window, step)
+        nwin = self.window_count(window, step)
+        rep = np.zeros((max(nwin, 1), max(self.n, 1)), dtype=np.int32)
+        check(lib().pfa_haplotypes(self.handle, int(window), int(step), rep.ctypes.data), self.ctx.handle)
+        return rep[:nwin, :self.n]
+
+    def haplotypes(self, window=None, step=None):
+        """number of haplotypes h, haplotype diversity Hd and its variance per population (set_pops; one population of all rows
+        when they were never set), for the whole alignment (window None: one entry) or in windows of `window` columns every
+        `step` (default: `window`) -> the list haplotype_results returns.  For a column shard: the shard's columns only."""
+        window, step = self._hap_span(window, step)
+        masks = getattr(self, "_pop_masks", None)
+        return haplotype_results(meet_classes([self.haplotype_classes(window, step)]), masks, self.pop_sizes(), self.total_len,
+                                 window, step)
+
+    def haplotypes_device(self, window, step, d_ptr):
+        """asynchronous: int32 [nwin][n] rep arrays of this shard into caller device memory (pfa_haplotypes_device)"""
+        check(lib().pfa_haplotypes_device(self.handle, int(window), int(step), ctypes.c_void_p(d_ptr)), self.ctx.handle)
+
+    def _hap_span(self, window, step):
+        if window is None:
+            if step is not None:
+                raise ValueError("haplotypes: step needs a window")
+            return max(self.total_len, 1), max(self.total_len, 1)
+        step = window if step is None else step
+        if window < 1 or step < 1:
+            raise ValueError("window and step must be >= 1")
+        return window, step
 
     def site_stats_device(self, d_out_ptr, d_isvar_ptr=None):
         """asynchronous K2 into caller device memory (int64[site_len]); for the multi-GPU all-reduce"""

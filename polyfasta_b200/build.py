@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libpolyfasta_b200.so")
-CU = ["pfa_api.cu", "pfa_encode.cu", "pfa_sites.cu", "pfa_codon.cu", "pfa_pairwise.cu", "pfa_finalize.cu", "pfa_batch.cu", "pfa_xchg.cu", "pfa_ingest.cu", "pfa_windows.cu", "pfa_divergence.cu"]
+CU = ["pfa_api.cu", "pfa_encode.cu", "pfa_sites.cu", "pfa_codon.cu", "pfa_pairwise.cu", "pfa_finalize.cu", "pfa_batch.cu", "pfa_xchg.cu", "pfa_ingest.cu", "pfa_windows.cu", "pfa_divergence.cu", "pfa_haplotypes.cu"]
 CPP = ["pfa_fasta.cpp", "pfa_codon_rules.cpp", "pfa_pack.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--fmad=false",
               "-Xcompiler", "-fPIC,-O2,-Wall,-Wno-deprecated-declarations", "-diag-suppress", "128", "-Xptxas", "-v"]

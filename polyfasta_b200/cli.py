@@ -65,6 +65,8 @@ HEADER_NONCDS = "file,seqlen,pop,N,seg_sites,pi,theta,tajimasD"
 HEADER_WINDOWS = "file,window_start,window_end,seqlen,pop,N,seg_sites,pi,theta,tajimasD"
 HEADER_DXY = "file,seqlen,pop1,pop2,N1,N2,dxy,da,Fst"
 HEADER_DXY_WINDOWS = "file,window_start,window_end,seqlen,pop1,pop2,N1,N2,dxy,da,Fst"
+HEADER_HAP = "file,seqlen,pop,N,haplotypes,Hd,Hd_var"
+HEADER_HAP_WINDOWS = "file,window_start,window_end,seqlen,pop,N,haplotypes,Hd,Hd_var"
 HEADER_CDS = ("file,sites_S,sites_N,pop,N,seg_sites_S,seg_sites_N,pi_S,pi_N,theta_S,theta_N,"
               "tajimasD_S,tajimasD_N,nstops")
 HEADER_CDS_WINDOWS = ("file,window_start,window_end,sites_S,sites_N,pop,N,seg_sites_S,seg_sites_N,pi_S,pi_N,theta_S,theta_N,"
@@ -88,7 +90,21 @@ def build_parser():
     parser.add_argument("--dxy", action="store_true", default=False,
                         help="d_xy, net divergence d_a and Hudson's F_ST between every pair of the -p populations (one row per\n"
                              "pair instead of the per-population rows; with --window, one row per window and pair). Not with --cds.")
+    # beyond the reference: haplotype statistics
+    parser.add_argument("--haplotypes", action="store_true", default=False,
+                        help="number of distinct haplotypes (rows), Nei's haplotype diversity Hd and its variance per population\n"
+                             "instead of the default statistics (with --window, per window). Not with --cds or --dxy.")
     return parser
+
+
+def check_hap_args(parser, args):
+    """the --haplotypes combinations that are errors"""
+    if not args.haplotypes:
+        return
+    if args.cds:
+        parser.error("--haplotypes does not work with --cds")
+    if args.dxy:
+        parser.error("--haplotypes does not work with --dxy")
 
 
 def check_dxy_args(parser, args):
@@ -122,8 +138,10 @@ class Sink:
         self.out = out
         self.silent = silent
 
-    def header(self, cds, windows=False, dxy=False):
-        if dxy:
+    def header(self, cds, windows=False, dxy=False, hap=False):
+        if hap:
+            line = HEADER_HAP_WINDOWS if windows else HEADER_HAP
+        elif dxy:
             line = HEADER_DXY_WINDOWS if windows else HEADER_DXY
         else:
             line = (HEADER_CDS_WINDOWS if cds else HEADER_WINDOWS) if windows else HEADER_CDS if cds else HEADER_NONCDS
@@ -224,6 +242,18 @@ def dxy_rows(file, found, wins, windowed):
         head = f"{file},{start + 1},{end},{end - start}" if windowed else f"{file},{end - start}"
         for (x, y), d in zip(pairs, w["pairs"]):
             lines.append(head + f",{found[x][0]},{found[y][0]},{found[x][2]},{found[y][2]},{d['dxy']},{d['da']},{d['fst']}")
+    return lines
+
+
+def hap_rows(file, found, wins, windowed):
+    """--haplotypes rows of one alignment: wins = the list api.haplotype_results returns (the whole alignment is one window).
+    Window by window, the populations in order; windowed: the window's 1-based inclusive coordinates go in front of seqlen (the
+    window's length)"""
+    lines = []
+    for w in wins:
+        head = f"{file},{w['start'] + 1},{w['end']},{w['seqlen']}" if windowed else f"{file},{w['seqlen']}"
+        for (label, _, n), p in zip(found, w["pops"]):
+            lines.append(head + f",{label},{n},{p['h']},{p['Hd']},{p['Hd_var']}")
     return lines
 
 
@@ -346,11 +376,13 @@ def plan_populations(fasta, popkeys):
     return plan
 
 
-def alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False, group=None):
-    """rows of one alignment through the single-alignment kernels (large alignments, --cds, --window, --cds --window and --dxy).
-    One process scans the whole alignment.  With `group`, every rank scans its codon-aligned column shard (SURVEY.md 8e.1), the
-    integer vectors are summed over the ranks, and rank 0 finalises and formats them as one process does (the other ranks
-    return None)."""
+def alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False, group=None, hap=False):
+    """rows of one alignment through the single-alignment kernels (large alignments, --cds, --window, --cds --window, --dxy and
+    --haplotypes).  One process scans the whole alignment.  With `group`, every rank scans its codon-aligned column shard
+    (SURVEY.md 8e.1), the integer vectors are summed over the ranks, and rank 0 finalises and formats them as one process does
+    (the other ranks return None).  --haplotypes: the classes of the shards are not a sum; each rank writes its int32 rep array
+    into its own slice of the vector and leaves the other slices zero, so the sum over the ranks gathers them, and rank 0 takes
+    their meet (api.meet_classes)."""
     import numpy as np
     from functools import partial
     L, k = fasta.seqlen, len(found)
@@ -367,7 +399,14 @@ def alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False, gro
         P = len(api.pop_pairs(k))
         fused = None
         # (words, synchronous counts, asynchronous launch into device memory) of every vector the rows need
-        if window is None:
+        if hap:
+            W, step = window if window is not None else (max(L, 1), max(L, 1))
+            nwin = api.window_count(L, W, step)
+            half = (nwin * fasta.nseq + 1) // 2   # int64 words of one rank's slice
+            rank, world = (0, 1) if group is None else (group.rank, group.world)
+            parts = [(world * half, partial(aln.haplotype_classes, W, step),
+                      lambda d: aln.haplotypes_device(W, step, d + 8 * half * rank))]
+        elif window is None:
             parts = [(aln.site_len(), aln.site_counts, aln.site_stats_device)]
             if cds:   # K2 leaves its vector in the exchange's buffer, K4's epilogue pushes both: ONE exchange per alignment
                 parts.append((k * api.PFA_CDS_LEN, aln.cds_counts, aln.cds_stats_device))
@@ -391,6 +430,14 @@ def alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False, gro
             vecs = sum_over_ranks(ctx, group, [(words, launch) for words, _, launch in parts], fused)
             if group.rank != 0:
                 return None
+        if hap:
+            if group is None:
+                reps = vecs
+            else:
+                reps = [vecs[0][r * half:(r + 1) * half].view(np.int32)[:nwin * fasta.nseq].reshape(nwin, fasta.nseq)
+                        for r in range(group.world)]
+            masks = None if found[0][1] is None else np.stack([mask for _, mask, _ in found])
+            return hap_rows(file, found, api.haplotype_results(api.meet_classes(reps), masks, sizes, L, W, step), window is not None)
         if window is None:
             site = aln.unpack_site(vecs[0])
             if dxy:
@@ -410,12 +457,12 @@ def alignment_rows(ctx, fasta, file, cds, jc, found, window=None, dxy=False, gro
         aln.free()
 
 
-def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None, dxy=False):
+def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None, dxy=False, hap=False):
     """items: [(path, Fasta | exception)] in output order -> ordered actions ('stdout' | 'note' | 'row', ...).
     Small non-CDS loci of the chunk share ONE batched GPU pass; everything else goes through the single-alignment path.
     window = (W, step): every alignment goes through the single-alignment path (or the column shards of `group`) and gives
     its window rows after its '# Pop ... not found' notes.  dxy: the same, with one row per population pair (and window); a file
-    with fewer than two populations found gives one more '#' note instead."""
+    with fewer than two populations found gives one more '#' note instead.  hap: the --haplotypes rows, through the same route."""
     actions = []
     pending = []   # (position in actions, locus, pop, file, seqlen, label, n)
     own_batch = None
@@ -437,14 +484,14 @@ def process_chunk(ctx, batch, items, cds, jc, popkeys, group=None, window=None, 
         plan = plan_populations(fasta, popkeys)
         found = [p for p in plan if p[2] > 0]
         rows = iter(())
-        if window is not None or dxy:
+        if window is not None or dxy or hap:
             for label, mask, hits in plan:
                 if hits == 0:
                     actions.append(("note", f"# Pop {label} string was not found in fasta headers."))   # :126-132
             if dxy and len(found) < 2:
                 actions.append(("note", f"# Fewer than two populations found in {file}: no divergence rows."))
             elif found:
-                lines = alignment_rows(ctx, fasta, file, cds, jc, found, window, dxy, group)
+                lines = alignment_rows(ctx, fasta, file, cds, jc, found, window, dxy, group, hap)
                 keys = ([f"{found[x][0]},{found[y][0]}" for x, y in api.pop_pairs(len(found))] if dxy
                         else [label for label, _, _ in found])
                 for i, line in enumerate(lines or ()):
@@ -597,17 +644,17 @@ def devices_from_env():
 _SLOTS = {}
 
 
-def run_files(paths, cds, jc, popkeys, sink, window=None, dxy=False):
+def run_files(paths, cds, jc, popkeys, sink, window=None, dxy=False, hap=False):
     """the per-file loop of PolyFastA.py:104-140 over sorted paths, in chunks; chunk i runs on device i mod G and the
     rows are emitted in the reference's order"""
     from concurrent.futures import ThreadPoolExecutor
     from . import parallel
     devs = devices_from_env()
     chunks = [ps for _, ps in parallel.plan_units(paths, [_file_size(p) for p in paths], None, BATCH_FILES, BATCH_BYTES)]
-    if window is not None or dxy:   # windows, divergence: file by file through the single-alignment path on the first listed device
+    if window is not None or dxy or hap:   # windows, divergence, haplotypes: file by file through the single-alignment path on the first listed device
         ctx = api.default_context(devs[0])
         for ps in chunks:
-            emit(process_chunk(ctx, None, list(zip(ps, api.parse_files(ps))), cds, jc, popkeys, window=window, dxy=dxy), sink)
+            emit(process_chunk(ctx, None, list(zip(ps, api.parse_files(ps))), cds, jc, popkeys, window=window, dxy=dxy, hap=hap), sink)
         return
     if len(chunks) > 1 and os.environ.get("POLYFASTA_DOUBLE_BUFFER", "1") != "0":
         devs = [d for d in devs for _ in (0, 1)]   # two slots per GPU: host staging of chunk i+1 overlaps the GPU pass of chunk i
@@ -636,7 +683,7 @@ def run_files(paths, cds, jc, popkeys, sink, window=None, dxy=False):
             pl.shutdown()
 
 
-def run_files_ranks(paths, cds, jc, popkeys, sink, group, window=None, dxy=False):
+def run_files_ranks(paths, cds, jc, popkeys, sink, group, window=None, dxy=False, hap=False):
     """the same loop under torchrun (one process per GPU).  Units in the reference's order: a file of at least
     SHARD_MIN_BYTES is ONE alignment scanned by ALL ranks in column shards (exchange fused into the kernels); the other
     files are grouped in chunks and chunk j goes to rank j mod world with no collective (SURVEY.md 8e.2).  Rank 0 gathers the
@@ -651,14 +698,14 @@ def run_files_ranks(paths, cds, jc, popkeys, sink, group, window=None, dxy=False
     for ui, (kind, ps) in enumerate(units):
         if kind == "all":
             fasta = group.parse_once(ps[0], threads)
-            acts = process_chunk(ctx, None, [(ps[0], fasta)], cds, jc, popkeys, group=group, window=window, dxy=dxy)
+            acts = process_chunk(ctx, None, [(ps[0], fasta)], cds, jc, popkeys, group=group, window=window, dxy=dxy, hap=hap)
             if group.rank == 0:
                 mine.append((ui, acts))
             continue
         if parallel.chunk_owner(j, group.world) == group.rank:
-            if window is not None or dxy:
+            if window is not None or dxy or hap:
                 mine.append((ui, process_chunk(ctx, None, list(zip(ps, api.parse_files(ps, threads))), cds, jc, popkeys, window=window,
-                                               dxy=dxy)))
+                                               dxy=dxy, hap=hap)))
             else:
                 mine.append((ui, process_chunk_native(ctx, batch, ps, jc, popkeys, threads, cds)))
         j += 1
@@ -674,6 +721,7 @@ def main(argv=None):
     args = parser.parse_args(argv)
     window = check_window_args(parser, args)
     check_dxy_args(parser, args)
+    check_hap_args(parser, args)
     if args.file == "" and args.dir == "." and not args.pipe:
         print("Both --file/-f and --dir/-d were not found.")
         r = input("Do you wish to run polySFS on all files in the current directory? [y|n]: ")
@@ -692,7 +740,7 @@ def main(argv=None):
     if group is not None and args.pipe:
         group = None
     if not args.silent and (group is None or group.rank == 0):
-        sink.header(args.cds, window is not None, args.dxy)
+        sink.header(args.cds, window is not None, args.dxy, args.haplotypes)
     popkeys = args.pops.split(",") if args.pops else None
     paths = sorted(args.file)
     if paths and args.pipe:
@@ -706,12 +754,13 @@ def main(argv=None):
                 fasta = api.Fasta.from_bytes(data)
             except api.NotFasta as e:
                 fasta = e
-            emit(process_chunk(ctx, batch, [(path, fasta)], args.cds, args.jc, popkeys, window=window, dxy=args.dxy), sink)
+            emit(process_chunk(ctx, batch, [(path, fasta)], args.cds, args.jc, popkeys, window=window, dxy=args.dxy,
+                               hap=args.haplotypes), sink)
             data = b""
     elif paths and group is not None:
-        run_files_ranks(paths, args.cds, args.jc, popkeys, sink, group, window, args.dxy)
+        run_files_ranks(paths, args.cds, args.jc, popkeys, sink, group, window, args.dxy, args.haplotypes)
     elif paths:
-        run_files(paths, args.cds, args.jc, popkeys, sink, window, args.dxy)
+        run_files(paths, args.cds, args.jc, popkeys, sink, window, args.dxy, args.haplotypes)
     if len(args.out) != 0 and not args.silent and (group is None or group.rank == 0):
         print("")
     return 0

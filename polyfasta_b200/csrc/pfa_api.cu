@@ -374,6 +374,9 @@ int pfa_aln_free(pfa_aln* a) {
     pfa_dfree(ctx, a->d_union);
     pfa_dfree(ctx, a->d_pop_n);
     pfa_dfree(ctx, a->rowmajor);
+    pfa_dfree(ctx, a->rowmajor_sites);
+    pfa_dfree(ctx, a->exc_rows);
+    pfa_dfree(ctx, a->exc_row_off);
     delete a;
     return PFA_OK;
 }
@@ -613,6 +616,15 @@ int pfa_divergence_windows(pfa_aln* a, int64_t window, int64_t step, int64_t* co
     if (!counts) return pfa_fail(a->ctx, PFA_ERR_ARG, "divergence windows: null output");
     return run_to_host(a, sizeof(int64_t) * 2 * (size_t)(P * nwin), counts, 0, nullptr,
                        [&](void* d_out, void*) { return pfa_divergence_windows_device(a, window, step, (int64_t*)d_out); });
+}
+
+int pfa_haplotypes(pfa_aln* a, int64_t window, int64_t step, int32_t* rep) {
+    if (!a) return PFA_ERR_ARG;
+    const int64_t nwin = pfa_window_count(a->L_total, window, step);
+    if (nwin <= 0 || a->n == 0) return pfa_haplotypes_device(a, window, step, nullptr);  // argument errors, or nothing to do
+    if (!rep) return pfa_fail(a->ctx, PFA_ERR_ARG, "haplotypes: null output");
+    return run_to_host(a, sizeof(int32_t) * (size_t)(nwin * a->n), rep, 0, nullptr,
+                       [&](void* d_rep, void*) { return pfa_haplotypes_device(a, window, step, (int32_t*)d_rep); });
 }
 
 int pfa_site_stats_xchg(pfa_aln* a, pfa_xchg* x, int64_t* d_out, uint8_t* d_isvar) {

@@ -87,10 +87,17 @@ struct pfa_aln {
     int64_t* d_site_off = nullptr;
     std::vector<int64_t> pop_n;
     std::vector<int64_t> site_off;  // offsets into the site result vector, size k+1
-    // row-major copy for the pairwise kernel (built lazily): [plane][n][Wl] uint32, Wl = ceil(ns/32) padded to 4
+    // row-major copy of the marked sites for the pairwise kernel and the haplotype classes (built lazily, pfa_rowmajor_ensure):
+    // [plane][n][Wl] uint32, Wl = ceil(nsel/32) padded to 4; rowmajor_sites: the nsel marked sites in ascending order
     uint32_t* rowmajor = nullptr;
     int rowmajor_planes = 0;  // 2: pure-ACGT shard (b0, b1), 3: with the validity plane
     int64_t Wl = 0;
+    int64_t* rowmajor_sites = nullptr;
+    int64_t rowmajor_nsel = 0;
+    // the exception list by row (built lazily, pfa_haplotypes.cu): keys (row:24 | site:32 | byte:8) sorted, and [n + 1] offsets:
+    // row r's entries are exc_rows[exc_row_off[r] .. exc_row_off[r + 1])
+    unsigned long long* exc_rows = nullptr;
+    int64_t* exc_row_off = nullptr;
 };
 
 // ---- error plumbing ----------------------------------------------------------------------------------
@@ -150,6 +157,8 @@ void pfa_xchg_set_carry(pfa_xchg* x, int64_t words);
 int64_t pfa_xchg_cap(const pfa_xchg* x);
 int pfa_xchg_launch_only(pfa_xchg* x, const int64_t* d_src, int64_t len, int64_t* d_out);
 int pfa_launch_pairwise(pfa_aln* a, int64_t* d_out, int32_t* d_matrix);
+// K3's steps 0 and 1 (pfa_pairwise.cu): a->rowmajor and a->rowmajor_sites, built once per alignment and number of planes
+cudaError_t pfa_rowmajor_ensure(pfa_aln* a);
 int pfa_upload_codon_tables(pfa_ctx* ctx);
 int pfa_ctx_work(pfa_ctx* ctx, unsigned int** out);
 int pfa_aln_alloc(pfa_ctx* ctx, int64_t n, int64_t L, int64_t col_begin, int64_t col_end, pfa_aln** out);

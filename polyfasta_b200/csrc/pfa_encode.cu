@@ -330,7 +330,10 @@ extern "C" int pfa_aln_poke_gaps(pfa_aln* a, uint64_t seed, uint32_t gap_ppm) {
     a->vflag_sites = -1;  // recount on the next sparse scan
     if (a->rowmajor) {  // the pairwise kernel's transposed copy is stale
         pfa_dfree(ctx, a->rowmajor);
+        pfa_dfree(ctx, a->rowmajor_sites);
         a->rowmajor = nullptr;
+        a->rowmajor_sites = nullptr;
+        a->rowmajor_nsel = 0;
     }
     return PFA_OK;
 }

@@ -8,7 +8,8 @@
 //     those can contribute to any d_ij -- the reference, too, runs over the variable columns only (:469) -- and they are
 //     a few per cent of a real alignment, so the K dimension of step 2 shrinks by that factor.
 //  1. pfa_rowmajor_kernel transposes the marked sites of the site-major planes into row-major bit-planes over SITES
-//     ([plane][row][word], 32 sites per word) with warp ballots.
+//     ([plane][row][word], 32 sites per word) with warp ballots.  Steps 0 and 1 run once per alignment (pfa_rowmajor_ensure):
+//     the planes and the list of marked sites stay with the alignment, and the haplotype classes (pfa_haplotypes.cu) reuse them.
 //  2. pfa_pairwise_kernel: one 64x64 tile of row pairs per CTA, 4x4 pairs per thread; the K dimension (site words)
 //     is staged through shared memory in [plane][word][row] order so that a thread fetches its four rows with one
 //     128-bit shared load; per word and pair: mismatch = (a0^b0)|(a1^b1)|(av^bv), POPC, add.
@@ -247,6 +248,78 @@ int pfa_launch_var_flags(pfa_aln* a, uint8_t* flags) {
     return PFA_OK;
 }
 
+// steps 0 and 1, cached with the alignment: the row-major planes of the marked sites and the sorted list of those sites (a
+// window [s, e) of this shard is the bit range [lower_bound(s), lower_bound(e)) of the row-major words).  Rebuilt when the
+// number of planes changes (pfa_aln_force_validity).
+cudaError_t pfa_rowmajor_ensure(pfa_aln* a) {
+    pfa_ctx* ctx = a->ctx;
+    const int64_t n = a->n;
+    const bool three = a->has_invalid != 0;  // the validity plane takes part only when a row shows a symbol outside ACGT
+    const int np = three ? 3 : 2;
+    if (a->ns == 0 || n == 0 || (a->rowmajor && a->rowmajor_planes == np)) return cudaSuccess;
+    pfa_dfree(ctx, a->rowmajor);
+    pfa_dfree(ctx, a->rowmajor_sites);
+    a->rowmajor = nullptr;
+    a->rowmajor_sites = nullptr;
+    a->rowmajor_nsel = 0;
+    const int Wn = a->Wq * 4;
+    const int64_t npad = (int64_t)a->Wq * 128;
+    // mark the sites at which two rows differ, list them, transpose only those
+    uint8_t* flags = nullptr;
+    int64_t *sites = nullptr, *d_num = nullptr;
+    void* tmp = nullptr;
+    size_t tmp_bytes = 0;
+    int64_t nsel = 0;
+    cudaError_t e = pfa_dmalloc(ctx, &flags, (size_t)a->ns);
+    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &sites, sizeof(int64_t) * (size_t)a->ns);
+    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &d_num, sizeof(int64_t));
+    if (e == cudaSuccess) {
+        const unsigned g = (unsigned)((a->ns + 7) / 8);
+        if (three) pfa_var_flags_kernel<3><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, n, flags);
+        else pfa_var_flags_kernel<2><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, n, flags);
+        ctx->launches++;
+        e = cudaGetLastError();
+    }
+    cub::CountingInputIterator<int64_t> idx(0);
+    if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(nullptr, tmp_bytes, idx, flags, sites, d_num, (int)a->ns, ctx->stream);
+    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &tmp, tmp_bytes);
+    if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(tmp, tmp_bytes, idx, flags, sites, d_num, (int)a->ns, ctx->stream);
+    ctx->launches += 2;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&nsel, d_num, sizeof nsel, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e == cudaSuccess) {
+        a->Wl = pfa_round_up(std::max<int64_t>((nsel + 31) / 32, 1), 4);
+        a->rowmajor_planes = np;
+        e = pfa_dmalloc(ctx, &a->rowmajor, sizeof(uint32_t) * (size_t)(np * npad * a->Wl));
+    }
+    if (e == cudaSuccess) e = cudaMemsetAsync(a->rowmajor, 0, sizeof(uint32_t) * (size_t)(np * npad * a->Wl), ctx->stream);
+    if (e == cudaSuccess && nsel > 0) {
+        const int64_t sw = (nsel + 31) / 32;
+        dim3 grid((unsigned)((sw + 7) / 8), (unsigned)Wn);
+        if (three)
+            pfa_rowmajor_kernel<3><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)a->b0, (const uint32_t*)a->b1, (const uint32_t*)a->v, sites, nsel,
+                                                                  Wn, npad, a->Wl, a->rowmajor);
+        else
+            pfa_rowmajor_kernel<2><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)a->b0, (const uint32_t*)a->b1, (const uint32_t*)a->v, sites, nsel,
+                                                                  Wn, npad, a->Wl, a->rowmajor);
+        ctx->launches++;
+        e = cudaGetLastError();
+    }
+    pfa_dfree(ctx, tmp);
+    pfa_dfree(ctx, flags);
+    pfa_dfree(ctx, d_num);
+    if (e == cudaSuccess) {
+        a->rowmajor_sites = sites;  // the first nsel entries: the marked sites in ascending order
+        a->rowmajor_nsel = nsel;
+    } else {
+        pfa_dfree(ctx, sites);
+        pfa_dfree(ctx, a->rowmajor);
+        a->rowmajor = nullptr;
+        a->rowmajor_planes = 0;
+    }
+    return e;
+}
+
 int pfa_launch_pairwise(pfa_aln* a, int64_t* d_out, int32_t* d_matrix) {
     pfa_ctx* ctx = a->ctx;
     PFA_CUDA(ctx, cudaMemsetAsync(d_out, 0, sizeof(int64_t) * (size_t)a->k, ctx->stream));
@@ -256,61 +329,12 @@ int pfa_launch_pairwise(pfa_aln* a, int64_t* d_out, int32_t* d_matrix) {
     int32_t* D = d_matrix;  // nullptr: sums only, the matrix is never materialised
     const int Wn = a->Wq * 4;
     const int64_t npad = (int64_t)a->Wq * 128;
-    const bool three = a->has_invalid != 0;  // the validity plane takes part only when a row shows a symbol outside ACGT
-    const int np = three ? 3 : 2;
+    const bool three = a->has_invalid != 0;
     int rc = PFA_OK;
     cudaError_t e = cudaSuccess;
     if (D) e = cudaMemsetAsync(D, 0, sizeof(int32_t) * (size_t)(n * n), ctx->stream);
     if (e == cudaSuccess && a->ns > 0) {
-        if (!a->rowmajor || a->rowmajor_planes != np) {
-            pfa_dfree(ctx, a->rowmajor);
-            a->rowmajor = nullptr;
-            // mark the sites at which two rows differ, list them, transpose only those
-            uint8_t* flags = nullptr;
-            int64_t *sites = nullptr, *d_num = nullptr;
-            void* tmp = nullptr;
-            size_t tmp_bytes = 0;
-            int64_t nsel = 0;
-            e = pfa_dmalloc(ctx, &flags, (size_t)a->ns);
-            if (e == cudaSuccess) e = pfa_dmalloc(ctx, &sites, sizeof(int64_t) * (size_t)a->ns);
-            if (e == cudaSuccess) e = pfa_dmalloc(ctx, &d_num, sizeof(int64_t));
-            if (e == cudaSuccess) {
-                const unsigned g = (unsigned)((a->ns + 7) / 8);
-                if (three) pfa_var_flags_kernel<3><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, n, flags);
-                else pfa_var_flags_kernel<2><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, n, flags);
-                ctx->launches++;
-                e = cudaGetLastError();
-            }
-            cub::CountingInputIterator<int64_t> idx(0);
-            if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(nullptr, tmp_bytes, idx, flags, sites, d_num, (int)a->ns, ctx->stream);
-            if (e == cudaSuccess) e = pfa_dmalloc(ctx, &tmp, tmp_bytes);
-            if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(tmp, tmp_bytes, idx, flags, sites, d_num, (int)a->ns, ctx->stream);
-            ctx->launches += 2;
-            if (e == cudaSuccess) e = cudaMemcpyAsync(&nsel, d_num, sizeof nsel, cudaMemcpyDeviceToHost, ctx->stream);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-            if (e == cudaSuccess) {
-                a->Wl = pfa_round_up(std::max<int64_t>((nsel + 31) / 32, 1), 4);
-                a->rowmajor_planes = np;
-                e = pfa_dmalloc(ctx, &a->rowmajor, sizeof(uint32_t) * (size_t)(np * npad * a->Wl));
-            }
-            if (e == cudaSuccess) e = cudaMemsetAsync(a->rowmajor, 0, sizeof(uint32_t) * (size_t)(np * npad * a->Wl), ctx->stream);
-            if (e == cudaSuccess && nsel > 0) {
-                const int64_t sw = (nsel + 31) / 32;
-                dim3 grid((unsigned)((sw + 7) / 8), (unsigned)Wn);
-                if (three)
-                    pfa_rowmajor_kernel<3><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)a->b0, (const uint32_t*)a->b1, (const uint32_t*)a->v, sites, nsel,
-                                                                          Wn, npad, a->Wl, a->rowmajor);
-                else
-                    pfa_rowmajor_kernel<2><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)a->b0, (const uint32_t*)a->b1, (const uint32_t*)a->v, sites, nsel,
-                                                                          Wn, npad, a->Wl, a->rowmajor);
-                ctx->launches++;
-                e = cudaGetLastError();
-            }
-            pfa_dfree(ctx, tmp);
-            pfa_dfree(ctx, flags);
-            pfa_dfree(ctx, sites);
-            pfa_dfree(ctx, d_num);
-        }
+        e = pfa_rowmajor_ensure(a);
         if (e == cudaSuccess) {
             const int64_t nt = npad / PW_TILE;
             const unsigned grid = (unsigned)(nt * (nt + 1) / 2);
