@@ -374,7 +374,7 @@ int pfa_aln_free(pfa_aln* a) {
     pfa_dfree(ctx, a->d_union);
     pfa_dfree(ctx, a->d_pop_n);
     pfa_dfree(ctx, a->rowmajor);
-    pfa_dfree(ctx, a->rowmajor_sites);
+    pfa_dfree(ctx, a->var_sites);
     pfa_dfree(ctx, a->exc_rows);
     pfa_dfree(ctx, a->exc_row_off);
     delete a;
@@ -775,6 +775,8 @@ void pfa_fill_site_args(const pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, PfaS
     args->hsite = d_hsite;
     args->ns = a->ns;
     args->vflag = nullptr;  // the launchers switch the sparse validity fetch on
+    args->sites = nullptr;  // ... and the site list
+    args->nsites = a->ns;
     args->gc = a->gc;
     args->vs = 0;
     args->Wq = a->Wq;

@@ -1214,7 +1214,7 @@ int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg*
         const int gw = 32 / lps, nwarp = nt / 32;
         const size_t queues = lps >= 4 ? (size_t)nwarp * PFA_CDS_QFIELDS * 32 * sizeof(uint32_t) : 0;  // pfa_cds_flush
         const int m = (int)std::max<int64_t>(1, 10000 / ((int64_t)gw * 3 * a->Wq * 16));
-        const PfaTmaShape shape = {3, args.ncf, lps, nt, m, "PFA_CDS_TMA_M", 8, 1, smem + queues, hv};
+        const PfaTmaShape shape = {3, args.ncf, lps, nt, m, "PFA_CDS_TMA_M", 8, 1, smem + queues, hv, a->ns};
         PfaTmaPlan p;
         if (int rc = pfa_tma_plan(a, shape, &p)) return rc;
         if (p.sparse_v) args.s.vflag = a->vflag;

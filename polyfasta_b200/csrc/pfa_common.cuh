@@ -87,13 +87,16 @@ struct pfa_aln {
     int64_t* d_site_off = nullptr;
     std::vector<int64_t> pop_n;
     std::vector<int64_t> site_off;  // offsets into the site result vector, size k+1
-    // row-major copy of the marked sites for the pairwise kernel and the haplotype classes (built lazily, pfa_rowmajor_ensure):
-    // [plane][n][Wl] uint32, Wl = ceil(nsel/32) padded to 4; rowmajor_sites: the nsel marked sites in ascending order
+    // the sites of this shard at which two of the n rows differ in the planes, ascending (built lazily, pfa_var_sites_ensure;
+    // dropped with rowmajor by every writer of the planes): the sites the TMA site scan, the divergence scan and the row-major
+    // planes visit.  n_var_sites: their number, -1 while the list is not built.
+    int64_t* var_sites = nullptr;
+    int64_t n_var_sites = -1;
+    // row-major copy of the listed sites for the pairwise kernel and the haplotype classes (built lazily, pfa_rowmajor_ensure):
+    // [plane][n][Wl] uint32, Wl = ceil(n_var_sites/32) padded to 4
     uint32_t* rowmajor = nullptr;
     int rowmajor_planes = 0;  // 2: pure-ACGT shard (b0, b1), 3: with the validity plane
     int64_t Wl = 0;
-    int64_t* rowmajor_sites = nullptr;
-    int64_t rowmajor_nsel = 0;
     // the exception list by row (built lazily, pfa_haplotypes.cu): keys (row:24 | site:32 | byte:8) sorted, and [n + 1] offsets:
     // row r's entries are exc_rows[exc_row_off[r] .. exc_row_off[r + 1])
     unsigned long long* exc_rows = nullptr;
@@ -142,8 +145,10 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
 // windows of this shard (pfa_windows.cu) for `rows` rows of per-site values d_persite [rows][ns]: d_counts [rows][nwin][2] =
 // (non-zero sites, sum); the site scan's per-site H gives (S, H) per population, the divergence scan's Dxy_site per pair
 int pfa_launch_row_windows(pfa_aln* a, int rows, const int64_t* d_persite, int64_t window, int64_t step, int64_t* d_counts);
-// K3's first step alone: flags[s] = 1 where two of the n rows differ in the planes (pfa_pairwise.cu)
-int pfa_launch_var_flags(pfa_aln* a, uint8_t* flags);
+// a->var_sites and a->n_var_sites, built once per alignment (pfa_pairwise.cu)
+cudaError_t pfa_var_sites_ensure(pfa_aln* a);
+// drops what was derived from the planes (the site list, the row-major planes): every writer of the planes after construction
+void pfa_aln_planes_changed(pfa_aln* a);
 int pfa_launch_cds_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_labels, pfa_xchg* x = nullptr);
 // codon windows: bins [k][PFA_CDS_WIN_LEN][nb] (zeroed) of this shard from K2's per-site H and K4's labels (pfa_codon.cu), and
 // the window vectors [k][nwin][PFA_CDS_WIN_LEN] from them (pfa_windows.cu)
@@ -157,7 +162,7 @@ void pfa_xchg_set_carry(pfa_xchg* x, int64_t words);
 int64_t pfa_xchg_cap(const pfa_xchg* x);
 int pfa_xchg_launch_only(pfa_xchg* x, const int64_t* d_src, int64_t len, int64_t* d_out);
 int pfa_launch_pairwise(pfa_aln* a, int64_t* d_out, int32_t* d_matrix);
-// K3's steps 0 and 1 (pfa_pairwise.cu): a->rowmajor and a->rowmajor_sites, built once per alignment and number of planes
+// K3's step 1 (pfa_pairwise.cu): a->rowmajor, built once per alignment and number of planes
 cudaError_t pfa_rowmajor_ensure(pfa_aln* a);
 int pfa_upload_codon_tables(pfa_ctx* ctx);
 int pfa_ctx_work(pfa_ctx* ctx, unsigned int** out);

@@ -5,8 +5,9 @@
 //   Dxy_site(c) = n_x n_y - sum_a c_{X,a} c_{Y,a}
 // = the number of ordered row pairs (i in X, j in Y) whose characters differ at c (a row in both populations compares equal to
 // itself).  D_xy = sum_c Dxy_site(c) is an exact int64 that column shards add up; floats appear only in the finalisation.
-//   0. pfa_launch_var_flags (K3's first step, pfa_pairwise.cu) marks the sites at which two rows differ in the planes;
-//      cub::DeviceSelect lists them.  No other site has a non-zero Dxy_site, except sites where only escape BYTES differ.
+//   0. the alignment's list of the sites at which two rows differ in the planes (pfa_var_sites_ensure, K3's first step in
+//      pfa_pairwise.cu, built once and shared with the site scan).  No other site has a non-zero Dxy_site, except sites where
+//      only escape BYTES differ.
 //   1. pfa_divergence_kernel<HAS_V>: one warp per listed site.  Class counts per population (pfa_class_counts), per-pair
 //      cross terms from the lanes, per-pair totals in registers / shared memory, one global atomic per block and pair.
 //      A site where some population has an escape row is left to step 2, so nothing is counted twice.
@@ -17,9 +18,6 @@
 //   4. pfa_div_finalize_kernel: dxy, d_a, F_ST in fp64 with round-to-nearest intrinsics (-fmad=false for the library).
 #include <algorithm>
 #include <climits>
-
-#include <cub/device/device_select.cuh>
-#include <cub/iterator/counting_input_iterator.cuh>
 
 #include "pfa_common.cuh"
 #include "pfa_sites.cuh"
@@ -78,7 +76,7 @@ __device__ __forceinline__ unsigned long long pfa_div_plane_d(const uint32_t* cx
 template <bool HAS_V>
 __global__ void __launch_bounds__(256) pfa_divergence_kernel(const uint4* __restrict__ b0, const uint4* __restrict__ b1, const uint4* __restrict__ v,
                                                              const uint4* __restrict__ masks, int Wq, const int64_t* __restrict__ pop_n, int k,
-                                                             const int64_t* __restrict__ sites, const int64_t* __restrict__ nsel, int64_t ns,
+                                                             const int64_t* __restrict__ sites, int64_t m, int64_t ns,
                                                              unsigned long long* __restrict__ out, int64_t* __restrict__ dsite) {
     __shared__ uint32_t cnt[PFA_DIV_WARPS][PFA_DIV_MAX_POPS][8];
     __shared__ unsigned long long tot[PFA_DIV_MAX_PAIRS];
@@ -89,7 +87,6 @@ __global__ void __launch_bounds__(256) pfa_divergence_kernel(const uint4* __rest
     __syncthreads();
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int64_t nwarps = (int64_t)gridDim.x * PFA_DIV_WARPS;
-    const int64_t m = *nsel;
     unsigned long long acc = 0;  // pair `lane` (the pairs from 32 on add into shared memory site by site)
     for (int64_t i = (int64_t)blockIdx.x * PFA_DIV_WARPS + wib; i < m; i += nwarps) {
         const int64_t s = sites[i];
@@ -222,32 +219,19 @@ static int pfa_launch_divergence(pfa_aln* a, int64_t* d_out, int64_t* d_dsite) {
     PFA_CUDA(ctx, cudaMemsetAsync(d_out, 0, sizeof(int64_t) * (size_t)P, ctx->stream));
     if (d_dsite && a->ns > 0) PFA_CUDA(ctx, cudaMemsetAsync(d_dsite, 0, sizeof(int64_t) * (size_t)(P * a->ns), ctx->stream));
     if (a->ns == 0 || a->n == 0) return PFA_OK;
-    uint8_t* flags = nullptr;
-    int64_t *sites = nullptr, *d_num = nullptr;
-    void* tmp = nullptr;
-    size_t tmp_bytes = 0;
-    cudaError_t e = pfa_dmalloc(ctx, &flags, (size_t)a->ns);
-    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &sites, sizeof(int64_t) * (size_t)a->ns);
-    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &d_num, sizeof(int64_t));
-    int rc = e == cudaSuccess ? PFA_OK : pfa_fail(ctx, PFA_ERR_CUDA, "divergence: cudaMallocAsync failed: %s", cudaGetErrorString(e));
-    if (!rc) rc = pfa_launch_var_flags(a, flags);
-    cub::CountingInputIterator<int64_t> idx(0);
-    if (!rc) {
-        e = cub::DeviceSelect::Flagged(nullptr, tmp_bytes, idx, flags, sites, d_num, (int)a->ns, ctx->stream);
-        if (e == cudaSuccess) e = pfa_dmalloc(ctx, &tmp, tmp_bytes);
-        if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(tmp, tmp_bytes, idx, flags, sites, d_num, (int)a->ns, ctx->stream);
-        ctx->launches++;
-        if (e != cudaSuccess) rc = pfa_fail(ctx, PFA_ERR_CUDA, "divergence: site list failed: %s", cudaGetErrorString(e));
-    }
+    cudaError_t e = pfa_var_sites_ensure(a);
+    if (e != cudaSuccess) return pfa_fail(ctx, PFA_ERR_CUDA, "divergence: site list failed: %s", cudaGetErrorString(e));
+    int rc = PFA_OK;
     unsigned long long* out = reinterpret_cast<unsigned long long*>(d_out);
     const uint4* masks = a->d_masks;
-    if (!rc) {
-        // the number of listed sites stays on the device: the grid covers every site, warps beyond the list exit at once
-        const unsigned grid = pfa_div_grid(ctx, a->ns);
+    if (!rc && a->n_var_sites > 0) {
+        const unsigned grid = pfa_div_grid(ctx, a->n_var_sites);
         if (a->has_invalid)
-            pfa_divergence_kernel<true><<<grid, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, masks, a->Wq, a->d_pop_n, a->k, sites, d_num, a->ns, out, d_dsite);
+            pfa_divergence_kernel<true><<<grid, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, masks, a->Wq, a->d_pop_n, a->k, a->var_sites, a->n_var_sites,
+                                                                       a->ns, out, d_dsite);
         else
-            pfa_divergence_kernel<false><<<grid, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, masks, a->Wq, a->d_pop_n, a->k, sites, d_num, a->ns, out, d_dsite);
+            pfa_divergence_kernel<false><<<grid, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, masks, a->Wq, a->d_pop_n, a->k, a->var_sites, a->n_var_sites,
+                                                                        a->ns, out, d_dsite);
         ctx->launches++;
         e = cudaGetLastError();
         if (e != cudaSuccess) rc = pfa_fail(ctx, PFA_ERR_CUDA, "divergence: kernel launch failed: %s", cudaGetErrorString(e));
@@ -259,10 +243,6 @@ static int pfa_launch_divergence(pfa_aln* a, int64_t* d_out, int64_t* d_dsite) {
         e = cudaGetLastError();
         if (e != cudaSuccess) rc = pfa_fail(ctx, PFA_ERR_CUDA, "divergence: escape kernel launch failed: %s", cudaGetErrorString(e));
     }
-    pfa_dfree(ctx, tmp);
-    pfa_dfree(ctx, d_num);
-    pfa_dfree(ctx, sites);
-    pfa_dfree(ctx, flags);
     return rc;
 }
 

@@ -3,7 +3,7 @@
 // K3's d_ij is 0 over those columns: their bits agree at every site K3 marks (the only sites where two rows can differ in the
 // planes) and they show the same escape bytes at the same sites.
 //
-//  0. K3's row-major planes of the marked sites and their sorted site list (pfa_rowmajor_ensure, cached with the alignment);
+//  0. K3's row-major planes of the listed sites (pfa_rowmajor_ensure) and the site list (pfa_aln::var_sites), cached with the alignment;
 //     window w of this shard is the local column range [s, e) and the bit range [lo, hi) of the row-major words, found by a
 //     binary search over the site list (pfa_hap_windows_kernel).  The exception list is copied once per alignment in row
 //     order: (row:24 | site:32 | byte:8) keys, radix-sorted, with an offset per row (pfa_hap_exc_rows_kernel, _offsets_kernel).
@@ -378,7 +378,7 @@ extern "C" int pfa_haplotypes_device(pfa_aln* a, int64_t window, int64_t step, i
     const int64_t cmax = (std::min(window, a->ns) / 32 + 5 + PFA_HAP_CHUNK - 1) / PFA_HAP_CHUNK;
     if (e == cudaSuccess && cmax > 1) e = cudaMemsetAsync(keys, 0, sizeof(unsigned long long) * (size_t)N, ctx->stream);
     if (e == cudaSuccess) {
-        pfa_hap_windows_kernel<<<(unsigned)((nwin + 255) / 256), 256, 0, ctx->stream>>>(a->rowmajor_sites, a->rowmajor_nsel, a->L_total, window, step,
+        pfa_hap_windows_kernel<<<(unsigned)((nwin + 255) / 256), 256, 0, ctx->stream>>>(a->var_sites, a->n_var_sites, a->L_total, window, step,
                                                                                       a->col_begin, a->ns, nwin, win);
         pfa_hap_offsets_kernel<<<(unsigned)((nwin + 1 + 255) / 256), 256, 0, ctx->stream>>>(n, nwin, off);
         pfa_hap_hash_kernel<<<pfa_hap_grid(ctx, N * cmax * 32), 256, 0, ctx->stream>>>(a->rowmajor, np, npad, a->Wl, win, nwin, n, cmax,

@@ -4,12 +4,13 @@
 // identity sum_{i<j} d_ij = H/2 ties it to the site scan.  Integer work on the INT pipe -- XOR / OR / POPC over
 // packed words -- not tensor cores.
 //
-//  0. pfa_var_flags_kernel marks the sites at which at least two rows differ (one memory-bound pass over the planes); only
+//  0. pfa_var_flags_kernel marks the sites at which at least two rows differ (one memory-bound pass over the planes) and cub
+//     lists them (pfa_var_sites_ensure, once per alignment; the site scan and the divergence scan use the same list); only
 //     those can contribute to any d_ij -- the reference, too, runs over the variable columns only (:469) -- and they are
 //     a few per cent of a real alignment, so the K dimension of step 2 shrinks by that factor.
-//  1. pfa_rowmajor_kernel transposes the marked sites of the site-major planes into row-major bit-planes over SITES
-//     ([plane][row][word], 32 sites per word) with warp ballots.  Steps 0 and 1 run once per alignment (pfa_rowmajor_ensure):
-//     the planes and the list of marked sites stay with the alignment, and the haplotype classes (pfa_haplotypes.cu) reuse them.
+//  1. pfa_rowmajor_kernel transposes the listed sites of the site-major planes into row-major bit-planes over SITES
+//     ([plane][row][word], 32 sites per word) with warp ballots, once per alignment (pfa_rowmajor_ensure): the planes stay
+//     with the alignment, and the haplotype classes (pfa_haplotypes.cu) reuse them.
 //  2. pfa_pairwise_kernel: one 64x64 tile of row pairs per CTA, 4x4 pairs per thread; the K dimension (site words)
 //     is staged through shared memory in [plane][word][row] order so that a thread fetches its four rows with one
 //     128-bit shared load; per word and pair: mismatch = (a0^b0)|(a1^b1)|(av^bv), POPC, add.
@@ -19,6 +20,8 @@
 // A pure-ACGT shard (no validity plane needed) runs the two-plane instantiations: a third fewer logic ops and shared-memory
 // traffic in step 2.  When the caller wants only the sums, the n x n matrix is never written: every tile folds its pairs
 // into the per-population sums in registers (pfa_pairwise_kernel<NP, false>).
+#include <climits>
+
 #include <cub/device/device_select.cuh>
 #include <cub/iterator/counting_input_iterator.cuh>
 
@@ -61,14 +64,14 @@ __global__ void __launch_bounds__(256) pfa_var_flags_kernel(const uint4* __restr
     if (lane == 0) flags[site] = (uint8_t)both;
 }
 
-// sites[i]: the i-th marked site; word sw of the row-major planes holds marked sites 32*sw .. 32*sw+31
+// sites[i]: the i-th listed site; word sw of the row-major planes holds listed sites 32*sw .. 32*sw+31
 template <int NP>
 __global__ void __launch_bounds__(256) pfa_rowmajor_kernel(const uint32_t* __restrict__ b0, const uint32_t* __restrict__ b1,
                                                            const uint32_t* __restrict__ v, const int64_t* __restrict__ sites,
                                                            int64_t nsel, int Wn, int64_t npad, int64_t Wl,
                                                            uint32_t* __restrict__ out) {
     const int lane = threadIdx.x & 31;
-    const int64_t sw = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);  // word over marked sites
+    const int64_t sw = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);  // word over listed sites
     const int64_t w = blockIdx.y;                                                      // word over rows
     if (sw * 32 >= nsel) return;
     const int64_t idx = sw * 32 + lane;
@@ -236,21 +239,65 @@ __global__ void __launch_bounds__(256) pfa_pairwise_popsum_kernel(const int32_t*
     }
 }
 
-// step 0 alone, for the divergence scan (pfa_divergence.cu): flags[s] = 1 where two rows differ in the planes; the two-plane
-// instantiation for a pure-ACGT shard, as below
-int pfa_launch_var_flags(pfa_aln* a, uint8_t* flags) {
+// step 0, cached with the alignment: the ascending list of the sites at which two rows differ.  The site scan walks it on
+// sparse shapes, the divergence scan takes its sites from it, step 1 transposes them.  A forced validity plane does not change
+// it (the v plane of a shard without invalid rows is all ones in the real rows), so two planes are read unless a row is invalid.
+cudaError_t pfa_var_sites_ensure(pfa_aln* a) {
+    if (a->n_var_sites >= 0) return cudaSuccess;
     pfa_ctx* ctx = a->ctx;
-    if (a->ns == 0) return PFA_OK;
-    const unsigned g = (unsigned)((a->ns + 7) / 8);
-    if (a->has_invalid) pfa_var_flags_kernel<3><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, a->n, flags);
-    else pfa_var_flags_kernel<2><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, a->n, flags);
-    PFA_LAUNCH_CHECK(ctx);
-    return PFA_OK;
+    if (a->ns > INT_MAX) return cudaErrorInvalidValue;  // cub's item count
+    uint8_t* flags = nullptr;
+    int64_t *sel = nullptr, *d_num = nullptr, *list = nullptr;
+    void* tmp = nullptr;
+    size_t tmp_bytes = 0;
+    int64_t nsel = 0;
+    cudaError_t e = cudaSuccess;
+    if (a->ns > 0 && a->n > 0) {
+        e = pfa_dmalloc(ctx, &flags, (size_t)a->ns);
+        if (e == cudaSuccess) e = pfa_dmalloc(ctx, &sel, sizeof(int64_t) * (size_t)a->ns);
+        if (e == cudaSuccess) e = pfa_dmalloc(ctx, &d_num, sizeof(int64_t));
+        if (e == cudaSuccess) {
+            const unsigned g = (unsigned)((a->ns + 7) / 8);
+            if (a->has_invalid & 1) pfa_var_flags_kernel<3><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, a->n, flags);
+            else pfa_var_flags_kernel<2><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, a->n, flags);
+            ctx->launches++;
+            e = cudaGetLastError();
+        }
+        cub::CountingInputIterator<int64_t> idx(0);
+        if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(nullptr, tmp_bytes, idx, flags, sel, d_num, (int)a->ns, ctx->stream);
+        if (e == cudaSuccess) e = pfa_dmalloc(ctx, &tmp, tmp_bytes);
+        if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(tmp, tmp_bytes, idx, flags, sel, d_num, (int)a->ns, ctx->stream);
+        ctx->launches += 2;
+        if (e == cudaSuccess) e = cudaMemcpyAsync(&nsel, d_num, sizeof nsel, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    }
+    // kept at its exact length: the select's output has room for every site of the shard
+    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &list, sizeof(int64_t) * (size_t)std::max<int64_t>(nsel, 1));
+    if (e == cudaSuccess && nsel > 0) e = cudaMemcpyAsync(list, sel, sizeof(int64_t) * (size_t)nsel, cudaMemcpyDeviceToDevice, ctx->stream);
+    pfa_dfree(ctx, tmp);
+    pfa_dfree(ctx, d_num);
+    pfa_dfree(ctx, sel);
+    pfa_dfree(ctx, flags);
+    if (e != cudaSuccess) {
+        pfa_dfree(ctx, list);
+        return e;
+    }
+    a->var_sites = list;
+    a->n_var_sites = nsel;
+    return cudaSuccess;
 }
 
-// steps 0 and 1, cached with the alignment: the row-major planes of the marked sites and the sorted list of those sites (a
-// window [s, e) of this shard is the bit range [lower_bound(s), lower_bound(e)) of the row-major words).  Rebuilt when the
-// number of planes changes (pfa_aln_force_validity).
+void pfa_aln_planes_changed(pfa_aln* a) {
+    pfa_dfree(a->ctx, a->rowmajor);
+    pfa_dfree(a->ctx, a->var_sites);
+    a->rowmajor = nullptr;
+    a->rowmajor_planes = 0;
+    a->var_sites = nullptr;
+    a->n_var_sites = -1;
+}
+
+// step 1, cached with the alignment: the row-major planes of the listed sites (a window [s, e) of this shard is the bit range
+// [lower_bound(s), lower_bound(e)) of the row-major words).  Rebuilt when the number of planes changes (pfa_aln_force_validity).
 cudaError_t pfa_rowmajor_ensure(pfa_aln* a) {
     pfa_ctx* ctx = a->ctx;
     const int64_t n = a->n;
@@ -258,64 +305,34 @@ cudaError_t pfa_rowmajor_ensure(pfa_aln* a) {
     const int np = three ? 3 : 2;
     if (a->ns == 0 || n == 0 || (a->rowmajor && a->rowmajor_planes == np)) return cudaSuccess;
     pfa_dfree(ctx, a->rowmajor);
-    pfa_dfree(ctx, a->rowmajor_sites);
     a->rowmajor = nullptr;
-    a->rowmajor_sites = nullptr;
-    a->rowmajor_nsel = 0;
+    a->rowmajor_planes = 0;
     const int Wn = a->Wq * 4;
     const int64_t npad = (int64_t)a->Wq * 128;
-    // mark the sites at which two rows differ, list them, transpose only those
-    uint8_t* flags = nullptr;
-    int64_t *sites = nullptr, *d_num = nullptr;
-    void* tmp = nullptr;
-    size_t tmp_bytes = 0;
-    int64_t nsel = 0;
-    cudaError_t e = pfa_dmalloc(ctx, &flags, (size_t)a->ns);
-    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &sites, sizeof(int64_t) * (size_t)a->ns);
-    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &d_num, sizeof(int64_t));
-    if (e == cudaSuccess) {
-        const unsigned g = (unsigned)((a->ns + 7) / 8);
-        if (three) pfa_var_flags_kernel<3><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, n, flags);
-        else pfa_var_flags_kernel<2><<<g, 256, 0, ctx->stream>>>(a->b0, a->b1, a->v, a->ns, a->Wq, n, flags);
-        ctx->launches++;
-        e = cudaGetLastError();
-    }
-    cub::CountingInputIterator<int64_t> idx(0);
-    if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(nullptr, tmp_bytes, idx, flags, sites, d_num, (int)a->ns, ctx->stream);
-    if (e == cudaSuccess) e = pfa_dmalloc(ctx, &tmp, tmp_bytes);
-    if (e == cudaSuccess) e = cub::DeviceSelect::Flagged(tmp, tmp_bytes, idx, flags, sites, d_num, (int)a->ns, ctx->stream);
-    ctx->launches += 2;
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&nsel, d_num, sizeof nsel, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e == cudaSuccess) {
-        a->Wl = pfa_round_up(std::max<int64_t>((nsel + 31) / 32, 1), 4);
-        a->rowmajor_planes = np;
-        e = pfa_dmalloc(ctx, &a->rowmajor, sizeof(uint32_t) * (size_t)(np * npad * a->Wl));
-    }
-    if (e == cudaSuccess) e = cudaMemsetAsync(a->rowmajor, 0, sizeof(uint32_t) * (size_t)(np * npad * a->Wl), ctx->stream);
+    cudaError_t e = pfa_var_sites_ensure(a);
+    if (e != cudaSuccess) return e;
+    const int64_t nsel = a->n_var_sites;
+    const int64_t Wl = pfa_round_up(std::max<int64_t>((nsel + 31) / 32, 1), 4);
+    e = pfa_dmalloc(ctx, &a->rowmajor, sizeof(uint32_t) * (size_t)(np * npad * Wl));
+    if (e == cudaSuccess) e = cudaMemsetAsync(a->rowmajor, 0, sizeof(uint32_t) * (size_t)(np * npad * Wl), ctx->stream);
     if (e == cudaSuccess && nsel > 0) {
         const int64_t sw = (nsel + 31) / 32;
         dim3 grid((unsigned)((sw + 7) / 8), (unsigned)Wn);
         if (three)
-            pfa_rowmajor_kernel<3><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)a->b0, (const uint32_t*)a->b1, (const uint32_t*)a->v, sites, nsel,
-                                                                  Wn, npad, a->Wl, a->rowmajor);
+            pfa_rowmajor_kernel<3><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)a->b0, (const uint32_t*)a->b1, (const uint32_t*)a->v, a->var_sites,
+                                                                  nsel, Wn, npad, Wl, a->rowmajor);
         else
-            pfa_rowmajor_kernel<2><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)a->b0, (const uint32_t*)a->b1, (const uint32_t*)a->v, sites, nsel,
-                                                                  Wn, npad, a->Wl, a->rowmajor);
+            pfa_rowmajor_kernel<2><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)a->b0, (const uint32_t*)a->b1, (const uint32_t*)a->v, a->var_sites,
+                                                                  nsel, Wn, npad, Wl, a->rowmajor);
         ctx->launches++;
         e = cudaGetLastError();
     }
-    pfa_dfree(ctx, tmp);
-    pfa_dfree(ctx, flags);
-    pfa_dfree(ctx, d_num);
     if (e == cudaSuccess) {
-        a->rowmajor_sites = sites;  // the first nsel entries: the marked sites in ascending order
-        a->rowmajor_nsel = nsel;
+        a->Wl = Wl;
+        a->rowmajor_planes = np;
     } else {
-        pfa_dfree(ctx, sites);
         pfa_dfree(ctx, a->rowmajor);
         a->rowmajor = nullptr;
-        a->rowmajor_planes = 0;
     }
     return e;
 }

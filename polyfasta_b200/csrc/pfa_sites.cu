@@ -11,10 +11,16 @@
 // symbol classes per population with popcounts and warp reductions.  Sites holding "escape" symbols (IUPAC
 // codes etc., which are distinct alleles in the reference) are finished by pfa_escape_sites_kernel from the
 // sorted exception list.
+#include <climits>
 #include <cstdio>
 #include <cstdlib>
 
 #include "pfa_sites.cuh"
+
+// the site scan walks the list of sites where two rows differ when at most this share of the shard's sites is listed
+// (pfa_launch_site_scan).  scripts/probe_var_sites.py, B200: the list path stops beating the dense one between 30 and 40 % at
+// 2,000 rows and between 70 and 100 % at 10,000 (profiles/r4_probe_var_sites.log)
+#define PFA_SITE_LIST_SHARE 0.4
 
 template <bool HAS_V>
 __global__ void __launch_bounds__(PFA_SITE_THREADS) pfa_site_scan_kernel(const PfaSiteArgs a) {
@@ -467,6 +473,8 @@ __device__ __forceinline__ void pfa_site_gap_apply(const PfaSiteArgs& a, int64_t
 // The slot is refilled once its last pass no longer needs it: right after pass 1 when that pass found no variable site,
 // else after their second pass -- every shared-memory read of the slot has then been consumed (its value was used), and a
 // proxy fence orders those generic-proxy reads before the bulk copy's async-proxy writes.
+// With a site list (a.sites: the sites where two rows differ, pfa_var_sites_ensure) a block is SPS consecutive ENTRIES of the
+// list and every record comes with a bulk copy of its own: the monomorphic sites of a sparse alignment are never read.
 template <int LPS, int ITER, bool HAS_V, bool MULTI>
 __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSiteArgs a, int m) {
     constexpr int NT = 512;
@@ -504,8 +512,13 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
     const unsigned gmask = LPS == 32 ? 0xffffffffu : (((1u << LPS) - 1u) << (lane - sub));
     unsigned char* ring = ring_base + (size_t)wib * slot_bytes;
     uint64_t* bar = bars + wib;
-    const int64_t nw = (int64_t)gridDim.x * NWARP;
-    const int64_t nblk = (a.ns + SPS - 1) / SPS;                     // blocks of SPS consecutive sites
+    // The validity-aware instantiations walk every site: they sit at the 128-register limit, and the list's indexing spilled
+    // 8-20 bytes there (ptxas), so the launcher gives the list to pure-ACGT shards only.
+    const int64_t* const sites = HAS_V ? nullptr : a.sites;
+    const int64_t nunits = HAS_V ? a.ns : a.nsites;  // entries of the site list, or sites
+    const int64_t nblk = (nunits + SPS - 1) / SPS;   // blocks of SPS consecutive entries (sites)
+    // the site of entry e: the e-th listed site, or site e; a.ns past the end (every use tests s < a.ns)
+    auto site_of = [&](int64_t e) -> int64_t { return !sites ? e : e < nunits ? __ldg(sites + e) : a.ns; };
     const unsigned char* planes[3] = {reinterpret_cast<const unsigned char*>(a.b0), reinterpret_cast<const unsigned char*>(a.b1),
                                       reinterpret_cast<const unsigned char*>(a.v)};
     uint32_t S_mine = 0;               // COOP: S and H of population `sub`
@@ -538,8 +551,8 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
     auto load_flags = [&]() {
 #pragma unroll
         for (int u = 0; u < PFA_VF_REGS; ++u) {
-            const int64_t s = (int64_t)pend * SPS + u * 32 + lane;
-            pfl[u] = (sparse && pend >= 0 && u * 32 + lane < SPS && s < a.ns) ? __ldg(a.vflag + s) : 0u;
+            const int64_t e = (int64_t)pend * SPS + u * 32 + lane;
+            pfl[u] = (sparse && pend >= 0 && u * 32 + lane < SPS && e < nunits) ? __ldg(a.vflag + site_of(e)) : 0u;
         }
     };
     load_flags();
@@ -547,9 +560,9 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
     auto issue_next = [&]() -> int {  // all lanes: fetch `pend` into the warp's slot, then look one block further ahead
         const int blk = pend;
         if (blk >= 0) {
-            const int64_t s0 = (int64_t)blk * SPS;
-            pend_v = pfa_slot_issue<HAS_V>(ring, bar, planes[0], planes[1], planes[2], sparse, gc, s0, (unsigned)min((int64_t)SPS, a.ns - s0),
-                                           (unsigned)SPS, VS, rec, Wq, pfl, lane);
+            const int64_t e0 = (int64_t)blk * SPS;
+            pend_v = pfa_slot_issue<HAS_V>(ring, bar, planes[0], planes[1], planes[2], sparse, gc, e0, (unsigned)min((int64_t)SPS, nunits - e0),
+                                           (unsigned)SPS, VS, rec, Wq, pfl, lane, sites ? sites + e0 : nullptr);
         }
         pend = blk >= 0 ? next_block() : -1;
         load_flags();
@@ -574,7 +587,7 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
                 // for both: the kernel's hot loop has to fit the instruction cache (a version with the refill and the second pass
                 // inlined per path -- 7,000 instructions -- stalled 6 cycles per issue on instruction fetch, ncu r2w_k2g).
                 const int idx = t * GW + grp;  // site of this group inside the slot
-                const int64_t s = blk * SPS + idx;
+                const int64_t s = site_of(blk * SPS + idx);
                 const uint4* q0 = reinterpret_cast<const uint4*>(slot + (size_t)idx * rec);
                 const uint4* q1 = reinterpret_cast<const uint4*>(slot + (size_t)(SPS + idx) * rec);
                 const uint32_t* fa = pfa_slot_flags(slot, (unsigned)SPS, VS, rec);  // flag words of the slot's sites (sparse)
@@ -633,12 +646,13 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
                     const uint32_t* r0 = reinterpret_cast<const uint32_t*>(slot + (size_t)vidx * rec);
                     const uint32_t* r1 = reinterpret_cast<const uint32_t*>(slot + (size_t)(SPS + vidx) * rec);
                     const uint32_t fwv = !(HAS_V && bv) ? 0u : sparse ? fa[vidx] : 0xffffffffu;
+                    const int64_t sv = site_of(blk * SPS + vidx);
                     if (HAS_V && fwv)
-                        pfa_site_coop<LPS, HAS_V, MULTI>(a, blk * SPS + vidx, r0, r1,
-                                                         reinterpret_cast<const uint32_t*>(pfa_slot_vrec(slot, (unsigned)SPS, VS, rec, sparse, vidx, planes[2] + (size_t)(blk * SPS + vidx) * rec)),
+                        pfa_site_coop<LPS, HAS_V, MULTI>(a, sv, r0, r1,
+                                                         reinterpret_cast<const uint32_t*>(pfa_slot_vrec(slot, (unsigned)SPS, VS, rec, sparse, vidx, planes[2] + (size_t)sv * rec)),
                                                          Wq * 4, lane, sm_SH, sm_sfs, S_mine, H_mine, fwv, gcr);
                     else
-                        pfa_site_coop<LPS, false, MULTI>(a, blk * SPS + vidx, r0, r1, r0, Wq * 4, lane, sm_SH, sm_sfs, S_mine, H_mine, 0u, 0u);
+                        pfa_site_coop<LPS, false, MULTI>(a, sv, r0, r1, r0, Wq * 4, lane, sm_SH, sm_sfs, S_mine, H_mine, 0u, 0u);
                 }
                 // the slot's last pass no longer needs it: fetch the next block; what is left of a gap site runs on registers
                 // while that block is on its way
@@ -646,7 +660,7 @@ __global__ void __launch_bounds__(512, 1) pfa_site_scan_tma_kernel(const PfaSite
                 if (HAS_V && !MULTI && gapsite) pfa_site_gap_apply<LPS, true>(a, s, 0, pa, pb, sub, gmask, sm_SH, S_mine, H_mine);
             } else {
                 const int idx = t * GW + grp;  // site of this group inside the slot
-                const int64_t s = blk * SPS + idx;
+                const int64_t s = site_of(blk * SPS + idx);
                 const uint4* q0 = reinterpret_cast<const uint4*>(slot + (size_t)idx * rec);
                 const uint4* q1 = reinterpret_cast<const uint4*>(slot + (size_t)(SPS + idx) * rec);
                 const uint4* qv = reinterpret_cast<const uint4*>(slot + (size_t)(2 * SPS + idx) * rec);
@@ -715,7 +729,7 @@ int pfa_tma_plan(pfa_aln* a, const PfaTmaShape& s, PfaTmaPlan* p) {
     p->v_div = 1;
     if (p->sparse_v && !(vcompact && atoi(vcompact) == 0))
         for (int d = s.v_div_max; d > 1 && p->v_div == 1; d /= 2)
-            if (p->flagged_sites * d * d <= a->ns) p->v_div = d;
+            if (p->flagged_sites * d * d <= s.sites) p->v_div = d;
     if (p->sparse_v && vdiv) p->v_div = std::max(1, std::min(8, atoi(vdiv)));  // tests: force a small v area
     if (p->v_div > 1 && !m_env) m = std::min(m + (m * s.m_raise + 1) / 2, m_sparse);
     auto vs_for = [&](int mm) { return s.has_v ? std::max(s.recs, s.recs * gw * mm / p->v_div) : 0; };
@@ -749,6 +763,26 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
         if (a->ns == 0 || a->n == 0) return PFA_OK;
     }
     if (a->ns == 0 || a->n == 0) return x ? pfa_xchg_launch_only(x, nullptr, out_len, d_out) : PFA_OK;
+    // lanes per site: the smallest power of two that leaves every lane at most 5 chunks
+    // (measured over n = 100 ... 10,000, DESIGN.md section 3: fewer chunks per lane with more lanes per site, at higher
+    // occupancy, is never faster -- bytes in flight per lane win)
+    int lps = 1;
+    while (lps < 32 && (a->Wq + lps - 1) / lps > 5) lps *= 2;
+    const int iter = (a->Wq + lps - 1) / lps;
+    const bool generic = iter > 5;  // lps = 32: records of more than 160 chunks (n > 20,480) stream through one warp per site
+    const bool tma = !generic && (lps >= 4 || a->Wq <= 3);
+    // The TMA kernel on records of 11-160 chunks of a pure-ACGT shard walks the list of sites where two rows differ
+    // (pfa_var_sites_ensure) when at most PFA_SITE_LIST_SHARE of the sites are on it: an unlisted site shows one symbol in
+    // every row and adds nothing to S, H, the SFS, isvar or the per-site H.  The list is built by the first such scan of an
+    // alignment -- a dense one pays that read of its planes once, and scans dense.  Shards with invalid rows, and a forced
+    // validity plane (the three-plane worst case of the benchmarks), keep the dense walk (see pfa_site_scan_tma_kernel).
+    bool listed = false;
+    if (tma && lps >= 4 && !a->has_invalid && a->ns <= INT_MAX) {
+        if (cudaError_t e = pfa_var_sites_ensure(a)) return pfa_fail(ctx, PFA_ERR_CUDA, "site scan: site list: %s", cudaGetErrorString(e));
+        listed = (double)a->n_var_sites <= PFA_SITE_LIST_SHARE * (double)a->ns;
+    }
+    // the list path visits listed sites only: every other site's isvar is 0
+    if (listed && d_isvar) PFA_CUDA(ctx, cudaMemsetAsync(d_isvar, 0, (size_t)a->k * (size_t)a->ns, ctx->stream));
     PfaSiteArgs args;
     unsigned int* work = nullptr;
     if (int rc = pfa_ctx_work(ctx, &work)) return rc;
@@ -766,15 +800,8 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
             if (rc) return rc;
         }
     }
-    // lanes per site: the smallest power of two that leaves every lane at most 5 chunks
-    // (measured over n = 100 ... 10,000, DESIGN.md section 3: fewer chunks per lane with more lanes per site, at higher
-    // occupancy, is never faster -- bytes in flight per lane win)
-    int lps = 1;
-    while (lps < 32 && (a->Wq + lps - 1) / lps > 5) lps *= 2;
-    const int iter = (a->Wq + lps - 1) / lps;
     const size_t smem = sizeof(unsigned long long) * 2 * (size_t)a->k + (args.sfs_in_smem ? sizeof(unsigned int) * (size_t)args.sfs_bins : 0);
     const bool hv = a->has_invalid != 0, multi = a->k > 1;
-    const bool generic = iter > 5;  // lps = 32: records of more than 160 chunks (n > 20,480) stream through one warp per site
     const char* planes = pfa_plane_alloc_name(a->plane_alloc);
     cudaStream_t st = ctx->stream;
     // The TMA variant: one CTA of 512 threads per SM, every warp fed by cp.async.bulk through its own shared-memory slot of
@@ -782,8 +809,9 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
     // over n = 100 ... 20,000 (DESIGN.md section 3): 1-2 % faster at n = 10,000, 6-20 % at n = 2,000 ... 6,000 and 16,000,
     // ~10 % for n <= 384; slower only for records of 4 ... 10 chunks handled by 1-2 lanes (n = 385 ... 1,280), which stay on
     // the register kernel.
-    if (!generic && (lps >= 4 || a->Wq <= 3)) {
+    if (tma) {
         constexpr int nt = 512;
+        const int64_t units = listed ? a->n_var_sites : a->ns;  // list entries or sites
         const int gw = 32 / lps, nwarp = nt / 32;
         const int64_t pass_bytes = (int64_t)gw * a->Wq * 16;  // one pass of a warp, per plane
         // passes per slot: ~5 KB per plane.  Rounded to the nearest when every warp still gets >= 512 blocks (C4 on one GPU, two
@@ -791,12 +819,16 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
         // blocks cost 4 % (0.476 against 0.458 ms), at 5 Mb they break even
         int m = (int)std::max<int64_t>(1, 5000 / pass_bytes);
         const int64_t m_near = std::max<int64_t>(1, (5000 + pass_bytes / 2) / pass_bytes);
-        if (m_near > m && a->ns / ((int64_t)gw * m_near * nwarp * ctx->sm_count) >= 512) m = (int)m_near;
-        const PfaTmaShape shape = {1, a->ns, lps, nt, m, "PFA_SITE_TMA_M", 4, 2, smem, hv};
+        if (m_near > m && units / ((int64_t)gw * m_near * nwarp * ctx->sm_count) >= 512) m = (int)m_near;
+        const PfaTmaShape shape = {1, units, lps, nt, m, "PFA_SITE_TMA_M", 4, 2, smem, hv, units};
         PfaTmaPlan p;
         if (int rc = pfa_tma_plan(a, shape, &p)) return rc;
         if (p.sparse_v) args.vflag = a->vflag;
         args.vs = p.vs;
+        if (listed) {
+            args.sites = a->var_sites;
+            args.nsites = a->n_var_sites;
+        }
         const bool found = pfa_for_shape<1, 1, 1, 2, 1, 3, 4, 3, 4, 4, 4, 5, 8, 3, 8, 4, 8, 5, 16, 3, 16, 4, 16, 5, 32, 3, 32, 4, 32, 5>(
             lps, iter, [&](auto L, auto I) {
                 pfa_for_v_multi(hv, multi, [&](auto V, auto M) {
@@ -806,8 +838,10 @@ int pfa_launch_site_scan(pfa_aln* a, int64_t* d_out, uint8_t* d_isvar, pfa_xchg*
                 });
             });
         if (!found) return pfa_fail(ctx, PFA_ERR_ARG, "site scan: no TMA kernel for lps=%d iter=%d", lps, iter);
-        pfa_note_kernel(ctx, "pfa_site_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d passes_per_slot=%d v_records_per_slot=%d planes=%s",
-                        lps, iter, (int)hv, (int)multi, p.grid, nt, p.m, args.vs, planes);
+        char list_note[64] = "";
+        if (listed) snprintf(list_note, sizeof list_note, " sites=%lld/%lld", (long long)a->n_var_sites, (long long)a->ns);
+        pfa_note_kernel(ctx, "pfa_site_scan_tma_kernel<LPS=%d,ITER=%d,HAS_V=%d,MULTI=%d> grid=%u block=%d passes_per_slot=%d v_records_per_slot=%d planes=%s%s",
+                        lps, iter, (int)hv, (int)multi, p.grid, nt, p.m, args.vs, planes, list_note);
         return pfa_scan_done(a, x, !defer, pfa_escape_sites_kernel, args);
     }
     args.x.wide = 0;  // several CTAs per SM, grids beyond the resident set: the last block alone runs the exchange

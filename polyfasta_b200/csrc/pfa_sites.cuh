@@ -37,6 +37,10 @@ struct PfaSiteArgs {
     const uint32_t* vflag;  // per-site validity flags (pfa_aln::vflag) or nullptr: fetch the whole v plane
     int gc;                 // chunks per flag bit
     int vs;                 // validity records per slot of the TMA kernels (pfa_slot_issue); 0: as many as sites
+    // TMA site scan: the sites it visits -- sites[0 .. nsites), ascending (pfa_aln::var_sites), or with sites == nullptr
+    // sites 0 .. nsites-1 (nsites = ns)
+    const int64_t* sites;
+    int64_t nsites;
     unsigned int* work;  // [2], zero between launches: next block to claim / CTAs done (TMA kernels, pfa_ctx_work)
     PfaXchgDev x;  // x.world > 0: the last block sums `out` over the column shards of all GPUs (pfa_xchg.cuh)
 };
@@ -282,7 +286,9 @@ __device__ __forceinline__ void pfa_mbar_wait(uint64_t* bar, unsigned parity) {
 //     decisions taken before the warp waits for its block and lane 0's bulk copies issued first 1.42 ms.  With every other
 //     site flagged the kernel is bound by instruction issue (ncu r2x: 970 instructions per pass of two sites, 60 % issue
 //     utilisation with four warps per scheduler), not by bytes or by the copy engine.)
-// All copies complete on the slot's mbarrier; lane 0 arms it last with the total byte count (bulk copies that finish before
+// A block is nsite consecutive sites from s0, or (list != nullptr) the nsite sites list[0 .. nsite): then every record of the
+// base planes (and of a whole v area) comes with a bulk copy of its own, issued by the lanes side by side.
+// All copies complete on the slot's mbarrier; lane 0 arms it with the total byte count (bulk copies that finish before
 // the expect_tx only drive the transaction count negative for a moment; the phase cannot complete before lane 0 arrives).
 // Called by ALL lanes of the warp; fl[u] = flag word of site 32 u + lane of the block (sparse only).
 #define PFA_VF_REGS 2  // sparse validity: at most 32 * PFA_VF_REGS sites per slot
@@ -315,9 +321,28 @@ __device__ __forceinline__ const unsigned char* pfa_slot_vrec(const unsigned cha
 template <bool HAS_V>
 __device__ __forceinline__ bool pfa_slot_issue(unsigned char* slot, uint64_t* bar, const unsigned char* p0, const unsigned char* p1,
                                                const unsigned char* pv, bool sparse, int gc, int64_t s0, unsigned nsite, unsigned cap_sites,
-                                               unsigned vs, unsigned rec, int Wq, const uint32_t (&fl)[PFA_VF_REGS], int lane) {
+                                               unsigned vs, unsigned rec, int Wq, const uint32_t (&fl)[PFA_VF_REGS], int lane,
+                                               const int64_t* list = nullptr) {
     __syncwarp();             // every lane has its last values of the slot's previous contents (consumed by pass 1) ...
     pfa_fence_proxy_async();  // ... and those generic-proxy reads come before the async-proxy writes of the copies
+    auto site = [&](unsigned i) -> int64_t { return list ? __ldg(list + i) : s0 + (int64_t)i; };
+    auto copy_planes = [&](unsigned np) {  // the block's records of planes 0 .. np-1 into their areas of the slot
+        if (!list) {
+            if (lane == 0) {
+                pfa_bulk_load(slot, p0 + (size_t)s0 * rec, nsite * rec, bar);
+                pfa_bulk_load(slot + (size_t)cap_sites * rec, p1 + (size_t)s0 * rec, nsite * rec, bar);
+                if (np == 3) pfa_bulk_load(slot + (size_t)2 * cap_sites * rec, pv + (size_t)s0 * rec, nsite * rec, bar);
+            }
+            return;
+        }
+        for (unsigned i = (unsigned)lane; i < nsite; i += 32u) {
+            const size_t off = (size_t)site(i) * rec;
+            unsigned char* d = slot + (size_t)i * rec;
+            pfa_bulk_load(d, p0 + off, rec, bar);
+            pfa_bulk_load(d + (size_t)cap_sites * rec, p1 + off, rec, bar);
+            if (np == 3) pfa_bulk_load(d + (size_t)2 * cap_sites * rec, pv + off, rec, bar);
+        }
+    };
     bool any_flag = HAS_V;
     if (HAS_V && sparse) {
         uint32_t mine = 0;
@@ -325,13 +350,9 @@ __device__ __forceinline__ bool pfa_slot_issue(unsigned char* slot, uint64_t* ba
         for (int u = 0; u < PFA_VF_REGS; ++u) mine |= fl[u];
         any_flag = __any_sync(0xffffffffu, mine != 0u);
     }
-    if (!(HAS_V && sparse) || !any_flag) {   // whole planes (or no validity piece at all): lane 0 alone
-        if (lane == 0) {
-            pfa_mbar_expect_tx(bar, (any_flag ? 3u : 2u) * nsite * rec);
-            pfa_bulk_load(slot, p0 + (size_t)s0 * rec, nsite * rec, bar);
-            pfa_bulk_load(slot + (size_t)cap_sites * rec, p1 + (size_t)s0 * rec, nsite * rec, bar);
-            if (any_flag) pfa_bulk_load(slot + (size_t)2 * cap_sites * rec, pv + (size_t)s0 * rec, nsite * rec, bar);
-        }
+    if (!(HAS_V && sparse) || !any_flag) {   // whole planes (or no validity piece at all)
+        if (lane == 0) pfa_mbar_expect_tx(bar, (any_flag ? 3u : 2u) * nsite * rec);
+        copy_planes(any_flag ? 3u : 2u);
         return any_flag;
     }
     unsigned vbytes = HAS_V ? nsite * rec : 0u;
@@ -362,7 +383,7 @@ __device__ __forceinline__ bool pfa_slot_issue(unsigned char* slot, uint64_t* ba
                     for (uint32_t w = fl[u]; w; w &= w - 1) {
                         const int c0 = (__ffs(w) - 1) * gc;
                         const unsigned len = (unsigned)min(gc, Wq - c0) * 16u;
-                        pfa_bulk_load(slot + (size_t)(2u * cap_sites + rank) * rec + (size_t)c0 * 16u, pv + (size_t)(s0 + si) * rec + (size_t)c0 * 16u, len, bar);
+                        pfa_bulk_load(slot + (size_t)(2u * cap_sites + rank) * rec + (size_t)c0 * 16u, pv + (size_t)site(si) * rec + (size_t)c0 * 16u, len, bar);
                         bytes += len;
                     }
             }
@@ -371,12 +392,8 @@ __device__ __forceinline__ bool pfa_slot_issue(unsigned char* slot, uint64_t* ba
         if (!whole_v) vbytes = bytes;
     }
     __syncwarp();
-    if (lane == 0) {
-        pfa_mbar_expect_tx(bar, 2u * nsite * rec + vbytes);
-        pfa_bulk_load(slot, p0 + (size_t)s0 * rec, nsite * rec, bar);
-        pfa_bulk_load(slot + (size_t)cap_sites * rec, p1 + (size_t)s0 * rec, nsite * rec, bar);
-        if (whole_v) pfa_bulk_load(slot + (size_t)2 * cap_sites * rec, pv + (size_t)s0 * rec, nsite * rec, bar);
-    }
+    if (lane == 0) pfa_mbar_expect_tx(bar, 2u * nsite * rec + vbytes);
+    copy_planes(whole_v ? 3u : 2u);
     return true;
 }
 
@@ -397,6 +414,7 @@ struct PfaTmaShape {
     int m_raise;        // a v area below a whole slot raises m to m + ceil(m * m_raise / 2) (no m_env)
     size_t smem;        // shared memory beyond the slots and their mbarriers: accumulators, queues
     bool has_v;         // the scan reads the validity plane (pfa_aln::has_invalid)
+    int64_t sites;      // sites the scan visits (the shard's, or the listed ones): the flagged share is taken over these
 };
 struct PfaTmaPlan {
     bool sparse_v;          // fetch only the flagged cells of the v plane (PfaSiteArgs::vflag)
